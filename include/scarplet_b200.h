@@ -85,6 +85,22 @@ int sb_plan_destroy(sb_plan* plan);
  * returns 0 if known */
 int sb_plan_set_option(sb_plan* plan, const char* key, long value);
 
+/* Nodata policy of the searches (sb_sweep / sb_sweep_ex); takes effect at the next sb_set_dem_*.
+ *   SB_NODATA_PROPAGATE (default): the reference's semantics -- a NaN anywhere in the DEM reaches
+ *     every un-masked pixel through the full-raster fft2 (dem.py:105, core.py:353-363).
+ *   SB_NODATA_MASK: a masked fit.  V(p) = 1 where the second differences at p (dem.py:88-99) read
+ *     only finite DEM cells; the curvature is zeroed where V = 0 and every fit uses the template
+ *     cells over V = 1 only: n_valid = n - rint(M (*) (1 - V)), ts_m = ts - t**2 (*) (1 - V),
+ *     amp = xcorr / ts_m, error = (T3 - xcorr**2 / ts_m) / (n_valid + eps) + eps.  A template is a
+ *     candidate at a pixel only if n_valid >= ceil(min_coverage * n); a pixel whose own DEM cell is
+ *     not finite gets no result (0 in all four planes).  With min_coverage = 1 every value equals
+ *     the reference's on the same DEM with its holes filled by any values.
+ * Fails for min_coverage outside (0, 1] and, for SB_NODATA_MASK, unless the plan runs the complex64
+ * pipelined kernels (precision 32, fast = 1, lincomb = 1); sb_match_template and
+ * sb_match_template_raster fail on a masked plan.  FFT tiles of a masked sweep are at most 4096. */
+enum { SB_NODATA_PROPAGATE = 0, SB_NODATA_MASK = 1 };
+int sb_plan_set_nodata(sb_plan* plan, int mode, double min_coverage);
+
 /* Spatial sharding of one raster over several GPUs (BASELINE config 5, SURVEY 8e; the reference's
  * analogue is file-level tiling, dem.py:249-278).  The plan keeps the geometry of the WHOLE raster
  * (template centring, edge masks and the circular wrap-around of core.py:359 are evaluated in

@@ -48,6 +48,7 @@ def _declare(lib):
                                    c_int, c_void_p, c_uint]
     lib.sb_plan_destroy.argtypes = [P]
     lib.sb_plan_set_option.argtypes = [P, c_char_p, c_long]
+    lib.sb_plan_set_nodata.argtypes = [P, c_int, c_double]
     lib.sb_plan_launch_count.argtypes = [P]
     lib.sb_plan_launch_count.restype = c_long
     lib.sb_plan_device_bytes.argtypes = [P]
@@ -98,7 +99,7 @@ def _declare(lib):
                  "sb_best_state", "sb_best_pack", "sb_best_select", "sb_best_unpack",
                  "sb_compare_host", "sb_debug_fft", "sb_sync", "sb_plan_set_slab", "sb_plan_dem_rows",
                  "sb_plan_curv_stats", "sb_plan_set_curv_stats", "sb_finalize_ex", "sb_best_state_ex",
-                 "sb_best_merge", "sb_curvature_noise_moments", "sb_fill_nodata"):
+                 "sb_best_merge", "sb_curvature_noise_moments", "sb_fill_nodata", "sb_plan_set_nodata"):
         getattr(lib, name).restype = c_int
     return lib
 
@@ -112,7 +113,7 @@ EXPORTED = ("sb_last_error", "sb_build_info", "sb_plan_create", "sb_plan_destroy
             "sb_debug_fft", "sb_sync", "sb_plan_set_slab", "sb_plan_dem_rows", "sb_plan_curv_stats",
             "sb_plan_set_curv_stats", "sb_plan_stream", "sb_plan_device_bytes", "sb_plan_last_fft_area",
             "sb_finalize_ex", "sb_best_state_ex", "sb_best_merge", "sb_curvature_noise_moments",
-            "sb_fill_nodata", "sb_debug_fft_bench", "sb_sweep_ex")
+            "sb_fill_nodata", "sb_debug_fft_bench", "sb_sweep_ex", "sb_plan_set_nodata")
 
 
 def library_path():

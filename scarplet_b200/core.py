@@ -58,13 +58,13 @@ class _Lease(object):
         return False
 
 
-def _plan_for(data, states=1):
+def _plan_for(data, states=1, nodata="propagate", min_coverage=1.0):
     """A plan for ``data``'s geometry with its DEM uploaded, out of the cache when one is
     free (a plan is used by one call at a time: concurrent callers get their own)."""
     z, dx, dy = _grid_fields(data)
     ny, nx = z.shape
     d = engine.DEFAULTS
-    key = (ny, nx, float(dx), float(dy), d["precision"], d["workspace_mb"], d["max_fft"])
+    key = (ny, nx, float(dx), float(dy), d["precision"], d["workspace_mb"], d["max_fft"], nodata, float(min_coverage))
     plan = None
     with _cache_lock:
         for i, (k, p) in enumerate(_cache):
@@ -74,7 +74,7 @@ def _plan_for(data, states=1):
     for attempt in (0, 1):
         try:
             if plan is None:
-                plan = Plan(ny, nx, dx, dy)
+                plan = Plan(ny, nx, dx, dy, nodata=nodata, min_coverage=min_coverage)
             if plan.states != states:
                 plan.set_states(states)
             plan.set_dem(z)
@@ -161,14 +161,20 @@ def match_template(data, Template, scale, age, angle, **kwargs):
     return amp, age, angle, snr
 
 
-def _sweep(data, Template, scales, ages, ang_max, ang_min, order, **kwargs):
+def _sweep(data, Template, scales, ages, ang_max, ang_min, order, masking, /, **kwargs):
     """One search per entry of ``scales`` in a single device sweep (they share each
-    orientation's curvature spectra); returns the list of (4, ny, nx) stacks."""
+    orientation's curvature spectra); returns the list of (4, ny, nx) stacks.
+    ``masking = (nodata, min_coverage)`` of ``engine.Plan.set_nodata`` (positional: every keyword
+    argument belongs to the template, as in ``calculate_best_fit_parameters_serial``)."""
+    nodata, min_coverage = masking
     spec = None if kwargs else device_spec(Template)
     if spec is None:
+        if nodata != "propagate":
+            raise ValueError("nodata=%r needs a built-in template class; plugin templates follow the "
+                             "reference's NaN semantics" % (nodata,))
         return [_plugin_sweep(data, Template, s, ages, ang_max, ang_min, order, **kwargs) for s in scales]
     angles = P.search_angles(ang_min, ang_max)
-    with _plan_for(data, states=len(scales)) as plan:
+    with _plan_for(data, states=len(scales), nodata=nodata, min_coverage=min_coverage) as plan:
         a_rec, t_rec, age_of, angle_of = plan.build_sweep(spec, list(scales), ages, angles, order)
         plan.reset()
         plan.sweep(a_rec, t_rec)
@@ -176,12 +182,13 @@ def _sweep(data, Template, scales, ages, ang_max, ang_min, order, **kwargs):
 
 
 def calculate_best_fit_parameters(dem, Template, scale, age, ang_max=np.pi / 2,
-                                  ang_min=-np.pi / 2, **kwargs):
+                                  ang_min=-np.pi / 2, nodata="propagate", min_coverage=1.0, **kwargs):
     """Best amplitude / orientation / SNR at one age over a 1-degree orientation
     search (core.py:139-195).  Returns ndarray (4, ny, nx): [amp, age, angle, snr].
     Like the reference (core.py:182) further keyword arguments are accepted and not
-    forwarded to the template."""
-    return _sweep(dem, Template, [scale], [age], ang_max, ang_min, "age_major")[0]
+    forwarded to the template.  ``nodata="mask"`` fits only the cells with data
+    (``engine.Plan.set_nodata``); the default keeps the reference's NaN semantics."""
+    return _sweep(dem, Template, [scale], [age], ang_max, ang_min, "age_major", (nodata, min_coverage))[0]
 
 
 def calculate_best_fit_parameters_serial(dem, Template, scale, ang_max=np.pi / 2,
@@ -189,7 +196,7 @@ def calculate_best_fit_parameters_serial(dem, Template, scale, ang_max=np.pi / 2
     """Flat search over orientations x the 35 default ages (core.py:65-136); keyword
     arguments are forwarded to the template's constructor (core.py:116-121).
     Returns ``(best_amp, best_age, best_angle, best_snr)``."""
-    out = _sweep(dem, Template, [scale], P.default_ages(), ang_max, ang_min, "angle_major", **kwargs)[0]
+    out = _sweep(dem, Template, [scale], P.default_ages(), ang_max, ang_min, "angle_major", _PROPAGATE, **kwargs)[0]
     return out[0], out[1], out[2], out[3]
 
 
@@ -204,14 +211,22 @@ def _match_args(kwargs):
     return ages, ang_max, ang_min, False
 
 
+_PROPAGATE = ("propagate", 1.0)
+
+
+def _masking(kwargs):
+    return kwargs.get("nodata", "propagate"), kwargs.get("min_coverage", 1.0)
+
+
 def match(data, Template, **kwargs):
     """core.py:266-294.  With ``age=`` one orientation search, returned as a stacked
     ndarray (4, ny, nx); without it the 35-age search, returned like
-    ``compare`` as a tuple of four planes."""
+    ``compare`` as a tuple of four planes.  ``nodata=`` / ``min_coverage=``: see
+    ``calculate_best_fit_parameters``."""
     if 'age' in kwargs:
         return calculate_best_fit_parameters(data, Template, **kwargs)
     ages, ang_max, ang_min, _ = _match_args(kwargs)
-    out = _sweep(data, Template, [kwargs['scale']], ages, ang_max, ang_min, "age_major")[0]
+    out = _sweep(data, Template, [kwargs['scale']], ages, ang_max, ang_min, "age_major", _masking(kwargs))[0]
     return out[0], out[1], out[2], out[3]
 
 
@@ -224,7 +239,7 @@ def match_scales(data, Template, scales, **kwargs):
     ``match(..., scale=scale)`` returns."""
     scales = list(scales)
     ages, ang_max, ang_min, single = _match_args(kwargs)
-    res = _sweep(data, Template, scales, ages, ang_max, ang_min, "age_major")
+    res = _sweep(data, Template, scales, ages, ang_max, ang_min, "age_major", _masking(kwargs))
     return {s: (r if single else (r[0], r[1], r[2], r[3])) for s, r in zip(scales, res)}
 
 

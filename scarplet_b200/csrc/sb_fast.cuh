@@ -388,6 +388,67 @@ SB_DEVICE void fit_pixel_fast(float X, float T, const FitT& k, float& amp, float
 }
 
 // ---------------------------------------------------------------------------
+// Nodata-masked fit (DESIGN.md 11).  Every template of a masked sweep has a companion record
+// (t**2 * s2 + i M, same support) whose column pass multiplies by F[U] in both fields, so the
+// inverse row transform of its gbuf plane is  D_t * s2 / norm + i D_m / norm  with
+// D_t = t**2 (*) U and D_m = M (*) U, the template mass over the missing cells.
+// ---------------------------------------------------------------------------
+struct FitM {
+    double ts;               // sum(t**2) of the template              core.py:356
+    double dt_k;             // norm / s2: D_t = dt_k * Re(companion)
+    double amp_f;            // xn: amp = X * xn / ts_m
+    double a_f;              // xn**2 / tn: the epilogue's a = a_f / ts_m
+    float dm_k;              // norm: D_m = dm_k * Im(companion)
+    int n;                   // sum(M)
+    int need;                // ceil(min_coverage * n): least n_valid of a candidate
+    int pad;
+};
+
+// k_tmpl_sums has run over the chunk's 2 * cnt records (templates, then their companions)
+SB_GLOBAL k_mask_consts(Geom g, const Tmpl* SB_RESTRICT tmpls, int tmpl_base, int cnt, double min_coverage,
+                        const TSum* SB_RESTRICT sums, FitM* SB_RESTRICT fitm) {
+    const int i = sb_bx() * 32 + sb_tid();
+    if (i >= cnt) return;
+    const Tmpl p = tmpls[tmpl_base + i];
+    const double xn = g.norm / p.tscale, tn = g.norm / g.c2_scale;      // powers of two
+    FitM m;
+    m.ts = sums[i].ts;
+    m.dt_k = g.norm / tmpls[tmpl_base + cnt + i].tscale;
+    m.amp_f = xn;
+    m.a_f = xn * xn / tn;
+    m.dm_k = (float)g.norm;
+    m.n = (int)rint(sums[i].n_eps);
+    m.need = (int)ceil(min_coverage * (double)m.n);
+    m.pad = 0;
+    fitm[i] = m;
+}
+
+// one pixel of the masked fit: X, T raw outputs of the template's transform, d = (Im, Re) of its
+// companion's (the transforms leave real and imaginary parts swapped).  Where no missing cell lies
+// under M the template's exact constants are used, i.e. the arithmetic of the unmasked fit.
+SB_DEVICE void fit_pixel_masked(float X, float T, const FitT& k, const FitM& m, float2 d, float& amp, float& snr) {
+    const float miss = rintf(d.x * m.dm_k);                              // rint(D_m)
+    if (miss == 0.f) {
+        fit_pixel_fast(X, T, k, amp, snr);
+        return;
+    }
+    const float nv = (float)m.n - miss;                                  // n_valid, exact
+    if (!(nv >= (float)m.need)) {                                        // below min_coverage: no candidate
+        amp = 0.f;
+        snr = -1.f;
+        return;
+    }
+    const double its = 1.0 / (m.ts - (double)d.y * m.dt_k);             // 1 / (ts - D_t)
+    const float its_hi = (float)its, its_lo = (float)(its - (double)its_hi);
+    FitT km = k;
+    km.amp_k = (float)((double)its_hi * m.amp_f);
+    km.a_hi = (float)((double)its_hi * m.a_f);
+    km.a_lo = (float)((double)its_lo * m.a_f);
+    km.inv_n = (float)(1.0 / ((double)nv + kEps));
+    fit_pixel_fast(X, T, km, amp, snr);
+}
+
+// ---------------------------------------------------------------------------
 // k_fit_rows_g<Px>: grid (Py / 2 / GP).  The two transforms
 // a thread group pipelines are the two raster rows that share every 32-byte sector of the
 // interleaved planes (gbuf_index), of ONE template: a thread fetches whole sectors with
@@ -396,7 +457,9 @@ SB_DEVICE void fit_pixel_fast(float X, float T, const FitT& k, float& amp, float
 // only the SNR in registers; amplitude and flat index go straight to the best state when a
 // pixel improves (rare after the first templates of a sweep).
 // ---------------------------------------------------------------------------
-template <int N>
+// MASKED (k_fit_rows_gm): per template, the companion's row pair runs first (comp) and parks its
+// outputs in `park`, every thread in the slots only it reads back; then the template's own.
+template <int N, bool MASKED = false>
 struct FitPairCtx {
     static constexpr int K = sbfft::num_stages(N);
     static constexpr int T = N / E;
@@ -406,6 +469,9 @@ struct FitPairCtx {
     const float2* tw;
     const float4* pair;               // the template's row pair: element kk of row F at pair[2 * kk + F]
     const FitT* s_fit;
+    const FitM* s_fm;                 // MASKED only
+    float2* park;                     // MASKED only: [row F][N]
+    bool comp;                        // MASKED only: this pass is the companion's
     int slot;
     int giA, giB;                     // raster rows of the two streams
     bool actA, actB;
@@ -458,7 +524,8 @@ struct FitPairCtx {
 #pragma unroll
         for (int q = 0; q < E; ++q) {
             float amp, snr;
-            fit_pixel_fast(v[q].y, v[q].x, k, amp, snr);
+            if constexpr (MASKED) fit_pixel_masked(v[q].y, v[q].x, k, s_fm[slot], park[F * N + t + q * T], amp, snr);
+            else fit_pixel_fast(v[q].y, v[q].x, k, amp, snr);
             snr = ((mk >> q) & 1u) ? snr : -1.f;              // edge-masked: never wins
             // first maximum wins (core.py:230-240); equal positive SNRs (in float32 mostly the
             // -90 / +90 degree pair) go to the lower flat index, whatever the batch order.
@@ -479,7 +546,7 @@ struct FitPairCtx {
     // Two pixels (q, q + 8) per packed instruction: X = xcorr pair, Tp = T3 pair (fit_pixel_fast).
     // The window mask is applied to the candidate bits, not to the 16 values; improvements
     // (rare after the first templates of a sweep) are resolved after the common path.
-    static constexpr bool SOA = K > 1;
+    static constexpr bool SOA = K > 1 && !MASKED;
     template <int F> SB_DEVICE void epilogue2(const sbfft::pk_t (&re)[8], const sbfft::pk_t (&im)[8], float (&bs)[E]) {
         using namespace sbfft;
         const int gi = F == 0 ? giA : giB;
@@ -560,6 +627,13 @@ struct FitPairCtx {
         sbfft::stage_math<N, P, float>(v, w);
         if constexpr (P == K - 1) {
             if (SB_DBG_ON(dbg, 64) && v[0].x != 1.2345e-30f) return;
+            if constexpr (MASKED) {
+                if (comp) {
+#pragma unroll
+                    for (int q = 0; q < E; ++q) park[F * N + t + q * T] = v[q];
+                    return;
+                }
+            }
             if constexpr (F == 0) epilogue<0>(v, bsA);
             else epilogue<1>(v, bsB);
         }
@@ -570,11 +644,17 @@ struct FitPairCtx {
     template <int F> SB_DEVICE void load(float2 (&v)[E]) { sbfft::stage_load<N, float>(v, t, F == 0 ? smA : smB); }
 };
 
+// shared memory of k_fit_rows_gm beyond k_fit_rows_g's: the batch's FitM, then the park buffers
 template <int N>
-SB_GLOBAL SB_LAUNCH_BOUNDS((N / E > 256 ? N / E : 256), (N / E > 256 ? 1 : 2))
-k_fit_rows_g(Geom g, int count, const int* SB_RESTRICT slots, const FitT* SB_RESTRICT fit,
-             const float4* SB_RESTRICT gbuf, float* SB_RESTRICT best_snr, float* SB_RESTRICT best_amp, int* best_idx,
-             const float2* SB_RESTRICT tw, const int4* SB_RESTRICT cross, long sub_stride) {
+SB_CONSTEXPR size_t fit_masked_extra_smem() {
+    return kFitMaxBatch * sizeof(FitM) + (size_t)((N / E > 256 ? N / E : 256) / (N / E)) * 2 * N * sizeof(float2);
+}
+
+template <int N, bool MASKED>
+SB_DEVICE void fit_rows_g_body(const Geom& g, int count, const int* SB_RESTRICT slots, const FitT* SB_RESTRICT fit,
+                               const FitM* SB_RESTRICT fitm, int comp_off, const float4* SB_RESTRICT gbuf,
+                               float* SB_RESTRICT best_snr, float* SB_RESTRICT best_amp, int* best_idx,
+                               const float2* SB_RESTRICT tw, const int4* SB_RESTRICT cross, long sub_stride) {
     // grid.y > 1 (small rasters, whose row pairs alone do not fill the GPU): the templates of the
     // launch are dealt round-robin to grid.y sub-streams; sub-stream j folds into copy j of the
     // best state (best_* + j * sub_stride; copy 0 is the state itself) and k_best_fold merges the
@@ -588,7 +668,7 @@ k_fit_rows_g(Geom g, int count, const int* SB_RESTRICT slots, const FitT* SB_RES
     constexpr int THREADS = T > 256 ? T : 256;
     constexpr int GP = THREADS / T;
     constexpr int PL = sbfft::padded_len(N);
-    typedef FitPairCtx<N> Ctx;
+    typedef FitPairCtx<N, MASKED> Ctx;
     const int grp = sb_tid() / T, t = sb_tid() % T;
     float2* sm = (float2*)sb_shared();
     FitT* s_fit = (FitT*)(sm + (long)GP * 2 * PL);
@@ -599,6 +679,13 @@ k_fit_rows_g(Geom g, int count, const int* SB_RESTRICT slots, const FitT* SB_RES
     int* s_gslot = s_flag + kFitMaxBatch + 2;
     float2* tw_s = (float2*)(s_gslot + kFitMaxBatch);
     sbfft::copy_ctw<N, float>(tw_s, tw, sb_tid(), THREADS);
+    FitM* s_fm = nullptr;
+    float2* park = nullptr;
+    if constexpr (MASKED) {
+        s_fm = (FitM*)(tw_s + sbfft::ctw_count<float>(N));
+        park = (float2*)(s_fm + kFitMaxBatch) + (long)grp * 2 * N;
+        if (sb_tid() < count) s_fm[sb_tid()] = fitm[slots ? slots[sb_tid()] : sb_tid()];
+    }
     const int pairs = g.Py / 2;
     const int pr = min(sb_bx() * GP + grp, pairs - 1);    // row pair of the FFT domain
     const int ioA = (2 * pr + g.dly) & (g.Py - 1), ioB = (2 * pr + 1 + g.dly) & (g.Py - 1);
@@ -645,6 +732,9 @@ k_fit_rows_g(Geom g, int count, const int* SB_RESTRICT slots, const FitT* SB_RES
     c.out_nx = g.out_nx;
     c.nx = g.nx;
     c.s_fit = s_fit;
+    c.s_fm = s_fm;
+    c.park = park;
+    c.comp = false;
     c.dbg = g.dbg;
     best_snr += sb_by() * sub_stride;
     best_amp += sb_by() * sub_stride;
@@ -670,10 +760,20 @@ k_fit_rows_g(Geom g, int count, const int* SB_RESTRICT slots, const FitT* SB_RES
 #pragma unroll 1
     for (int i = 0; i < n_act; ++i) {
         const int p = s_list[i];
-        c.pair = gbuf + s_gslot[p] * tmpl_pitch + row_off;
         c.slot = p;
+        if constexpr (MASKED) {
+            // the companion's row pair first (its gbuf plane is comp_off slots further on); no
+            // barrier between the two passes, for the reason given below
+            c.pair = gbuf + (s_gslot[p] + comp_off) * tmpl_pitch + row_off;
+            c.comp = true;
+            const float4* nx0 = gbuf + s_gslot[p] * tmpl_pitch + pf_off;
+            for (int l = t; l < lines; l += T) sb_prefetch_l2(nx0 + 8 * l);
+            leapfrog<Ctx::K>(c, va, vb);
+            c.comp = false;
+        }
+        c.pair = gbuf + s_gslot[p] * tmpl_pitch + row_off;
         if (i + 1 < n_act) {                                // next template's row pair towards L2
-            const float4* nx0 = gbuf + s_gslot[s_list[i + 1]] * tmpl_pitch + pf_off;
+            const float4* nx0 = gbuf + (s_gslot[s_list[i + 1]] + (MASKED ? comp_off : 0)) * tmpl_pitch + pf_off;
             for (int l = t; l < lines; l += T) sb_prefetch_l2(nx0 + 8 * l);
         }
         // no barrier between templates: buffer A was last read before the final barrier,
@@ -686,6 +786,27 @@ k_fit_rows_g(Geom g, int count, const int* SB_RESTRICT slots, const FitT* SB_RES
         if ((c.chg >> q) & 1u) best_snr[(long)c.giA * g.nx + g.ox + jo] = bsA[q];
         if ((c.chg >> (q + 16)) & 1u) best_snr[(long)c.giB * g.nx + g.ox + jo] = bsB[q];
     }
+}
+
+template <int N>
+SB_GLOBAL SB_LAUNCH_BOUNDS((N / E > 256 ? N / E : 256), (N / E > 256 ? 1 : 2))
+k_fit_rows_g(Geom g, int count, const int* SB_RESTRICT slots, const FitT* SB_RESTRICT fit,
+             const float4* SB_RESTRICT gbuf, float* SB_RESTRICT best_snr, float* SB_RESTRICT best_amp, int* best_idx,
+             const float2* SB_RESTRICT tw, const int4* SB_RESTRICT cross, long sub_stride) {
+    fit_rows_g_body<N, false>(g, count, slots, fit, nullptr, 0, gbuf, best_snr, best_amp, best_idx, tw, cross,
+                              sub_stride);
+}
+
+// k_fit_rows_g of a masked sweep: `fitm` per batch slot, the companion of slot s in gbuf slot
+// s + comp_off.  One CTA per SM (the park buffers), so the kernel may use every register.
+template <int N>
+SB_GLOBAL SB_LAUNCH_BOUNDS((N / E > 256 ? N / E : 256), 1)
+k_fit_rows_gm(Geom g, int count, const int* SB_RESTRICT slots, const FitT* SB_RESTRICT fit,
+              const FitM* SB_RESTRICT fitm, int comp_off, const float4* SB_RESTRICT gbuf, float* SB_RESTRICT best_snr,
+              float* SB_RESTRICT best_amp, int* best_idx, const float2* SB_RESTRICT tw, const int4* SB_RESTRICT cross,
+              long sub_stride) {
+    fit_rows_g_body<N, true>(g, count, slots, fit, fitm, comp_off, gbuf, best_snr, best_amp, best_idx, tw, cross,
+                             sub_stride);
 }
 
 // ---------------------------------------------------------------------------
@@ -813,14 +934,15 @@ k_curv_rows_f(Geom g, const float4* SB_RESTRICT diffs, const Angle* SB_RESTRICT 
 // every orientation's F[curv], F[curv^2] are combinations of them with nine scalars --
 // k_combine_spectra, an elementwise pass at HBM speed -- instead of a row kernel and a column
 // kernel per orientation.  Plane order (pair pp, field f -> plane 2 pp + f):
-//   0 dxx   1 dxy   2 dyy   3 s dxx^2   4 s dxy^2   5 s dyy^2   6 s dxx dxy   7 s dxx dyy   8 s dxy dyy   9 unused
+//   0 dxx   1 dxy   2 dyy   3 s dxx^2   4 s dxy^2   5 s dyy^2   6 s dxx dxy   7 s dxx dyy   8 s dxy dyy
+//   9 U (the nodata plane of a masked search, k_second_differences_m; 0 otherwise)
 // (s = c2_scale, the power of two that brings the quadratic planes to the magnitude of the
 // linear ones in the packed transforms).
 // ---------------------------------------------------------------------------
 constexpr int kDiffPairs = 5;
 constexpr int kDiffPlanes = 9;
 
-template <int N>
+template <int N, bool WITH_U = false>
 struct DiffCtx {
     static constexpr int K = sbfft::num_stages(N);
     static constexpr int T = N / E;
@@ -845,7 +967,7 @@ struct DiffCtx {
             case 1: return make_float2(d.z, d.x * d.x * s);
             case 2: return make_float2(d.y * d.y * s, d.z * d.z * s);
             case 3: return make_float2(d.x * d.y * s, d.x * d.z * s);
-            default: return make_float2(d.y * d.z * s, 0.f);
+            default: return make_float2(d.y * d.z * s, WITH_U ? d.w : 0.f);     // d.w: U (k_second_differences_m)
         }
     }
     template <int F> SB_DEVICE void fill(float2 (&v)[E]) const {
@@ -878,15 +1000,15 @@ struct DiffCtx {
 
 // grid (kDiffPairs, ceil(need_rows / 2 / GP)); output layout as k_curv_rows_f with the plane
 // pair in the place of the orientation: cr[pp][kx][rpitch rows] float4
-template <int N>
-SB_GLOBAL SB_LAUNCH_BOUNDS((N / E > 256 ? N / E : 256), (N / E > 256 ? 1 : 2))
-k_diff_rows_f(Geom g, const float4* SB_RESTRICT diffs, float4* SB_RESTRICT cr, const float2* SB_RESTRICT tw) {
+template <int N, bool WITH_U>
+SB_DEVICE void diff_rows_body(const Geom& g, const float4* SB_RESTRICT diffs, float4* SB_RESTRICT cr,
+                              const float2* SB_RESTRICT tw) {
     constexpr int T = N / E;
     constexpr int GP = (T > 256 ? T : 256) / T;
     constexpr int PL = sbfft::padded_len(N);
     const int grp = sb_tid() / T, t = sb_tid() % T;
     const int KX = N / 2 + 1;
-    DiffCtx<N> c;
+    DiffCtx<N, WITH_U> c;
     c.t = t;
     c.smA = (float2*)sb_shared() + (long)grp * 2 * PL;
     c.smB = c.smA + PL;
@@ -902,7 +1024,7 @@ k_diff_rows_f(Geom g, const float4* SB_RESTRICT diffs, float4* SB_RESTRICT cr, c
     float2 va[E], vb[E];
     c.template fill<0>(va);
     c.template fill<1>(vb);
-    leapfrog<DiffCtx<N>::K>(c, va, vb);
+    leapfrog<DiffCtx<N, WITH_U>::K>(c, va, vb);
     sb_sync();                                  // every thread is done with the exchange buffers
 #pragma unroll
     for (int q = 0; q < E; ++q) {
@@ -915,6 +1037,19 @@ k_diff_rows_f(Geom g, const float4* SB_RESTRICT diffs, float4* SB_RESTRICT cr, c
     split_from_shared<N>(c.smB, t, h1);
     if (2 * c.rp < c.need_rows)
         store_row_pair<N, float>(h0, h1, t, cr + (long)c.pp * KX * g.rpitch + 2 * c.rp, g.rpitch);
+}
+
+template <int N>
+SB_GLOBAL SB_LAUNCH_BOUNDS((N / E > 256 ? N / E : 256), (N / E > 256 ? 1 : 2))
+k_diff_rows_f(Geom g, const float4* SB_RESTRICT diffs, float4* SB_RESTRICT cr, const float2* SB_RESTRICT tw) {
+    diff_rows_body<N, false>(g, diffs, cr, tw);
+}
+
+// masked search: plane 9 = U (the .w lane of k_second_differences_m's output)
+template <int N>
+SB_GLOBAL SB_LAUNCH_BOUNDS((N / E > 256 ? N / E : 256), (N / E > 256 ? 1 : 2))
+k_diff_rows_fm(Geom g, const float4* SB_RESTRICT diffs, float4* SB_RESTRICT cr, const float2* SB_RESTRICT tw) {
+    diff_rows_body<N, true>(g, diffs, cr, tw);
 }
 
 // per-orientation coefficients of the nine planes (host: float32 of the float64 cos / sin values)

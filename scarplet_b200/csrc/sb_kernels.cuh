@@ -236,6 +236,81 @@ SB_GLOBAL k_second_differences(int ny, int nx, int row0, int drows, const double
 }
 
 // ---------------------------------------------------------------------------
+// Nodata-masked search (sb_plan_set_nodata, SB_NODATA_MASK).  V(p) = 1 when every DEM cell the
+// second differences at p depend on (dem.py:88-99, second_differences_at) is finite, U = 1 - V.
+// ---------------------------------------------------------------------------
+SB_DEVICE bool finite_cell(double v) { return v - v == 0.0; }     // false for NaN and +-Inf
+
+SB_DEVICE bool stencil_finite(const double* SB_RESTRICT z, int ny, int nx, int gi, int li, int drows, int j) {
+    const long o = (long)li * nx + j;
+    const bool jm = j >= 1, jp = j <= nx - 2;
+    const bool im = gi >= 1 && li >= 1, ip = gi <= ny - 2 && li <= drows - 2;
+    bool ok = finite_cell(sb_ldg(z + o));
+    if (jm && (jp || im)) ok &= finite_cell(sb_ldg(z + o - 1));       // dxx, dxy
+    if (jm && jp) ok &= finite_cell(sb_ldg(z + o + 1));               // dxx
+    if (im && (ip || jm)) ok &= finite_cell(sb_ldg(z + o - nx));      // dyy, dxy
+    if (im && ip) ok &= finite_cell(sb_ldg(z + o + nx));              // dyy
+    if (im && jm) ok &= finite_cell(sb_ldg(z + o - nx - 1));          // dxy
+    return ok;
+}
+
+// k_second_differences for the masked search: out32 = (V dxx, V dxy, V dyy, U)
+SB_GLOBAL k_second_differences_m(int ny, int nx, int row0, int drows, const double* SB_RESTRICT dem, double dx,
+                                 double dx2, double dy2, float4* SB_RESTRICT out32) {
+    const long n = (long)drows * nx;
+    const long i = (long)sb_bx() * 256 + sb_tid();
+    if (i >= n) return;
+    const int li = (int)(i / nx), j = (int)(i % nx);
+    int gi = row0 + li;
+    gi -= gi >= ny ? ny : 0;
+    if (!stencil_finite(dem, ny, nx, gi, li, drows, j)) {
+        out32[i] = make_float4(0.f, 0.f, 0.f, 1.f);
+        return;
+    }
+    const Diff3 d = second_differences_at(dem, ny, nx, gi, li, drows, j, dx, dx2, dy2);
+    out32[i] = make_float4((float)d.dxx, (float)d.dxy, (float)d.dyy, 0.f);
+}
+
+// k_curv_sumsq for the masked search: dxx**2 + dyy**2 summed over the pixels with V = 1 only
+SB_GLOBAL k_curv_sumsq_m(int ny, int nx, int row0, int drows, int own_first, int own_rows,
+                         const double* SB_RESTRICT dem, double dx, double dx2, double dy2, double* SB_RESTRICT partial) {
+    double* sd = (double*)sb_shared();
+    const long n = (long)own_rows * nx;
+    double acc = 0.0;
+    for (long i = (long)sb_bx() * 256 + sb_tid(); i < n; i += (long)sb_nbx() * 256) {
+        const int r = own_first + (int)(i / nx), c = (int)(i % nx);
+        int gr = row0 + r;
+        gr -= gr >= ny ? ny : 0;
+        if (!stencil_finite(dem, ny, nx, gr, r, drows, c)) continue;
+        const Diff3 d = second_differences_at(dem, ny, nx, gr, r, drows, c, dx, dx2, dy2);
+        acc += d.dxx * d.dxx + d.dyy * d.dyy;
+    }
+    sd[sb_tid()] = acc;
+    sb_sync();
+    for (int w = 128; w > 0; w >>= 1) {
+        if (sb_tid() < w) sd[sb_tid()] += sd[sb_tid() + w];
+        sb_sync();
+    }
+    if (sb_tid() == 0) partial[sb_bx()] = sd[0];
+}
+
+// After a masked sweep: a pixel whose own DEM cell is not finite gets no result (initial best
+// state in every state).  The plan's best rows are brow0 .. brow0 + brows - 1; state s at s * bn.
+SB_GLOBAL k_best_clear_nodata(int ny, int nx, int row0, int brow0, int brows, int n_states, long bn,
+                              const double* SB_RESTRICT dem, float* snr, float* amp, int* idx) {
+    const long i = (long)sb_bx() * 256 + sb_tid();
+    if (i >= (long)brows * nx) return;
+    int li = brow0 + (int)(i / nx) - row0;
+    li += li < 0 ? ny : 0;
+    if (finite_cell(sb_ldg(dem + (long)li * nx + i % nx))) return;
+    for (int s = 0; s < n_states; ++s) {
+        snr[s * bn + i] = 0.f;
+        amp[s * bn + i] = 0.f;
+        idx[s * bn + i] = 0x7fffffff;
+    }
+}
+
+// ---------------------------------------------------------------------------
 // windowed template value at one pixel (float64)
 // ---------------------------------------------------------------------------
 SB_DEVICE double template_at(const Tmpl& p, double x, double y) {
@@ -453,11 +528,12 @@ k_curv_cols(Geom g, const typename Vec<R>::v4* SB_RESTRICT cr, typename Vec<R>::
 // so a thread's only non-zero samples are its first and its last: two template evaluations
 // per row instead of sixteen guarded ones (the unrolled float64 exp made this the largest
 // kernel of the library, 70 KB of code), and a sparse first FFT stage.
-template <int N, typename R, bool XSPARSE>
-SB_GLOBAL SB_LAUNCH_BOUNDS((N / E > 256 ? N / E : 256), ((N / E > 256 || sizeof(R) == 8) ? 1 : 2))
-k_tmpl_rows(Geom g, const Tmpl* SB_RESTRICT tmpls, int tmpl_base, const double* SB_RESTRICT xvec,
-            const double* SB_RESTRICT yvec, typename Vec<R>::v4* SB_RESTRICT trt, double2* SB_RESTRICT part,
-            const typename Vec<R>::v2* SB_RESTRICT tw, const double* SB_RESTRICT box) {
+// SQUARED (k_tmpl_rows_sq, the companions of a masked sweep): t**2 * tscale is packed in place of t * tscale
+template <int N, typename R, bool XSPARSE, bool SQUARED>
+SB_DEVICE void tmpl_rows_body(const Geom& g, const Tmpl* SB_RESTRICT tmpls, int tmpl_base, const double* SB_RESTRICT xvec,
+                              const double* SB_RESTRICT yvec, typename Vec<R>::v4* SB_RESTRICT trt,
+                              double2* SB_RESTRICT part, const typename Vec<R>::v2* SB_RESTRICT tw,
+                              const double* SB_RESTRICT box) {
     typedef typename Vec<R>::v2 C2;
     typedef typename Vec<R>::v4 C4;
     constexpr int T = N / E;
@@ -491,7 +567,7 @@ k_tmpl_rows(Geom g, const Tmpl* SB_RESTRICT tmpls, int tmpl_base, const double* 
                 if (w != 0.0) {                                   // M = template != 0, core.py:348
                     cnt += 1.0;
                     ssq += w * w;
-                    val = mk2<R>((R)(w * p.tscale), (R)1);
+                    val = mk2<R>((R)((SQUARED ? w * w : w) * p.tscale), (R)1);
                 }
             }
             v[q] = val;
@@ -521,6 +597,22 @@ k_tmpl_rows(Geom g, const Tmpl* SB_RESTRICT tmpls, int tmpl_base, const double* 
     }
     if (2 * rp < rows)
         store_row_pair<N, R>(h0, h1, t, trt + (long)p_loc * KX * g.syp + 2 * rp, g.syp);
+}
+
+template <int N, typename R, bool XSPARSE>
+SB_GLOBAL SB_LAUNCH_BOUNDS((N / E > 256 ? N / E : 256), ((N / E > 256 || sizeof(R) == 8) ? 1 : 2))
+k_tmpl_rows(Geom g, const Tmpl* SB_RESTRICT tmpls, int tmpl_base, const double* SB_RESTRICT xvec,
+            const double* SB_RESTRICT yvec, typename Vec<R>::v4* SB_RESTRICT trt, double2* SB_RESTRICT part,
+            const typename Vec<R>::v2* SB_RESTRICT tw, const double* SB_RESTRICT box) {
+    tmpl_rows_body<N, R, XSPARSE, false>(g, tmpls, tmpl_base, xvec, yvec, trt, part, tw, box);
+}
+
+template <int N, bool XSPARSE>
+SB_GLOBAL SB_LAUNCH_BOUNDS((N / E > 256 ? N / E : 256), (N / E > 256 ? 1 : 2))
+k_tmpl_rows_sq(Geom g, const Tmpl* SB_RESTRICT tmpls, int tmpl_base, const double* SB_RESTRICT xvec,
+               const double* SB_RESTRICT yvec, float4* SB_RESTRICT trt, double2* SB_RESTRICT part,
+               const float2* SB_RESTRICT tw) {
+    tmpl_rows_body<N, float, XSPARSE, true>(g, tmpls, tmpl_base, xvec, yvec, trt, part, tw, nullptr);
 }
 
 // fixed-order sum of the per-row partials of each template

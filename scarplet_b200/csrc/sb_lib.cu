@@ -53,6 +53,7 @@ struct Buf {
 bool is_pow2(int n) { return n > 0 && (n & (n - 1)) == 0; }
 constexpr int kMinFft = 128;
 constexpr int kMaxFftSupported = 8192;
+constexpr int kMaxFftMasked = 4096;      // k_fit_rows_gm's shared memory
 
 // One FFT tile along an axis: domain length P, first output pixel o, out output pixels.
 struct TileSpec {
@@ -110,6 +111,10 @@ struct sb_plan {
     double c2_scale = 1.0;
     double curv_sumsq = 0.0, curv_count = 0.0;   // over the plan's own rows (slab_lo .. slab_hi)
     bool dem_nonfinite = false;    // the DEM holds a NaN / Inf: every FFT domain is poisoned like the reference's
+    // nodata policy (sb_plan_set_nodata): requested, and in force for the current DEM
+    int nodata_req = SB_NODATA_PROPAGATE, nodata = SB_NODATA_PROPAGATE;
+    double min_cov_req = 1.0, min_cov = 1.0;
+    Buf fitm;
     int profile = 0;
     int dbg = 0;                   // ablation switches (-DSB_ABLATE builds only)
     std::vector<sb_event_t> ev_pool;
@@ -296,7 +301,7 @@ void apply_curv_stats(sb_plan* pl, double sumsq, double count) {
     pl->c2_scale = 1.0;
     if (std::isfinite(sigma) && sigma > 1e-150 && sigma < 1e150)
         pl->c2_scale = std::exp2(std::round(-std::log2(sigma)));
-    pl->dem_nonfinite = !std::isfinite(sumsq);
+    pl->dem_nonfinite = pl->nodata != SB_NODATA_MASK && !std::isfinite(sumsq);
 }
 
 long bn_all(const sb_plan* pl) { return pl->bn() * pl->n_states; }
@@ -320,15 +325,25 @@ int after_dem(sb_plan* pl) {
     const long n = (long)pl->drows * pl->nx;
     if (!pl->d_diffs32) SB_TRY(sb_rt_malloc((void**)&pl->d_diffs32, (size_t)n * sizeof(float4)));
     pl->diffs64_valid = false;
-    SB_LAUNCH(sb::k_second_differences, dim3(div_up(n, 256)), dim3(256), 0, pl->stream, pl->ny, pl->nx, pl->row0,
-              pl->drows, (const double*)pl->d_dem, pl->dx, pl->dx2, pl->dy2, (double*)nullptr, pl->d_diffs32);
-    SB_OK(check_launch(pl, "k_second_differences"));
+    pl->nodata = pl->nodata_req;
+    pl->min_cov = pl->min_cov_req;
+    const bool masked = pl->nodata == SB_NODATA_MASK;
+    if (masked) {
+        SB_LAUNCH(sb::k_second_differences_m, dim3(div_up(n, 256)), dim3(256), 0, pl->stream, pl->ny, pl->nx, pl->row0,
+                  pl->drows, (const double*)pl->d_dem, pl->dx, pl->dx2, pl->dy2, pl->d_diffs32);
+        SB_OK(check_launch(pl, "k_second_differences_m"));
+    } else {
+        SB_LAUNCH(sb::k_second_differences, dim3(div_up(n, 256)), dim3(256), 0, pl->stream, pl->ny, pl->nx, pl->row0,
+                  pl->drows, (const double*)pl->d_dem, pl->dx, pl->dx2, pl->dy2, (double*)nullptr, pl->d_diffs32);
+        SB_OK(check_launch(pl, "k_second_differences"));
+    }
     // statistics over the plan's own rows only, so that the slabs of a sharded raster add up
     const int own_first = pl->slab_lo - pl->row0 + (pl->slab_lo < pl->row0 ? pl->ny : 0);
     const long own = pl->brows() * (long)pl->nx;
     const int blocks = std::max(1, std::min(1024, div_up(own, 256)));
     SB_OK(ensure(pl->raw, (size_t)blocks * sizeof(double)));
-    SB_LAUNCH(sb::k_curv_sumsq, dim3(blocks), dim3(256), 256 * sizeof(double), pl->stream, pl->ny, pl->nx, pl->row0,
+    auto sumsq_kern = masked ? sb::k_curv_sumsq_m : sb::k_curv_sumsq;
+    SB_LAUNCH(sumsq_kern, dim3(blocks), dim3(256), 256 * sizeof(double), pl->stream, pl->ny, pl->nx, pl->row0,
               pl->drows, own_first, (int)pl->brows(), (const double*)pl->d_dem, pl->dx, pl->dx2, pl->dy2,
               (double*)pl->raw.p);
     SB_OK(check_launch(pl, "k_curv_sumsq"));
@@ -381,8 +396,10 @@ int plan_axis(const sb_plan* pl, int n, int r0, int r1, int lo, int hi, bool all
     ax->tiles.clear();
     const int ext = hi - lo + 1;
     const int len = r1 - r0;
-    // complex128 at 8192 would need 270 KB of shared memory per column in k_conv_cols
-    const int max_fft = std::min(pl->max_fft, pl->precision == 64 ? 4096 : kMaxFftSupported);
+    // complex128 at 8192 would need 270 KB of shared memory per column in k_conv_cols, the masked
+    // fit kernel 264 KB per CTA
+    const int max_fft = std::min(pl->max_fft, pl->precision == 64 ? 4096
+                                              : pl->nodata == SB_NODATA_MASK ? kMaxFftMasked : kMaxFftSupported);
     const bool can_periodic = allow_periodic && r0 == 0 && r1 == n && is_pow2(n) && n >= kMinFft && n <= max_fft &&
                               !pl->force_pad;
     auto take_periodic = [&]() {
@@ -503,6 +520,11 @@ int run_sweep_t(sb_plan* pl, const sb_angle* angles, int n_angles, const sb_temp
     if (so.raw_amp && !pl->whole()) return fail("match_template planes need a plan over the whole raster");
     constexpr bool kF32 = std::is_same<R, float>::value;
     const bool fast = kF32 && pl->fast;
+    // nodata-masked search: complex64 pipelined kernels with the linear-combination set-up only
+    const bool masked = pl->nodata == SB_NODATA_MASK;
+    if (masked && so.raw_amp) return fail("nodata mask: sb_match_template keeps the reference's NaN semantics");
+    if (masked && !(fast && pl->lincomb))
+        return fail("nodata mask needs precision 32 and the options fast and lincomb");
     if (!fast) SB_OK(ensure_diffs64(pl));
 
     // order templates by search angle (then best state) so that each curvature spectrum is built once
@@ -580,7 +602,10 @@ int run_sweep_t(sb_plan* pl, const sb_angle* angles, int n_angles, const sb_temp
         first[a + 1] += first[a];
     }
     if (hint) max_per_angle = std::max(max_per_angle, hint[4]);
-    int Bt = (int)std::max<size_t>(1, std::min<size_t>(64, (budget * 6 / 10) / per_tmpl));
+    // a masked sweep carries a companion per template through the per-template kernels, in the same
+    // launches (at most 64 records)
+    const int rec_per_tmpl = masked ? 2 : 1;
+    int Bt = (int)std::max<size_t>(1, std::min<size_t>(64 / rec_per_tmpl, (budget * 6 / 10) / (per_tmpl * rec_per_tmpl)));
     int Ba = (int)std::max<size_t>(1, std::min<size_t>((size_t)n_angles, (budget * 4 / 10) / per_angle));
     Ba = std::min(Ba, 64);
     if (max_per_angle == 1) Bt = std::min(Bt, Ba), Ba = std::min(Ba, Bt);
@@ -608,13 +633,16 @@ int run_sweep_t(sb_plan* pl, const sb_angle* angles, int n_angles, const sb_temp
         SB_TRY(sb_rt_h2d(pl->coef.p, coef.data(), coef.size() * sizeof(sb::SpecCoef), pl->stream));
         SB_TRY(sb_rt_sync(pl->stream));
     }
-    SB_OK(ensure(pl->fct, (size_t)Ba * 2 * KXm * Pym * sizeof(C2)));
-    SB_OK(ensure(pl->trt, (size_t)Bt * KXm * syp * sizeof(C4)));
-    SB_OK(ensure(pl->part, (size_t)Bt * syp * sizeof(double2)));
-    SB_OK(ensure(pl->gbuf, (size_t)Bt * Pym * kpitch_m * sizeof(C4)));
-    SB_OK(ensure(pl->sums, (size_t)Bt * sizeof(sb::TSum)));
-    SB_OK(ensure(pl->fit, (size_t)Bt * sizeof(sb::FitT)));
-    SB_OK(ensure(pl->tmpls, (size_t)n_tmpls * sizeof(sb::Tmpl)));
+    // masked: orientation slot Ba of fct holds (F[U], F[U]), the spectra the companions multiply by
+    SB_OK(ensure(pl->fct, (size_t)(Ba + (masked ? 1 : 0)) * 2 * KXm * Pym * sizeof(C2)));
+    const int Br = Bt * rec_per_tmpl;
+    SB_OK(ensure(pl->trt, (size_t)Br * KXm * syp * sizeof(C4)));
+    SB_OK(ensure(pl->part, (size_t)Br * syp * sizeof(double2)));
+    SB_OK(ensure(pl->gbuf, (size_t)Br * Pym * kpitch_m * sizeof(C4)));
+    SB_OK(ensure(pl->sums, (size_t)Br * sizeof(sb::TSum)));
+    SB_OK(ensure(pl->fit, (size_t)Br * sizeof(sb::FitT)));
+    if (masked) SB_OK(ensure(pl->fitm, (size_t)Bt * sizeof(sb::FitM)));
+    SB_OK(ensure(pl->tmpls, (size_t)n_tmpls * rec_per_tmpl * sizeof(sb::Tmpl)));
     SB_OK(ensure(pl->angles, (size_t)n_angles * sizeof(sb::Angle)));
 
     // the schedule: angle batches, chunks of templates, and per chunk the slots of each best state
@@ -660,7 +688,24 @@ int run_sweep_t(sb_plan* pl, const sb_angle* angles, int n_angles, const sb_temp
     SB_OK(ensure(pl->slots, std::max<size_t>(1, slot_table.size()) * sizeof(int)));
     if (!slot_table.empty())
         SB_TRY(sb_rt_h2d(pl->slots.p, slot_table.data(), slot_table.size() * sizeof(int), pl->stream));
-    SB_TRY(sb_rt_h2d(pl->tmpls.p, tm.data(), (size_t)n_tmpls * sizeof(sb::Tmpl), pl->stream));
+    // device records: a masked sweep lays each chunk out as its templates, then their companions
+    // (k_tmpl_rows_sq packs t**2 with the power of two tscale**2; fct orientation slot Ba = F[U]) --
+    // one run of the persistent column kernels, which stage their spectrum column per run of equal slots
+    std::vector<sb_template> dev;
+    if (masked) {
+        dev.resize((size_t)2 * n_tmpls);
+        for (auto& ab : batches)
+            for (auto& ch : ab.chunks)
+                for (int i = 0; i < ch.cnt; ++i) {
+                    sb_template t = tm[ch.pb + i];
+                    dev[2 * ch.pb + i] = t;
+                    t.angle_id = ab.a0 + Ba;
+                    t.tscale = t.tscale * t.tscale;
+                    dev[2 * ch.pb + ch.cnt + i] = t;
+                }
+    }
+    const std::vector<sb_template>& recs = masked ? dev : tm;
+    SB_TRY(sb_rt_h2d(pl->tmpls.p, recs.data(), recs.size() * sizeof(sb::Tmpl), pl->stream));
     SB_TRY(sb_rt_h2d(pl->angles.p, angles, (size_t)n_angles * sizeof(sb::Angle), pl->stream));
     std::vector<double> casa;
     if (any_err && fast && !so.raw_amp) {
@@ -750,7 +795,7 @@ int run_sweep_t(sb_plan* pl, const sb_angle* angles, int n_angles, const sb_temp
                 SB_OK(dispatch_n(Px, [&](auto nn) {
                     constexpr int N = decltype(nn)::value;
                     using S = Shape<N, float>;
-                    auto kern = sb::k_diff_rows_f<N>;
+                    auto kern = masked ? sb::k_diff_rows_fm<N> : sb::k_diff_rows_f<N>;
                     SB_ALLOW_SMEM(kern, S::smem_conv_f);
                     ProfScope prof(pl, K_CURV_ROWS);
                     SB_LAUNCH(kern, dim3(sb::kDiffPairs, div_up(div_up(need_rows, 2), S::GP)), dim3(S::threads),
@@ -768,6 +813,13 @@ int run_sweep_t(sb_plan* pl, const sb_angle* angles, int n_angles, const sb_temp
                               pl->stream, g, (const float4*)pl->cr.p, (float2*)pl->spec9.p, (const float2*)twy);
                     return check_launch(pl, "k_curv_cols");
                 }));
+                if (masked) {
+                    const size_t plane = (size_t)KX * Py;       // float2 elements of one spectrum plane
+                    const float2* fu = (const float2*)pl->spec9.p + (size_t)sb::kDiffPlanes * plane;
+                    for (int f = 0; f < 2; ++f)
+                        SB_TRY(sb_rt_d2d((float2*)pl->fct.p + (size_t)(2 * Ba + f) * plane, fu, plane * sizeof(float2),
+                                         pl->stream));
+                }
             }
             for (auto& ab : batches) {
                 const int a0 = ab.a0, a1 = ab.a1;
@@ -813,34 +865,60 @@ int run_sweep_t(sb_plan* pl, const sb_angle* angles, int n_angles, const sb_temp
                     return check_launch(pl, "k_curv_cols");
                 }));
                 for (auto& ch : ab.chunks) {
-                    const int pb = ch.pb, cnt = ch.cnt;
+                    // the chunk's device records (a masked sweep: templates, then companions)
+                    const int pb = ch.pb * rec_per_tmpl, cnt = ch.cnt * rec_per_tmpl;
                     SB_OK(dispatch_n(Px, [&](auto nn) {
                         constexpr int N = decltype(nn)::value;
                         using S = Shape<N, R>;
                         ProfScope prof(pl, K_TMPL_ROWS);
                         // narrow templates: two samples per thread (needs a radix-16 first stage)
+                        const bool xsparse = N >= 256 && hi_x <= S::T - 1 && lo_x >= -S::T;
+                        const int nt = ch.cnt;            // the templates; a masked sweep's companions follow
                         if constexpr (N >= 256) {
-                            if (hi_x <= S::T - 1 && lo_x >= -S::T) {
+                            if (xsparse) {
                                 auto kern = sb::k_tmpl_rows<N, R, true>;
                                 SB_ALLOW_SMEM(kern, S::smem);
-                                SB_LAUNCH(kern, dim3(div_up(syp / 2, S::GP), cnt), dim3(S::threads), S::smem,
+                                SB_LAUNCH(kern, dim3(div_up(syp / 2, S::GP), nt), dim3(S::threads), S::smem,
                                           pl->stream, g, d_tm, pb, (const double*)pl->d_x, (const double*)pl->d_y,
                                           (C4*)pl->trt.p, (double2*)pl->part.p, twx, (const double*)pl->tbox.p);
-                                return check_launch(pl, "k_tmpl_rows");
+                                SB_OK(check_launch(pl, "k_tmpl_rows"));
                             }
                         }
-                        auto kern = sb::k_tmpl_rows<N, R, false>;
-                        SB_ALLOW_SMEM(kern, S::smem);
-                        SB_LAUNCH(kern, dim3(div_up(syp / 2, S::GP), cnt), dim3(S::threads), S::smem,
-                                  pl->stream, g, d_tm, pb, (const double*)pl->d_x, (const double*)pl->d_y,
-                                  (C4*)pl->trt.p, (double2*)pl->part.p, twx, (const double*)pl->tbox.p);
-                        return check_launch(pl, "k_tmpl_rows");
+                        if (!xsparse) {
+                            auto kern = sb::k_tmpl_rows<N, R, false>;
+                            SB_ALLOW_SMEM(kern, S::smem);
+                            SB_LAUNCH(kern, dim3(div_up(syp / 2, S::GP), nt), dim3(S::threads), S::smem,
+                                      pl->stream, g, d_tm, pb, (const double*)pl->d_x, (const double*)pl->d_y,
+                                      (C4*)pl->trt.p, (double2*)pl->part.p, twx, (const double*)pl->tbox.p);
+                            SB_OK(check_launch(pl, "k_tmpl_rows"));
+                        }
+                        if constexpr (kF32) {
+                            if (masked) {
+                                // the companions: t**2, records pb + nt ..; trt / part slots nt ..
+                                auto kern = sb::k_tmpl_rows_sq<N, false>;
+                                if constexpr (N >= 256) {
+                                    if (xsparse) kern = sb::k_tmpl_rows_sq<N, true>;
+                                }
+                                SB_ALLOW_SMEM(kern, S::smem);
+                                SB_LAUNCH(kern, dim3(div_up(syp / 2, S::GP), nt), dim3(S::threads), S::smem,
+                                          pl->stream, g, d_tm, pb + nt, (const double*)pl->d_x, (const double*)pl->d_y,
+                                          (float4*)pl->trt.p + (size_t)nt * (N / 2 + 1) * syp,
+                                          (double2*)pl->part.p + (size_t)nt * syp, (const float2*)twx);
+                                SB_OK(check_launch(pl, "k_tmpl_rows_sq"));
+                            }
+                        }
+                        return 0;
                     }));
                     {
                         ProfScope prof(pl, K_TMPL_SUMS);
                         SB_LAUNCH(sb::k_tmpl_sums, dim3(cnt), dim3(32), 32 * sizeof(double2), pl->stream, g, d_tm, pb, cnt,
                                   (const double2*)pl->part.p, (sb::TSum*)pl->sums.p, (sb::FitT*)pl->fit.p);
                         SB_OK(check_launch(pl, "k_tmpl_sums"));
+                        if (masked) {
+                            SB_LAUNCH(sb::k_mask_consts, dim3(div_up(ch.cnt, 32)), dim3(32), 0, pl->stream, g, d_tm, pb,
+                                      ch.cnt, pl->min_cov, (const sb::TSum*)pl->sums.p, (sb::FitM*)pl->fitm.p);
+                            SB_OK(check_launch(pl, "k_mask_consts"));
+                        }
                     }
                     const bool fast_fit = fast && !so.raw_amp;
                     if constexpr (kF32) {
@@ -937,6 +1015,22 @@ int run_sweep_t(sb_plan* pl, const sb_angle* angles, int n_angles, const sb_temp
                                     constexpr int N = decltype(nn)::value;
                                     using S = Shape<N, float>;
                                     ProfScope prof(pl, K_FIT_ROWS);
+                                    if (masked) {
+                                        // FFT lengths <= 4096 only: the park buffers need 2 N float2 per group
+                                        if constexpr (N <= kMaxFftMasked) {
+                                            auto kern = sb::k_fit_rows_gm<N>;
+                                            constexpr size_t smem = S::smem_fit_f + sb::fit_masked_extra_smem<N>();
+                                            SB_ALLOW_SMEM(kern, smem);
+                                            SB_LAUNCH(kern, dim3(div_up(Py / 2, S::GP), nsub), dim3(S::threads), smem,
+                                                      pl->stream, g, gp.count, d_slots, (const sb::FitT*)pl->fit.p,
+                                                      (const sb::FitM*)pl->fitm.p, ch.cnt, (const float4*)pl->gbuf.p,
+                                                      bsnr, bamp, bidx, (const float2*)twx,
+                                                      gp.err ? (const int4*)pl->cross.p : (const int4*)nullptr,
+                                                      sub_stride);
+                                            return check_launch(pl, "k_fit_rows_gm");
+                                        }
+                                        return fail("internal: masked fit at FFT length " + std::to_string(N));
+                                    }
                                     // (a variant without the get_err_mask members spills MORE: 564 bytes against 312)
                                     auto kern = sb::k_fit_rows_g<N>;
                                     SB_ALLOW_SMEM(kern, S::smem_fit_f);
@@ -977,6 +1071,12 @@ int run_sweep_t(sb_plan* pl, const sb_angle* angles, int n_angles, const sb_temp
                   (const float*)pl->d_bsnr + sub_stride, (const float*)pl->d_bamp + sub_stride,
                   (const int*)pl->d_bidx + sub_stride, pl->d_bsnr, pl->d_bamp, pl->d_bidx);
         SB_OK(check_launch(pl, "k_best_fold"));
+    }
+    if (masked) {
+        SB_LAUNCH(sb::k_best_clear_nodata, dim3(div_up(bn, 256)), dim3(256), 0, pl->stream, pl->ny, pl->nx, pl->row0,
+                  pl->slab_lo, (int)pl->brows(), pl->n_states, bn, (const double*)pl->d_dem, pl->d_bsnr, pl->d_bamp,
+                  pl->d_bidx);
+        SB_OK(check_launch(pl, "k_best_clear_nodata"));
     }
     drain_profile(pl);
     return 0;
@@ -1072,7 +1172,8 @@ int sb_plan_destroy(sb_plan* pl) {
     for (auto& kv : pl->tw) sb_rt_free(kv.second);
     for (auto e : pl->ev_pool) sb_rt_event_destroy(e);
     for (Buf* b : {&pl->cr, &pl->fct, &pl->trt, &pl->part, &pl->gbuf, &pl->sums, &pl->fit, &pl->tmpls, &pl->angles,
-                   &pl->tables, &pl->raw, &pl->tbox, &pl->slots, &pl->cross, &pl->casa, &pl->aux, &pl->spec9, &pl->coef})
+                   &pl->tables, &pl->raw, &pl->tbox, &pl->slots, &pl->cross, &pl->casa, &pl->aux, &pl->spec9, &pl->coef,
+                   &pl->fitm})
         release(*b);
 #ifndef SB_EMU
     if (pl->own_stream) cudaStreamDestroy(pl->stream);
@@ -1113,6 +1214,20 @@ int sb_plan_set_option(sb_plan* pl, const char* key, long value) {
         return 0;
     }
     return fail("unknown option " + k);
+}
+
+int sb_plan_set_nodata(sb_plan* pl, int mode, double min_coverage) {
+    if (!pl) return fail("null plan");
+    if (mode != SB_NODATA_PROPAGATE && mode != SB_NODATA_MASK)
+        return fail("sb_plan_set_nodata: mode must be SB_NODATA_PROPAGATE or SB_NODATA_MASK");
+    if (!(min_coverage > 0.0 && min_coverage <= 1.0)) return fail("sb_plan_set_nodata: min_coverage must be in (0, 1]");
+    if (mode == SB_NODATA_MASK && pl->precision != 32)
+        return fail("sb_plan_set_nodata: the nodata mask needs precision 32 (the complex64 pipeline)");
+    if (mode == SB_NODATA_MASK && !pl->fast)
+        return fail("sb_plan_set_nodata: the nodata mask needs the pipelined kernels (option fast = 1)");
+    pl->nodata_req = mode;
+    pl->min_cov_req = min_coverage;
+    return 0;
 }
 
 int sb_plan_set_slab(sb_plan* pl, int row_lo, int row_hi, int halo) {
@@ -1163,7 +1278,8 @@ long sb_plan_device_bytes(const sb_plan* pl) {
     if (pl->d_diffs32) b += n * sizeof(float4);
     b += (size_t)pl->bn() * pl->n_states * pl->best_copies * 12;
     for (const Buf* q : {&pl->cr, &pl->fct, &pl->trt, &pl->part, &pl->gbuf, &pl->sums, &pl->fit, &pl->tmpls, &pl->angles,
-                         &pl->tables, &pl->raw, &pl->tbox, &pl->slots, &pl->cross, &pl->casa, &pl->aux, &pl->spec9, &pl->coef})
+                         &pl->tables, &pl->raw, &pl->tbox, &pl->slots, &pl->cross, &pl->casa, &pl->aux, &pl->spec9, &pl->coef,
+                         &pl->fitm})
         b += q->cap;
     return (long)b;
 }
@@ -1260,6 +1376,8 @@ int sb_render_template(sb_plan* pl, const sb_template* tmpl, double* out, int ou
 int sb_match_template(sb_plan* pl, const sb_angle* angle, const sb_template* tmpl, double* amp, double* snr,
                       int out_is_device) {
     if (!pl || !angle || !tmpl || !amp || !snr) return fail("sb_match_template: null");
+    if (pl->nodata == SB_NODATA_MASK || pl->nodata_req == SB_NODATA_MASK)
+        return fail("nodata mask: sb_match_template keeps the reference's NaN semantics");
     const size_t n = (size_t)pl->ny * pl->nx;
     SweepOut so;
     if (out_is_device) {

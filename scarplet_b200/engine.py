@@ -44,11 +44,13 @@ class Plan(object):
     """One raster geometry bound to one CUDA device."""
 
     def __init__(self, ny, nx, dx, dy, device=-1, stream=None, workspace_mb=None,
-                 max_fft=None, force_pad=None, precision=None, slab=None, states=1):
+                 max_fft=None, force_pad=None, precision=None, slab=None, states=1,
+                 nodata="propagate", min_coverage=1.0):
         """``slab=(row_lo, row_hi, halo)``: the plan keeps the geometry of the whole ``ny x nx``
         raster but computes (and holds the DEM for) that band of rows only -- one rank's share
         of a raster sharded spatially over GPUs.  ``states``: independent best states (one per
-        template scale of a multi-scale search)."""
+        template scale of a multi-scale search).  ``nodata``, ``min_coverage``: see
+        ``set_nodata``."""
         self.lib = _lib.load()
         self.ny, self.nx = int(ny), int(nx)
         self.dx, self.dy = dx, dy
@@ -78,6 +80,9 @@ class Plan(object):
             self.set_states(states)
         if slab is not None:
             self.set_slab(*slab)
+        self.nodata, self.min_coverage = "propagate", 1.0
+        if nodata != "propagate" or min_coverage != 1.0:
+            self.set_nodata(nodata, min_coverage)
 
     # -- lifecycle ---------------------------------------------------------
     def close(self):
@@ -100,6 +105,23 @@ class Plan(object):
 
     def set_option(self, key, value):
         check(self.lib, self.lib.sb_plan_set_option(self._h, key.encode(), int(value)))
+
+    NODATA_MODES = {"propagate": 0, "mask": 1}      # SB_NODATA_PROPAGATE, SB_NODATA_MASK
+
+    def set_nodata(self, mode="propagate", min_coverage=1.0):
+        """Nodata policy of the searches; takes effect at the next ``set_dem``.
+
+        ``"propagate"`` (default): the reference's semantics, a NaN anywhere in the DEM makes
+        every un-masked pixel NaN.  ``"mask"``: each fit uses only the template cells whose
+        curvature is defined (every DEM cell of its stencil finite); a template counts at a pixel
+        when those cells are at least ``min_coverage`` (in (0, 1]) of its support, and a pixel
+        whose own cell is nodata gets no result.  With ``min_coverage=1`` the values equal the
+        reference's on the DEM with its holes filled by anything.  Masked plans need
+        precision 32; ``match_template`` keeps the reference's semantics and refuses them."""
+        if mode not in Plan.NODATA_MODES:
+            raise ValueError("nodata must be 'propagate' or 'mask', not %r" % (mode,))
+        check(self.lib, self.lib.sb_plan_set_nodata(self._h, Plan.NODATA_MODES[mode], float(min_coverage)))
+        self.nodata, self.min_coverage = mode, float(min_coverage)
 
     def set_states(self, n):
         """Number of independent best states (resets them)."""
