@@ -78,10 +78,11 @@ int sb_plan_destroy(sb_plan* plan);
  * "precision" (32 = complex64 pipeline, default; 64 = complex128 pipeline),
  * "states" (number of independent best states, default 1; resets them),
  * and the kernel-selection switches, all on by default (off = the slower variant, same results
- * to rounding): "fast" (pipelined complex64 kernels), "conv_persist" (persistent column kernel:
- * minimum templates per orientation run, 0 = never), "conv_r64" (radix-64 column kernel at
- * Py = 4096), "lincomb" (curvature spectra as combinations of nine plane spectra),
- * "fit_substreams" (0 = automatic, 1..8 = sub-streams of the row kernel on small rasters)};
+ * to rounding): "fast" (pipelined complex64 kernels; the curvature spectra of every orientation
+ * are combinations of nine plane spectra computed once per FFT tile), "conv_persist" (persistent
+ * column kernel: minimum templates per orientation run, 0 = never), "conv_r64" (radix-64 column
+ * kernel at Py = 4096), "fit_substreams" (0 = automatic, 1..8 = sub-streams of the row kernel on
+ * small rasters)};
  * returns 0 if known */
 int sb_plan_set_option(sb_plan* plan, const char* key, long value);
 
@@ -96,7 +97,7 @@ int sb_plan_set_option(sb_plan* plan, const char* key, long value);
  *     not finite gets no result (0 in all four planes).  With min_coverage = 1 every value equals
  *     the reference's on the same DEM with its holes filled by any values.
  * Fails for min_coverage outside (0, 1] and, for SB_NODATA_MASK, unless the plan runs the complex64
- * pipelined kernels (precision 32, fast = 1, lincomb = 1); sb_match_template and
+ * pipelined kernels (precision 32, fast = 1); sb_match_template and
  * sb_match_template_raster fail on a masked plan.  FFT tiles of a masked sweep are at most 4096. */
 enum { SB_NODATA_PROPAGATE = 0, SB_NODATA_MASK = 1 };
 int sb_plan_set_nodata(sb_plan* plan, int mode, double min_coverage);

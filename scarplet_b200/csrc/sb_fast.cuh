@@ -27,15 +27,6 @@ using std::max;
 using std::min;
 #endif
 
-// Developer ablation switches (scratch/ablate.sh): build with -DSB_ABLATE and set SB_DBG to
-// switch parts of the kernels' memory traffic off and time what is left.  Compiled out of
-// the product build.
-#ifdef SB_ABLATE
-#define SB_DBG_ON(flags, bit) (((flags) & (bit)) != 0)
-#else
-#define SB_DBG_ON(flags, bit) false
-#endif
-
 SB_CONSTEXPR int ilog2(int n) { return n <= 1 ? 0 : 1 + ilog2(n / 2); }
 
 // ---------------------------------------------------------------------------
@@ -100,25 +91,18 @@ struct ConvCtx {
     const float2 *specA, *specB;      // curvature-spectrum columns of the two fields (+ t)
     float4* dst;                      // gbuf plane of this template (nullptr: inactive group)
     int kx, dly, out_ny, kpitch;
-    int dbg;
     int bar_id;                       // PERSIST: named barrier of this thread group
-    const float2* va_fin;             // SB_CONV_KEEP_A: field a's registers (the array handed to leapfrog)
+    // field a's result waits in its registers (the array handed to leapfrog) for field b
+    // (parking it in shared memory instead: +2 %)
+    const float2* va_fin;
 
     SB_DEVICE void bar() const {
-#ifdef SB_ABL_NOBAR
-        return;
-#endif
         if constexpr (PERSIST) sb_bar(bar_id, T);
         else sb_sync();
     }
     SB_CONSTEXPR static int stage_of(int P) { return P < NST ? P : P - NST + 1; }
 
     template <int P> SB_DEVICE void twid(float2 (&w)[TW]) {
-        if (SB_DBG_ON(dbg, 4)) {
-#pragma unroll
-            for (int i = 0; i < TW; ++i) w[i] = make_float2(0.6f, 0.8f);
-            return;
-        }
         sbfft::load_tw<N, stage_of(P), float, PERSIST>(w, t, tw);   // PERSIST: the CTA's shared-memory copy
     }
 
@@ -129,22 +113,12 @@ struct ConvCtx {
             const float2* spec = F == 0 ? specA : specB;
 #pragma unroll
             for (int q = 0; q < E; ++q) {
-                const float2 s = SB_DBG_ON(dbg, 2) ? make_float2(0.5f, 0.25f)
-                                 : PERSIST ? spec[q * T] : sb_ld_stream(spec + q * T);
+                const float2 s = PERSIST ? spec[q * T] : sb_ld_stream(spec + q * T);
                 const float2 pr = sbfft::cmul(v[q], s);
                 v[q] = make_float2(pr.y, pr.x);                  // swap: inverse via forward
             }
             sbfft::stage_math<N, 0, float>(v, w);
         }
-#define SB_CONV_KEEP_A 1    // field a's result waits in registers for field b (parking it in shared memory: +2 %)
-#ifndef SB_CONV_KEEP_A
-        if constexpr (P == K - 1 && F == 0) {
-            // field a is done; park it in its own (now idle) exchange buffer, every thread in
-            // the slots only it will read back, so that its registers are free for field b
-#pragma unroll
-            for (int q = 0; q < E; ++q) smA[t + q * T] = v[q];
-        }
-#endif
         if constexpr (P == K - 1 && F == 1) {
             if (dst) {
                 // row m = t + q T lies at gbuf_index(t, kx) + q * T * kpitch (T is even): one pointer,
@@ -155,17 +129,8 @@ struct ConvCtx {
                 const int io0 = t + dly;
 #pragma unroll
                 for (int q = 0; q < E; ++q) {
-#ifdef SB_CONV_KEEP_A
                     const float2 a = va_fin[q];      // field a's result, still in the caller's registers
-#else
-                    const float2 a = smA[t + q * T];
-#endif
-                    if (SB_DBG_ON(dbg, 1) && v[q].x != 1.2345e-30f) continue;
                     const float4 out = gbuf_pack<float2, float4>(a, v[q]);
-                    if (SB_DBG_ON(dbg, 128)) {      // timing only: same bytes, fully coalesced
-                        sb_st_stream(dst + ((long)kx * N + t + q * T), out);
-                        continue;
-                    }
                     if (((io0 + q * T) & (N - 1)) < out_ny) sb_st_stream(p, out);
                     p += step;
                 }
@@ -174,17 +139,9 @@ struct ConvCtx {
     }
     template <int P, int F> SB_DEVICE void store(const float2 (&v)[E]) {
         constexpr int S = (P == NST - 1) ? 0 : stage_of(P);
-#ifdef SB_ABL_NOXCHG
-        if (v[0].x != 1.2345e-30f) return;
-#endif
         sbfft::stage_store<N, S, float>(v, t, F == 0 ? smA : smB);
     }
-    template <int F> SB_DEVICE void load(float2 (&v)[E]) {
-#ifdef SB_ABL_NOXCHG
-        if (t >= 0) return;
-#endif
-        sbfft::stage_load<N, float>(v, t, F == 0 ? smA : smB);
-    }
+    template <int F> SB_DEVICE void load(float2 (&v)[E]) { sbfft::stage_load<N, float>(v, t, F == 0 ? smA : smB); }
 };
 
 template <int N, bool SPARSE>
@@ -217,7 +174,6 @@ k_conv_cols_f(Geom g, const Tmpl* SB_RESTRICT tmpls, int tmpl_base, int angle_ba
     c.dly = g.dly;
     c.out_ny = g.out_ny;
     c.kpitch = g.kpitch;
-    c.dbg = g.dbg;
     // one 128-byte line of each spectrum column per thread (T lines per column)
     sb_prefetch_l2(c.specA + 15 * t);
     sb_prefetch_l2(c.specB + 15 * t);
@@ -232,7 +188,7 @@ k_conv_cols_f(Geom g, const Tmpl* SB_RESTRICT tmpls, int tmpl_base, int angle_ba
         const int qy = t + q * T;
         const int s = qy < N / 2 ? qy : qy - N;
         if (active && s >= sy_lo && s <= sy_hi) {
-            const float4 w = SB_DBG_ON(g.dbg, 8) ? make_float4(1.f, 2.f, 3.f, 4.f) : sb_ld_stream(src + (s - sy_lo));
+            const float4 w = sb_ld_stream(src + (s - sy_lo));
             va[q] = make_float2(w.x, w.y);
             vb[q] = make_float2(w.z, w.w);
         }
@@ -291,7 +247,6 @@ k_conv_cols_p(Geom g, const Tmpl* SB_RESTRICT tmpls, int tmpl_base, int cnt, int
     c.dly = g.dly;
     c.out_ny = g.out_ny;
     c.kpitch = g.kpitch;
-    c.dbg = g.dbg;
     c.bar_id = 1 + grp;
     sb_sync();
 
@@ -355,9 +310,6 @@ k_conv_cols_p(Geom g, const Tmpl* SB_RESTRICT tmpls, int tmpl_base, int cnt, int
             }
             c.va_fin = va;
             leapfrog<Ctx::K>(c, va, vb);                    // the last phase of field b writes gbuf
-#ifndef SB_CONV_KEEP_A
-            c.bar();                                        // parked field a has been read back
-#endif
         }
         s0 = s1;
     }
@@ -480,7 +432,6 @@ struct FitPairCtx {
     int* best_idx;
     const int4* cross;                // get_err_mask column ranges per (angle, raster row), or null
     int ny;
-    int dbg;
     float (&bsA)[E];
     float (&bsB)[E];
     float2 (&vb_in)[E];               // stream b's input, filled together with stream a's
@@ -608,8 +559,7 @@ struct FitPairCtx {
                 int kk = q < E / 2 ? t + q * T : N - (t + q * T);
                 if (q == E / 2) { direct = t == 0; kk = direct ? N / 2 : N / 2 - t; }
                 float4 ga, gb;
-                if (SB_DBG_ON(dbg, 16)) { ga = make_float4(1.f, 2.f, 3.f, (float)q); gb = ga; }
-                else sb_ld_sector(pair + kGbufRows * kk, ga, gb);
+                sb_ld_sector(pair + kGbufRows * kk, ga, gb);
                 v[q] = herm(ga, direct);
                 vb_in[q] = herm(gb, direct);
             }
@@ -618,7 +568,6 @@ struct FitPairCtx {
         if constexpr (P == K - 1 && SOA) {
             sbfft::pk_t re[8], im[8];
             sbfft::stage_math_soa<N, P>(v, w, re, im);
-            if (SB_DBG_ON(dbg, 64) && v[0].x != 1.2345e-30f) return;
             if constexpr (F == 0) epilogue2<0>(re, im, bsA);
             else epilogue2<1>(re, im, bsB);
             return;
@@ -626,7 +575,6 @@ struct FitPairCtx {
 #endif
         sbfft::stage_math<N, P, float>(v, w);
         if constexpr (P == K - 1) {
-            if (SB_DBG_ON(dbg, 64) && v[0].x != 1.2345e-30f) return;
             if constexpr (MASKED) {
                 if (comp) {
 #pragma unroll
@@ -735,7 +683,6 @@ SB_DEVICE void fit_rows_g_body(const Geom& g, int count, const int* SB_RESTRICT 
     c.s_fm = s_fm;
     c.park = park;
     c.comp = false;
-    c.dbg = g.dbg;
     best_snr += sb_by() * sub_stride;
     best_amp += sb_by() * sub_stride;
     best_idx += sb_by() * sub_stride;
@@ -809,60 +756,6 @@ k_fit_rows_gm(Geom g, int count, const int* SB_RESTRICT slots, const FitT* SB_RE
                              sub_stride);
 }
 
-// ---------------------------------------------------------------------------
-// k_curv_rows_f<Px>: pipelined k_curv_rows (complex64): the two rows of a pair are the two
-// transforms a thread group carries (one barrier per exchange); grid and layouts as k_curv_rows.
-// ---------------------------------------------------------------------------
-template <int N>
-struct CurvCtx {
-    static constexpr int K = sbfft::num_stages(N);
-    static constexpr int T = N / E;
-    int t;
-    float2 *smA, *smB;
-    const float2* tw;
-    const float4* diffs;               // [pixel][dxx, dxy, dyy, -] float32
-    float ca2, sc2, sa2;               // cos**2, 2 sin cos, sin**2 of the search angle
-    int oy, ox, ny, nx, need_y_lo, need_x_lo, need_x_hi, split_x, poison, dbg;
-    int row0;                          // global raster row of row 0 of `diffs` (row slab; 0 for a whole raster)
-    float c2_scale;
-    int rp;                            // row pair: rows 2 rp (stream a) and 2 rp + 1 (stream b)
-    int need_rows;
-
-    SB_DEVICE void bar() const { sb_sync(); }
-    template <int P> SB_DEVICE void twid(float2 (&w)[TW]) { sbfft::load_tw<N, P, float>(w, t, tw); }
-
-    template <int F> SB_DEVICE void fill(float2 (&v)[E]) const {
-        const int r = 2 * rp + F;
-        const bool active = r < need_rows;
-        int gi = wrap(oy + need_y_lo + (active ? r : 0), ny) - row0;
-        gi += gi < 0 ? ny : 0;                   // row of the slab
-#pragma unroll
-        for (int q = 0; q < E; ++q) {
-            const int qx = t + q * T;
-            const int sx = qx < split_x ? qx : qx - N;
-            float2 val = make_float2(0.f, 0.f);
-            if (active && sx >= need_x_lo && sx <= need_x_hi) {
-                const int gj = wrap_near(ox + sx, nx);
-                const long o = (long)gi * nx + gj;
-                // dem.py:103-104 on the float32 second differences: the transform rounds the
-                // curvature to float32 anyway, and one 16-byte load replaces three 8-byte ones
-                const float4 d = SB_DBG_ON(dbg, 256) ? make_float4((float)o * 1e-9f, 1.f, 2.f, 0.f) : sb_ldg(diffs + o);
-                const float c = (d.x * ca2 - d.y * sc2) + d.z * sa2;
-                val = make_float2(c, c * c * c2_scale);                    // curv, curv**2 (core.py:355)
-            }
-            if (poison && r == 0 && qx == 0) val = make_float2(NAN, NAN);
-            v[q] = val;
-        }
-    }
-    template <int P, int F> SB_DEVICE void phase(float2 (&v)[E], const float2 (&w)[TW]) {
-        sbfft::stage_math<N, P, float>(v, w);       // both rows are filled before the pipeline starts
-    }
-    template <int P, int F> SB_DEVICE void store(const float2 (&v)[E]) {
-        sbfft::stage_store<N, P, float>(v, t, F == 0 ? smA : smB);
-    }
-    template <int F> SB_DEVICE void load(float2 (&v)[E]) { sbfft::stage_load<N, float>(v, t, F == 0 ? smA : smB); }
-};
-
 // Hermitian split (sb_kernels.cuh) of the spectrum parked in natural order in `sm`
 template <int N>
 SB_DEVICE void split_from_shared(const float2* sm, int t, float4 (&h)[E / 2 + 1]) {
@@ -876,52 +769,6 @@ SB_DEVICE void split_from_shared(const float2* sm, int t, float4 (&h)[E / 2 + 1]
     }
     const float2 ny = sm[sbfft::pad_index(N / 2)];
     h[E / 2] = make_float4(ny.x, 0.f, ny.y, 0.f);
-}
-
-template <int N>
-SB_GLOBAL SB_LAUNCH_BOUNDS((N / E > 256 ? N / E : 256), (N / E > 256 ? 1 : 2))
-k_curv_rows_f(Geom g, const float4* SB_RESTRICT diffs, const Angle* SB_RESTRICT angles, int angle_base,
-              float4* SB_RESTRICT cr, const float2* SB_RESTRICT tw) {
-    constexpr int T = N / E;
-    constexpr int GP = (T > 256 ? T : 256) / T;
-    constexpr int PL = sbfft::padded_len(N);
-    const int grp = sb_tid() / T, t = sb_tid() % T;
-    const int KX = N / 2 + 1;
-    const int a_loc = sb_bx();
-    CurvCtx<N> c;
-    c.t = t;
-    c.smA = (float2*)sb_shared() + (long)grp * 2 * PL;
-    c.smB = c.smA + PL;
-    c.tw = tw;
-    c.diffs = diffs;
-    c.oy = g.oy; c.ox = g.ox; c.ny = g.ny; c.nx = g.nx;
-    c.need_y_lo = g.need_y_lo; c.need_x_lo = g.need_x_lo; c.need_x_hi = g.need_x_hi;
-    c.split_x = g.split_x; c.poison = g.poison; c.c2_scale = (float)g.c2_scale; c.dbg = g.dbg;
-    c.row0 = g.row0;
-    {
-        const Angle ang = angles[angle_base + a_loc];
-        c.ca2 = (float)ang.ca2;
-        c.sc2 = (float)(2.0 * ang.sa * ang.ca);
-        c.sa2 = (float)ang.sa2;
-    }
-    c.rp = sb_by() * GP + grp;
-    c.need_rows = g.need_y_hi - g.need_y_lo + 1;
-    float2 va[E], vb[E];
-    c.template fill<0>(va);                     // all 32 loads of the pair in flight together
-    c.template fill<1>(vb);
-    leapfrog<CurvCtx<N>::K>(c, va, vb);
-    sb_sync();                                  // every thread is done with the exchange buffers
-#pragma unroll
-    for (int q = 0; q < E; ++q) {
-        c.smA[sbfft::pad_index(t + q * T)] = va[q];
-        c.smB[sbfft::pad_index(t + q * T)] = vb[q];
-    }
-    sb_sync();
-    float4 h0[E / 2 + 1], h1[E / 2 + 1];
-    split_from_shared<N>(c.smA, t, h0);
-    split_from_shared<N>(c.smB, t, h1);
-    if (2 * c.rp < c.need_rows)
-        store_row_pair<N, float>(h0, h1, t, cr + (long)a_loc * KX * g.rpitch + 2 * c.rp, g.rpitch);
 }
 
 // ---------------------------------------------------------------------------
@@ -998,7 +845,7 @@ struct DiffCtx {
     template <int F> SB_DEVICE void load(float2 (&v)[E]) { sbfft::stage_load<N, float>(v, t, F == 0 ? smA : smB); }
 };
 
-// grid (kDiffPairs, ceil(need_rows / 2 / GP)); output layout as k_curv_rows_f with the plane
+// grid (kDiffPairs, ceil(need_rows / 2 / GP)); output layout as k_curv_rows with the plane
 // pair in the place of the orientation: cr[pp][kx][rpitch rows] float4
 template <int N, bool WITH_U>
 SB_DEVICE void diff_rows_body(const Geom& g, const float4* SB_RESTRICT diffs, float4* SB_RESTRICT cr,

@@ -81,7 +81,7 @@ template <typename C> SB_DEVICE C mul_mi(C a) { C r; r.x = a.y; r.y = -a.x; retu
 // instead of 2, a complex multiply 2 instead of 4, and multiplying by -i is free.  The
 // butterflies below are written against these helpers; the emulator build and complex128
 // use the scalar forms above.
-#if !defined(SB_EMU) && !defined(SB_NO_F32X2)
+#ifndef SB_EMU
 #define SB_F32X2 1
 typedef unsigned long long pk_t;
 SB_DEVICE pk_t pk(float lo, float hi) { pk_t r; asm("mov.b64 %0, {%1, %2};" : "=l"(r) : "f"(lo), "f"(hi)); return r; }
@@ -262,7 +262,7 @@ constexpr int TW = E - 1;    // twiddle registers a thread needs for one stage (
 // and 18 fewer registers are live across the barrier that follows the fetch.
 template <typename R, int RADIX>
 SB_CONSTEXPR bool tw_derived(int u) {
-#if defined(SB_F32X2) && !defined(SB_NO_TW_DIET)
+#ifdef SB_F32X2
     return sizeof(R) == 4 && RADIX == 16 && !(u <= 4 || u == 8 || u == 12);
 #else
     return false;
@@ -333,9 +333,6 @@ SB_DEVICE void stage_math(typename Vec<R>::v2 (&v)[E], const typename Vec<R>::v2
     typedef typename Vec<R>::v2 C;
     constexpr int RADIX = stage_radix(N, S);
     constexpr int B = E / RADIX;
-#ifdef SB_ABL_NOMATH
-    if (v[0].x != 1.2345e-30f) return;
-#endif
 #pragma unroll
     for (int m = 0; m < B; ++m) {
         C x[RADIX];

@@ -18,10 +18,6 @@
 #pragma once
 #include "sb_fft.cuh"
 
-#ifndef SB_CONV_BLOCKS
-#define SB_CONV_BLOCKS 3     // resident CTAs per SM targeted by k_conv_cols (complex64)
-#endif
-
 namespace sb {
 
 using sbfft::E;
@@ -44,7 +40,6 @@ struct Geom {
     double dx, dx2, dy2;     // cell size, dx**2, dy**2 as the host computes them
     double norm;             // 1 / (Px * Py)
     double c2_scale;         // power of two: curv**2 is packed as curv**2 * c2_scale next to curv
-    int dbg;                 // developer ablation switches (SB_DBG; builds with -DSB_ABLATE only), else 0
     int poison;              // the DEM holds a NaN: every FFT domain gets one (the reference's fft2 spans the raster)
     // Row slab (spatial sharding over GPUs, SURVEY 8e): the buffers derived from the DEM hold the
     // `drows` raster rows starting at global row `row0` (periodic in ny), the best state holds
@@ -113,10 +108,7 @@ struct FitT {
 // store fills whole 32-byte sectors (a 16-byte half-sector store runs at 0.9 TB/s on
 // B200, a full-sector one at 4.7 TB/s: scratch/ubench_scatter.cu); the row kernel reads
 // its row at a 32-byte stride.
-#ifndef SB_GBUF_ROWS
-#define SB_GBUF_ROWS 2
-#endif
-constexpr int kGbufRows = SB_GBUF_ROWS;      // rows interleaved per spectrum column (power of two, even)
+constexpr int kGbufRows = 2;      // rows interleaved per spectrum column (power of two, even)
 // a, b: the two fields' inverse-column results as the transforms leave them (swapped: (im, re))
 template <typename C2, typename C4>
 SB_DEVICE C4 gbuf_pack(const C2 a, const C2 b) {
@@ -670,8 +662,9 @@ SB_GLOBAL k_tmpl_sums(Geom g, const Tmpl* SB_RESTRICT tmpls, int tmpl_base, int 
 // field's result waits in the park buffer (each thread re-reads only what it wrote, so no
 // barrier) until the second is done, and both leave in one 16-byte store.
 // ---------------------------------------------------------------------------
+// complex64 below 4096 targets three resident CTAs per SM
 template <int N, typename R>
-SB_GLOBAL SB_LAUNCH_BOUNDS((N / E > 256 ? N / E : 256), ((N / E > 256 || sizeof(R) == 8) ? 1 : SB_CONV_BLOCKS))
+SB_GLOBAL SB_LAUNCH_BOUNDS((N / E > 256 ? N / E : 256), ((N / E > 256 || sizeof(R) == 8) ? 1 : 3))
 k_conv_cols(Geom g, const Tmpl* SB_RESTRICT tmpls, int tmpl_base, int angle_base,
             const typename Vec<R>::v4* SB_RESTRICT trt, const typename Vec<R>::v2* SB_RESTRICT fct,
             typename Vec<R>::v4* SB_RESTRICT gbuf, const typename Vec<R>::v2* SB_RESTRICT tw) {

@@ -94,7 +94,7 @@ struct sb_plan {
     float* d_bsnr = nullptr;        // [best_copies][n_states][slab rows][nx]; copy 0 is the state
     float* d_bamp = nullptr;
     int* d_bidx = nullptr;
-    std::map<long, void*> tw;      // twiddle tables keyed by 2 * n + (float64 ? 1 : 0)
+    std::map<long, void*> tw;      // twiddle tables keyed by 2 * n + (float64 ? 1 : 0); -64: radix-64 core
     int precision = 32;            // 32: complex64 pipeline, 64: complex128 pipeline
     Buf cr, fct, trt, part, gbuf, sums, fit, tmpls, angles, tables, raw, tbox, slots, cross, casa, aux, spec9, coef;
     int fit_substreams = 0;        // 0: automatic (small rasters), else the number of sub-streams of the fit kernel
@@ -104,9 +104,6 @@ struct sb_plan {
     // the spectrum columns is not amortised (C2: 94 ms persistent, 69 ms per-template)
     int conv_persist = -1;
     int conv_r64 = 1;              // Py = 4096: column kernel on the radix-64 core (sb_r64.cuh)
-    // 1: the curvature spectra of an orientation are combinations of nine spectra computed once per
-    // FFT tile (k_diff_rows_f / k_combine_spectra); 0: one row + one column transform per orientation
-    int lincomb = 1;
     long launches = 0;
     double c2_scale = 1.0;
     double curv_sumsq = 0.0, curv_count = 0.0;   // over the plan's own rows (slab_lo .. slab_hi)
@@ -116,7 +113,6 @@ struct sb_plan {
     double min_cov_req = 1.0, min_cov = 1.0;
     Buf fitm;
     int profile = 0;
-    int dbg = 0;                   // ablation switches (-DSB_ABLATE builds only)
     std::vector<sb_event_t> ev_pool;
     struct EvPair { int kind; sb_event_t a, b; };
     std::vector<EvPair> ev_live;
@@ -153,15 +149,25 @@ void release(Buf& b) {
     b.cap = 0;
 }
 
+// a table of `count` elements in pl->tw under `key`: filled on the host and uploaded on first use
+template <typename C, typename Fill>
+int cached_table(sb_plan* pl, long key, size_t count, Fill fill, const C** out) {
+    auto it = pl->tw.find(key);
+    if (it == pl->tw.end()) {
+        std::vector<C> host(count);
+        fill(host.data());
+        void* d = nullptr;
+        SB_TRY(sb_rt_malloc(&d, count * sizeof(C)));
+        SB_TRY(sb_rt_h2d(d, host.data(), count * sizeof(C), pl->stream));
+        SB_TRY(sb_rt_sync(pl->stream));
+        it = pl->tw.emplace(key, d).first;
+    }
+    *out = (const C*)it->second;
+    return 0;
+}
+
 template <typename R>
 int twiddles(sb_plan* pl, int n, const typename Vec<R>::v2** out) {
-    typedef typename Vec<R>::v2 C2;
-    const long key = 2L * n + (sizeof(R) == 8 ? 1 : 0);
-    auto it = pl->tw.find(key);
-    if (it != pl->tw.end()) {
-        *out = (const C2*)it->second;
-        return 0;
-    }
     int count = 0;
     {   // same stage walk as sbfft::fill_twiddles
         int ns = 1;
@@ -171,30 +177,13 @@ int twiddles(sb_plan* pl, int n, const typename Vec<R>::v2** out) {
             ns *= r;
         }
     }
-    std::vector<C2> host(std::max(count, 1));
-    sbfft::fill_twiddles<R>(n, host.data());
-    void* d = nullptr;
-    SB_TRY(sb_rt_malloc(&d, host.size() * sizeof(C2)));
-    SB_TRY(sb_rt_h2d(d, host.data(), host.size() * sizeof(C2), pl->stream));
-    SB_TRY(sb_rt_sync(pl->stream));
-    pl->tw[key] = d;
-    *out = (const C2*)d;
-    return 0;
+    return cached_table(pl, 2L * n + (sizeof(R) == 8 ? 1 : 0), std::max(count, 1),
+                        [n](typename Vec<R>::v2* h) { sbfft::fill_twiddles<R>(n, h); }, out);
 }
 
-// table of the radix-64 core (sb_r64.cuh), key -64
+// table of the radix-64 core (sb_r64.cuh)
 int twiddles64(sb_plan* pl, const float2** out) {
-    auto it = pl->tw.find(-64);
-    if (it != pl->tw.end()) { *out = (const float2*)it->second; return 0; }
-    std::vector<float2> host((size_t)sb64::kTwRows * sb64::R);
-    sb64::fill_twiddles64(host.data());
-    void* d = nullptr;
-    SB_TRY(sb_rt_malloc(&d, host.size() * sizeof(float2)));
-    SB_TRY(sb_rt_h2d(d, host.data(), host.size() * sizeof(float2), pl->stream));
-    SB_TRY(sb_rt_sync(pl->stream));
-    pl->tw[-64] = d;
-    *out = (const float2*)d;
-    return 0;
+    return cached_table(pl, -64, (size_t)sb64::kTwRows * sb64::R, sb64::fill_twiddles64, out);
 }
 
 template <typename F>
@@ -233,21 +222,18 @@ struct Shape {
                                          (size_t)sbfft::ctw_count<float>(N) * sizeof(float2);
 };
 
+// Every kernel launch of the library: a kernel that asks for more than the default 48 KB of
+// dynamic shared memory is allowed it first, then it runs on the plan's stream; the launch is
+// counted (sb_plan_launch_count) and checked.
+template <typename... P, typename... A>
+int launch(sb_plan* pl, const char* what, void (*kern)(P...), dim3 grid, dim3 block, size_t smem, A... args) {
 #ifndef SB_EMU
-template <typename K>
-int allow_smem(K kernel, size_t bytes) {
-    if (bytes > 48 * 1024)
-        SB_TRY((int)cudaFuncSetAttribute(kernel, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)bytes));
-    return 0;
-}
-#define SB_ALLOW_SMEM(kern, bytes) SB_OK(allow_smem(kern, bytes))
-#else
-#define SB_ALLOW_SMEM(kern, bytes)
+    if (smem > 48 * 1024)
+        SB_TRY((int)cudaFuncSetAttribute(kern, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem));
 #endif
-
-int check_launch(sb_plan* pl, const char* what) {
+    SB_LAUNCH(kern, grid, block, smem, pl->stream, args...);
     pl->launches++;
-    int e = sb_rt_last_error();
+    const int e = sb_rt_last_error();
     if (e != 0) return fail(std::string(what) + ": " + sb_rt_error_string(e));
     return 0;
 }
@@ -329,13 +315,13 @@ int after_dem(sb_plan* pl) {
     pl->min_cov = pl->min_cov_req;
     const bool masked = pl->nodata == SB_NODATA_MASK;
     if (masked) {
-        SB_LAUNCH(sb::k_second_differences_m, dim3(div_up(n, 256)), dim3(256), 0, pl->stream, pl->ny, pl->nx, pl->row0,
-                  pl->drows, (const double*)pl->d_dem, pl->dx, pl->dx2, pl->dy2, pl->d_diffs32);
-        SB_OK(check_launch(pl, "k_second_differences_m"));
+        SB_OK(launch(pl, "k_second_differences_m", sb::k_second_differences_m, dim3(div_up(n, 256)), dim3(256), 0,
+                     pl->ny, pl->nx, pl->row0, pl->drows, (const double*)pl->d_dem, pl->dx, pl->dx2, pl->dy2,
+                     pl->d_diffs32));
     } else {
-        SB_LAUNCH(sb::k_second_differences, dim3(div_up(n, 256)), dim3(256), 0, pl->stream, pl->ny, pl->nx, pl->row0,
-                  pl->drows, (const double*)pl->d_dem, pl->dx, pl->dx2, pl->dy2, (double*)nullptr, pl->d_diffs32);
-        SB_OK(check_launch(pl, "k_second_differences"));
+        SB_OK(launch(pl, "k_second_differences", sb::k_second_differences, dim3(div_up(n, 256)), dim3(256), 0, pl->ny,
+                     pl->nx, pl->row0, pl->drows, (const double*)pl->d_dem, pl->dx, pl->dx2, pl->dy2, (double*)nullptr,
+                     pl->d_diffs32));
     }
     // statistics over the plan's own rows only, so that the slabs of a sharded raster add up
     const int own_first = pl->slab_lo - pl->row0 + (pl->slab_lo < pl->row0 ? pl->ny : 0);
@@ -343,10 +329,9 @@ int after_dem(sb_plan* pl) {
     const int blocks = std::max(1, std::min(1024, div_up(own, 256)));
     SB_OK(ensure(pl->raw, (size_t)blocks * sizeof(double)));
     auto sumsq_kern = masked ? sb::k_curv_sumsq_m : sb::k_curv_sumsq;
-    SB_LAUNCH(sumsq_kern, dim3(blocks), dim3(256), 256 * sizeof(double), pl->stream, pl->ny, pl->nx, pl->row0,
-              pl->drows, own_first, (int)pl->brows(), (const double*)pl->d_dem, pl->dx, pl->dx2, pl->dy2,
-              (double*)pl->raw.p);
-    SB_OK(check_launch(pl, "k_curv_sumsq"));
+    SB_OK(launch(pl, "k_curv_sumsq", sumsq_kern, dim3(blocks), dim3(256), 256 * sizeof(double), pl->ny, pl->nx,
+                 pl->row0, pl->drows, own_first, (int)pl->brows(), (const double*)pl->d_dem, pl->dx, pl->dx2, pl->dy2,
+                 (double*)pl->raw.p));
     std::vector<double> part(blocks);
     SB_TRY(sb_rt_d2h(part.data(), pl->raw.p, (size_t)blocks * sizeof(double), pl->stream));
     SB_TRY(sb_rt_sync(pl->stream));
@@ -362,9 +347,9 @@ int ensure_diffs64(sb_plan* pl) {
     if (pl->diffs64_valid) return 0;
     const long n = (long)pl->drows * pl->nx;
     if (!pl->d_diffs) SB_TRY(sb_rt_malloc((void**)&pl->d_diffs, (size_t)n * 3 * sizeof(double)));
-    SB_LAUNCH(sb::k_second_differences, dim3(div_up(n, 256)), dim3(256), 0, pl->stream, pl->ny, pl->nx, pl->row0,
-              pl->drows, (const double*)pl->d_dem, pl->dx, pl->dx2, pl->dy2, pl->d_diffs, (float4*)nullptr);
-    SB_OK(check_launch(pl, "k_second_differences"));
+    SB_OK(launch(pl, "k_second_differences", sb::k_second_differences, dim3(div_up(n, 256)), dim3(256), 0, pl->ny,
+                 pl->nx, pl->row0, pl->drows, (const double*)pl->d_dem, pl->dx, pl->dx2, pl->dy2, pl->d_diffs,
+                 (float4*)nullptr));
     pl->diffs64_valid = true;
     return 0;
 }
@@ -520,11 +505,10 @@ int run_sweep_t(sb_plan* pl, const sb_angle* angles, int n_angles, const sb_temp
     if (so.raw_amp && !pl->whole()) return fail("match_template planes need a plan over the whole raster");
     constexpr bool kF32 = std::is_same<R, float>::value;
     const bool fast = kF32 && pl->fast;
-    // nodata-masked search: complex64 pipelined kernels with the linear-combination set-up only
+    // nodata-masked search: complex64 pipelined kernels only
     const bool masked = pl->nodata == SB_NODATA_MASK;
     if (masked && so.raw_amp) return fail("nodata mask: sb_match_template keeps the reference's NaN semantics");
-    if (masked && !(fast && pl->lincomb))
-        return fail("nodata mask needs precision 32 and the options fast and lincomb");
+    if (masked && !fast) return fail("nodata mask needs precision 32 and the option fast");
     if (!fast) SB_OK(ensure_diffs64(pl));
 
     // order templates by search angle (then best state) so that each curvature spectrum is built once
@@ -616,14 +600,13 @@ int run_sweep_t(sb_plan* pl, const sb_angle* angles, int n_angles, const sb_temp
     }
 
     const int rpitch_max = need_rows_max + (need_rows_max & 1);
-    const bool lincomb = fast && pl->lincomb;
-    SB_OK(ensure(pl->cr, (size_t)std::max(Ba, lincomb ? sb::kDiffPairs : 0) * KXm * rpitch_max * sizeof(C4)));
-    if (lincomb) {
+    SB_OK(ensure(pl->cr, (size_t)std::max(Ba, fast ? sb::kDiffPairs : 0) * KXm * rpitch_max * sizeof(C4)));
+    if (fast) {
         SB_OK(ensure(pl->spec9, (size_t)2 * sb::kDiffPairs * KXm * Pym * sizeof(float2)));
         SB_OK(ensure(pl->coef, (size_t)n_angles * sizeof(sb::SpecCoef)));
         std::vector<sb::SpecCoef> coef(n_angles);
         for (int a = 0; a < n_angles; ++a) {
-            // the float32 values k_curv_rows_f uses: cos^2, 2 sin cos, sin^2 of the search angle
+            // cos^2, 2 sin cos, sin^2 of the search angle, each rounded to float32, and their products
             const double c2 = (double)(float)angles[a].cos2_a, sc = (double)(float)(2.0 * angles[a].sin_a * angles[a].cos_a),
                          s2 = (double)(float)angles[a].sin2_a;
             const double v[sb::kDiffPlanes] = {c2, -sc, s2, c2 * c2, sc * sc, s2 * s2, -2.0 * c2 * sc, 2.0 * c2 * s2, -2.0 * sc * s2};
@@ -715,9 +698,9 @@ int run_sweep_t(sb_plan* pl, const sb_angle* angles, int n_angles, const sb_temp
         SB_OK(ensure(pl->casa, casa.size() * sizeof(double)));
         SB_OK(ensure(pl->cross, (size_t)n_angles * pl->ny * sizeof(int4)));
         SB_TRY(sb_rt_h2d(pl->casa.p, casa.data(), casa.size() * sizeof(double), pl->stream));
-        SB_LAUNCH(sb::k_err_cross, dim3(div_up((long)n_angles * pl->ny, 256)), dim3(256), 0, pl->stream, pl->ny, pl->nx,
-                  n_angles, (const double*)pl->casa.p, (const double*)pl->d_x, (const double*)pl->d_y, (int4*)pl->cross.p);
-        SB_OK(check_launch(pl, "k_err_cross"));
+        SB_OK(launch(pl, "k_err_cross", sb::k_err_cross, dim3(div_up((long)n_angles * pl->ny, 256)), dim3(256), 0,
+                     pl->ny, pl->nx, n_angles, (const double*)pl->casa.p, (const double*)pl->d_x,
+                     (const double*)pl->d_y, (int4*)pl->cross.p));
     }
     // the host vectors must outlive the async copies
     SB_TRY(sb_rt_sync(pl->stream));
@@ -753,9 +736,8 @@ int run_sweep_t(sb_plan* pl, const sb_angle* angles, int n_angles, const sb_temp
             pl->best_copies = nsub;
         }
         const long cnt_x = (long)(nsub - 1) * sub_stride;
-        SB_LAUNCH(sb::k_best_init, dim3(div_up(cnt_x, 256)), dim3(256), 0, pl->stream, cnt_x, pl->d_bsnr + sub_stride,
-                  pl->d_bamp + sub_stride, pl->d_bidx + sub_stride);
-        SB_OK(check_launch(pl, "k_best_init"));
+        SB_OK(launch(pl, "k_best_init", sb::k_best_init, dim3(div_up(cnt_x, 256)), dim3(256), 0, cnt_x,
+                     pl->d_bsnr + sub_stride, pl->d_bamp + sub_stride, pl->d_bidx + sub_stride));
     }
 
     pl->last_geom[0] = Pym; pl->last_geom[1] = Pxm; pl->last_geom[2] = (int)ay.tiles.size();
@@ -784,34 +766,29 @@ int run_sweep_t(sb_plan* pl, const sb_angle* angles, int n_angles, const sb_temp
             g.dx = pl->dx; g.dx2 = pl->dx2; g.dy2 = pl->dy2;
             g.norm = 1.0 / ((double)Px * (double)Py);
             g.c2_scale = pl->c2_scale;
-            g.dbg = pl->dbg;
             g.poison = pl->dem_nonfinite ? 1 : 0;
             g.row0 = pl->row0; g.drows = pl->drows; g.brow0 = pl->slab_lo;
             const int need_rows = g.need_y_hi - g.need_y_lo + 1;
             g.rpitch = need_rows + (need_rows & 1);
 
-            if (lincomb) {
+            if (fast) {
                 // the nine plane spectra of this tile, once: five packed row transforms, column transforms
                 SB_OK(dispatch_n(Px, [&](auto nn) {
                     constexpr int N = decltype(nn)::value;
                     using S = Shape<N, float>;
                     auto kern = masked ? sb::k_diff_rows_fm<N> : sb::k_diff_rows_f<N>;
-                    SB_ALLOW_SMEM(kern, S::smem_conv_f);
                     ProfScope prof(pl, K_CURV_ROWS);
-                    SB_LAUNCH(kern, dim3(sb::kDiffPairs, div_up(div_up(need_rows, 2), S::GP)), dim3(S::threads),
-                              S::smem_conv_f, pl->stream, g, (const float4*)pl->d_diffs32, (float4*)pl->cr.p,
-                              (const float2*)twx);
-                    return check_launch(pl, "k_diff_rows_f");
+                    return launch(pl, "k_diff_rows_f", kern, dim3(sb::kDiffPairs, div_up(div_up(need_rows, 2), S::GP)),
+                                  dim3(S::threads), S::smem_conv_f, g, (const float4*)pl->d_diffs32, (float4*)pl->cr.p,
+                                  (const float2*)twx);
                 }));
                 SB_OK(dispatch_n(Py, [&](auto nn) {
                     constexpr int N = decltype(nn)::value;
                     using S = Shape<N, float>;
-                    auto kern = sb::k_curv_cols<N, float>;
-                    SB_ALLOW_SMEM(kern, S::smem);
                     ProfScope prof(pl, K_CURV_ROWS);
-                    SB_LAUNCH(kern, dim3(div_up(KX, S::GP), sb::kDiffPairs), dim3(S::threads), S::smem,
-                              pl->stream, g, (const float4*)pl->cr.p, (float2*)pl->spec9.p, (const float2*)twy);
-                    return check_launch(pl, "k_curv_cols");
+                    return launch(pl, "k_curv_cols", sb::k_curv_cols<N, float>, dim3(div_up(KX, S::GP), sb::kDiffPairs),
+                                  dim3(S::threads), S::smem, g, (const float4*)pl->cr.p, (float2*)pl->spec9.p,
+                                  (const float2*)twy);
                 }));
                 if (masked) {
                     const size_t plane = (size_t)KX * Py;       // float2 elements of one spectrum plane
@@ -823,47 +800,29 @@ int run_sweep_t(sb_plan* pl, const sb_angle* angles, int n_angles, const sb_temp
             }
             for (auto& ab : batches) {
                 const int a0 = ab.a0, a1 = ab.a1;
-                if (lincomb) {
+                if (fast) {
                     const long n2 = (long)KX * Py / 2;
                     ProfScope prof(pl, K_CURV_COLS);
-                    SB_LAUNCH(sb::k_combine_spectra, dim3(div_up(n2, 256)), dim3(256), (a1 - a0) * sizeof(sb::SpecCoef),
-                              pl->stream, n2, a1 - a0, a0, (const sb::SpecCoef*)pl->coef.p, (const float4*)pl->spec9.p,
-                              (float4*)pl->fct.p);
-                    SB_OK(check_launch(pl, "k_combine_spectra"));
-                } else if (fast) {
+                    SB_OK(launch(pl, "k_combine_spectra", sb::k_combine_spectra, dim3(div_up(n2, 256)), dim3(256),
+                                 (a1 - a0) * sizeof(sb::SpecCoef), n2, a1 - a0, a0, (const sb::SpecCoef*)pl->coef.p,
+                                 (const float4*)pl->spec9.p, (float4*)pl->fct.p));
+                } else {
                     SB_OK(dispatch_n(Px, [&](auto nn) {
                         constexpr int N = decltype(nn)::value;
-                        using S = Shape<N, float>;
-                        auto kern = sb::k_curv_rows_f<N>;
-                        SB_ALLOW_SMEM(kern, S::smem_conv_f);
+                        using S = Shape<N, R>;
                         ProfScope prof(pl, K_CURV_ROWS);
-                        SB_LAUNCH(kern, dim3(a1 - a0, div_up(div_up(need_rows, 2), S::GP)), dim3(S::threads),
-                                  S::smem_conv_f, pl->stream, g, (const float4*)pl->d_diffs32, d_an, a0,
-                                  (float4*)pl->cr.p, (const float2*)twx);
-                        return check_launch(pl, "k_curv_rows_f");
+                        return launch(pl, "k_curv_rows", sb::k_curv_rows<N, R>,
+                                      dim3(a1 - a0, div_up(div_up(need_rows, 2), S::GP)), dim3(S::threads), S::smem, g,
+                                      (const double*)pl->d_diffs, d_an, a0, (C4*)pl->cr.p, twx);
                     }));
-                } else
-                SB_OK(dispatch_n(Px, [&](auto nn) {
-                    constexpr int N = decltype(nn)::value;
-                    using S = Shape<N, R>;
-                    auto kern = sb::k_curv_rows<N, R>;
-                    SB_ALLOW_SMEM(kern, S::smem);
-                    ProfScope prof(pl, K_CURV_ROWS);
-                    SB_LAUNCH(kern, dim3(a1 - a0, div_up(div_up(need_rows, 2), S::GP)), dim3(S::threads),
-                              S::smem, pl->stream, g, (const double*)pl->d_diffs, d_an, a0, (C4*)pl->cr.p, twx);
-                    return check_launch(pl, "k_curv_rows");
-                }));
-                if (!lincomb)
-                SB_OK(dispatch_n(Py, [&](auto nn) {
-                    constexpr int N = decltype(nn)::value;
-                    using S = Shape<N, R>;
-                    auto kern = sb::k_curv_cols<N, R>;
-                    SB_ALLOW_SMEM(kern, S::smem);
-                    ProfScope prof(pl, K_CURV_COLS);
-                    SB_LAUNCH(kern, dim3(div_up(KX, S::GP), a1 - a0), dim3(S::threads), S::smem,
-                              pl->stream, g, (const C4*)pl->cr.p, (C2*)pl->fct.p, twy);
-                    return check_launch(pl, "k_curv_cols");
-                }));
+                    SB_OK(dispatch_n(Py, [&](auto nn) {
+                        constexpr int N = decltype(nn)::value;
+                        using S = Shape<N, R>;
+                        ProfScope prof(pl, K_CURV_COLS);
+                        return launch(pl, "k_curv_cols", sb::k_curv_cols<N, R>, dim3(div_up(KX, S::GP), a1 - a0),
+                                      dim3(S::threads), S::smem, g, (const C4*)pl->cr.p, (C2*)pl->fct.p, twy);
+                    }));
+                }
                 for (auto& ch : ab.chunks) {
                     // the chunk's device records (a masked sweep: templates, then companions)
                     const int pb = ch.pb * rec_per_tmpl, cnt = ch.cnt * rec_per_tmpl;
@@ -874,51 +833,38 @@ int run_sweep_t(sb_plan* pl, const sb_angle* angles, int n_angles, const sb_temp
                         // narrow templates: two samples per thread (needs a radix-16 first stage)
                         const bool xsparse = N >= 256 && hi_x <= S::T - 1 && lo_x >= -S::T;
                         const int nt = ch.cnt;            // the templates; a masked sweep's companions follow
+                        const dim3 grid(div_up(syp / 2, S::GP), nt);
+                        auto kern = sb::k_tmpl_rows<N, R, false>;
                         if constexpr (N >= 256) {
-                            if (xsparse) {
-                                auto kern = sb::k_tmpl_rows<N, R, true>;
-                                SB_ALLOW_SMEM(kern, S::smem);
-                                SB_LAUNCH(kern, dim3(div_up(syp / 2, S::GP), nt), dim3(S::threads), S::smem,
-                                          pl->stream, g, d_tm, pb, (const double*)pl->d_x, (const double*)pl->d_y,
-                                          (C4*)pl->trt.p, (double2*)pl->part.p, twx, (const double*)pl->tbox.p);
-                                SB_OK(check_launch(pl, "k_tmpl_rows"));
-                            }
+                            if (xsparse) kern = sb::k_tmpl_rows<N, R, true>;
                         }
-                        if (!xsparse) {
-                            auto kern = sb::k_tmpl_rows<N, R, false>;
-                            SB_ALLOW_SMEM(kern, S::smem);
-                            SB_LAUNCH(kern, dim3(div_up(syp / 2, S::GP), nt), dim3(S::threads), S::smem,
-                                      pl->stream, g, d_tm, pb, (const double*)pl->d_x, (const double*)pl->d_y,
-                                      (C4*)pl->trt.p, (double2*)pl->part.p, twx, (const double*)pl->tbox.p);
-                            SB_OK(check_launch(pl, "k_tmpl_rows"));
-                        }
+                        SB_OK(launch(pl, "k_tmpl_rows", kern, grid, dim3(S::threads), S::smem, g, d_tm, pb,
+                                     (const double*)pl->d_x, (const double*)pl->d_y, (C4*)pl->trt.p,
+                                     (double2*)pl->part.p, twx, (const double*)pl->tbox.p));
                         if constexpr (kF32) {
                             if (masked) {
                                 // the companions: t**2, records pb + nt ..; trt / part slots nt ..
-                                auto kern = sb::k_tmpl_rows_sq<N, false>;
+                                auto kern_sq = sb::k_tmpl_rows_sq<N, false>;
                                 if constexpr (N >= 256) {
-                                    if (xsparse) kern = sb::k_tmpl_rows_sq<N, true>;
+                                    if (xsparse) kern_sq = sb::k_tmpl_rows_sq<N, true>;
                                 }
-                                SB_ALLOW_SMEM(kern, S::smem);
-                                SB_LAUNCH(kern, dim3(div_up(syp / 2, S::GP), nt), dim3(S::threads), S::smem,
-                                          pl->stream, g, d_tm, pb + nt, (const double*)pl->d_x, (const double*)pl->d_y,
-                                          (float4*)pl->trt.p + (size_t)nt * (N / 2 + 1) * syp,
-                                          (double2*)pl->part.p + (size_t)nt * syp, (const float2*)twx);
-                                SB_OK(check_launch(pl, "k_tmpl_rows_sq"));
+                                SB_OK(launch(pl, "k_tmpl_rows_sq", kern_sq, grid, dim3(S::threads), S::smem, g, d_tm,
+                                             pb + nt, (const double*)pl->d_x, (const double*)pl->d_y,
+                                             (float4*)pl->trt.p + (size_t)nt * (N / 2 + 1) * syp,
+                                             (double2*)pl->part.p + (size_t)nt * syp, (const float2*)twx));
                             }
                         }
                         return 0;
                     }));
                     {
                         ProfScope prof(pl, K_TMPL_SUMS);
-                        SB_LAUNCH(sb::k_tmpl_sums, dim3(cnt), dim3(32), 32 * sizeof(double2), pl->stream, g, d_tm, pb, cnt,
-                                  (const double2*)pl->part.p, (sb::TSum*)pl->sums.p, (sb::FitT*)pl->fit.p);
-                        SB_OK(check_launch(pl, "k_tmpl_sums"));
-                        if (masked) {
-                            SB_LAUNCH(sb::k_mask_consts, dim3(div_up(ch.cnt, 32)), dim3(32), 0, pl->stream, g, d_tm, pb,
-                                      ch.cnt, pl->min_cov, (const sb::TSum*)pl->sums.p, (sb::FitM*)pl->fitm.p);
-                            SB_OK(check_launch(pl, "k_mask_consts"));
-                        }
+                        SB_OK(launch(pl, "k_tmpl_sums", sb::k_tmpl_sums, dim3(cnt), dim3(32), 32 * sizeof(double2), g,
+                                     d_tm, pb, cnt, (const double2*)pl->part.p, (sb::TSum*)pl->sums.p,
+                                     (sb::FitT*)pl->fit.p));
+                        if (masked)
+                            SB_OK(launch(pl, "k_mask_consts", sb::k_mask_consts, dim3(div_up(ch.cnt, 32)), dim3(32), 0,
+                                         g, d_tm, pb, ch.cnt, pl->min_cov, (const sb::TSum*)pl->sums.p,
+                                         (sb::FitM*)pl->fitm.p));
                     }
                     const bool fast_fit = fast && !so.raw_amp;
                     if constexpr (kF32) {
@@ -934,20 +880,11 @@ int run_sweep_t(sb_plan* pl, const sb_angle* angles, int n_angles, const sb_temp
                                     if (pl->conv_r64 && persist && cnt <= sb64::kConvRMaxBatch) {
                                         const float2* tw64 = nullptr;
                                         SB_OK(twiddles64(pl, &tw64));
-                                        if (hi_y <= 3 * sb64::R - 1 && lo_y >= -3 * sb64::R) {
-                                            auto kern = sb64::k_conv_cols_r<true>;
-                                            SB_ALLOW_SMEM(kern, sb64::kConvRSmem);
-                                            SB_LAUNCH(kern, dim3(KX), dim3(sb64::kConvRThreads), sb64::kConvRSmem, pl->stream, g,
-                                                      d_tm, pb, cnt, a0, (const float4*)pl->trt.p, (const float2*)pl->fct.p,
-                                                      (float4*)pl->gbuf.p, tw64);
-                                        } else {
-                                            auto kern = sb64::k_conv_cols_r<false>;
-                                            SB_ALLOW_SMEM(kern, sb64::kConvRSmem);
-                                            SB_LAUNCH(kern, dim3(KX), dim3(sb64::kConvRThreads), sb64::kConvRSmem, pl->stream, g,
-                                                      d_tm, pb, cnt, a0, (const float4*)pl->trt.p, (const float2*)pl->fct.p,
-                                                      (float4*)pl->gbuf.p, tw64);
-                                        }
-                                        return check_launch(pl, "k_conv_cols_r");
+                                        const bool sparse64 = hi_y <= 3 * sb64::R - 1 && lo_y >= -3 * sb64::R;
+                                        auto kern = sparse64 ? sb64::k_conv_cols_r<true> : sb64::k_conv_cols_r<false>;
+                                        return launch(pl, "k_conv_cols_r", kern, dim3(KX), dim3(sb64::kConvRThreads),
+                                                      sb64::kConvRSmem, g, d_tm, pb, cnt, a0, (const float4*)pl->trt.p,
+                                                      (const float2*)pl->fct.p, (float4*)pl->gbuf.p, tw64);
                                     }
                                 }
                                 if constexpr (N >= 1024 && N <= 4096) {
@@ -956,37 +893,18 @@ int run_sweep_t(sb_plan* pl, const sb_angle* angles, int n_angles, const sb_temp
                                             (size_t)(sb::kConvPThreads / S::T) * 2 * sbfft::padded_len(N) * sizeof(float2) +
                                             (size_t)2 * N * sizeof(float2) + sb::kConvPMaxBatch * 4 * sizeof(int) +
                                             (size_t)sbfft::ctw_count<float>(N) * sizeof(float2);
-                                        if (sparse) {
-                                            auto kern = sb::k_conv_cols_p<N, true>;
-                                            SB_ALLOW_SMEM(kern, smem_p);
-                                            SB_LAUNCH(kern, dim3(KX), dim3(sb::kConvPThreads), smem_p, pl->stream, g, d_tm,
-                                                      pb, cnt, a0, (const float4*)pl->trt.p, (const float2*)pl->fct.p,
-                                                      (float4*)pl->gbuf.p, (const float2*)twy);
-                                        } else {
-                                            auto kern = sb::k_conv_cols_p<N, false>;
-                                            SB_ALLOW_SMEM(kern, smem_p);
-                                            SB_LAUNCH(kern, dim3(KX), dim3(sb::kConvPThreads), smem_p, pl->stream, g, d_tm,
-                                                      pb, cnt, a0, (const float4*)pl->trt.p, (const float2*)pl->fct.p,
-                                                      (float4*)pl->gbuf.p, (const float2*)twy);
-                                        }
-                                        return check_launch(pl, "k_conv_cols_p");
+                                        auto kern = sparse ? sb::k_conv_cols_p<N, true> : sb::k_conv_cols_p<N, false>;
+                                        return launch(pl, "k_conv_cols_p", kern, dim3(KX), dim3(sb::kConvPThreads),
+                                                      smem_p, g, d_tm, pb, cnt, a0, (const float4*)pl->trt.p,
+                                                      (const float2*)pl->fct.p, (float4*)pl->gbuf.p,
+                                                      (const float2*)twy);
                                     }
                                 }
-                                const dim3 grid(cnt, div_up(KX, S::GP));
-                                if (sparse) {
-                                    auto kern = sb::k_conv_cols_f<N, true>;
-                                    SB_ALLOW_SMEM(kern, S::smem_conv_f);
-                                    SB_LAUNCH(kern, grid, dim3(S::threads), S::smem_conv_f, pl->stream, g, d_tm, pb, a0,
-                                              (const float4*)pl->trt.p, (const float2*)pl->fct.p, (float4*)pl->gbuf.p,
+                                auto kern = sparse ? sb::k_conv_cols_f<N, true> : sb::k_conv_cols_f<N, false>;
+                                return launch(pl, "k_conv_cols_f", kern, dim3(cnt, div_up(KX, S::GP)), dim3(S::threads),
+                                              S::smem_conv_f, g, d_tm, pb, a0, (const float4*)pl->trt.p,
+                                              (const float2*)pl->fct.p, (float4*)pl->gbuf.p,
                                               (const float2*)twy);
-                                } else {
-                                    auto kern = sb::k_conv_cols_f<N, false>;
-                                    SB_ALLOW_SMEM(kern, S::smem_conv_f);
-                                    SB_LAUNCH(kern, grid, dim3(S::threads), S::smem_conv_f, pl->stream, g, d_tm, pb, a0,
-                                              (const float4*)pl->trt.p, (const float2*)pl->fct.p, (float4*)pl->gbuf.p,
-                                              (const float2*)twy);
-                                }
-                                return check_launch(pl, "k_conv_cols_f");
                             }));
                         }
                     }
@@ -994,13 +912,10 @@ int run_sweep_t(sb_plan* pl, const sb_angle* angles, int n_angles, const sb_temp
                         SB_OK(dispatch_n(Py, [&](auto nn) {
                             constexpr int N = decltype(nn)::value;
                             using S = Shape<N, R>;
-                            auto kern = sb::k_conv_cols<N, R>;
-                            SB_ALLOW_SMEM(kern, S::smem_conv);
                             ProfScope prof(pl, K_CONV_COLS);
-                            SB_LAUNCH(kern, dim3(div_up(KX, S::GP), cnt), dim3(S::threads), S::smem_conv,
-                                      pl->stream, g, d_tm, pb, a0, (const C4*)pl->trt.p, (const C2*)pl->fct.p,
-                                      (C4*)pl->gbuf.p, twy);
-                            return check_launch(pl, "k_conv_cols");
+                            return launch(pl, "k_conv_cols", sb::k_conv_cols<N, R>, dim3(div_up(KX, S::GP), cnt),
+                                          dim3(S::threads), S::smem_conv, g, d_tm, pb, a0, (const C4*)pl->trt.p,
+                                          (const C2*)pl->fct.p, (C4*)pl->gbuf.p, twy);
                         }));
                     }
                     // fold: one launch per best state present in the chunk
@@ -1011,40 +926,35 @@ int run_sweep_t(sb_plan* pl, const sb_angle* angles, int n_angles, const sb_temp
                         int* bidx = pl->d_bidx + (long)gp.state * bn - boff;
                         if constexpr (kF32) {
                             if (fast_fit) {
+                                const int4* cross = gp.err ? (const int4*)pl->cross.p : (const int4*)nullptr;
                                 SB_OK(dispatch_n(Px, [&](auto nn) {
                                     constexpr int N = decltype(nn)::value;
                                     using S = Shape<N, float>;
                                     ProfScope prof(pl, K_FIT_ROWS);
+                                    const dim3 grid(div_up(Py / 2, S::GP), nsub);
                                     if (masked) {
                                         // FFT lengths <= 4096 only: the park buffers need 2 N float2 per group
                                         if constexpr (N <= kMaxFftMasked) {
-                                            auto kern = sb::k_fit_rows_gm<N>;
-                                            constexpr size_t smem = S::smem_fit_f + sb::fit_masked_extra_smem<N>();
-                                            SB_ALLOW_SMEM(kern, smem);
-                                            SB_LAUNCH(kern, dim3(div_up(Py / 2, S::GP), nsub), dim3(S::threads), smem,
-                                                      pl->stream, g, gp.count, d_slots, (const sb::FitT*)pl->fit.p,
-                                                      (const sb::FitM*)pl->fitm.p, ch.cnt, (const float4*)pl->gbuf.p,
-                                                      bsnr, bamp, bidx, (const float2*)twx,
-                                                      gp.err ? (const int4*)pl->cross.p : (const int4*)nullptr,
-                                                      sub_stride);
-                                            return check_launch(pl, "k_fit_rows_gm");
+                                            return launch(pl, "k_fit_rows_gm", sb::k_fit_rows_gm<N>, grid,
+                                                          dim3(S::threads),
+                                                          S::smem_fit_f + sb::fit_masked_extra_smem<N>(), g,
+                                                          gp.count, d_slots, (const sb::FitT*)pl->fit.p,
+                                                          (const sb::FitM*)pl->fitm.p, ch.cnt,
+                                                          (const float4*)pl->gbuf.p, bsnr, bamp, bidx,
+                                                          (const float2*)twx, cross, sub_stride);
                                         }
                                         return fail("internal: masked fit at FFT length " + std::to_string(N));
                                     }
                                     // (a variant without the get_err_mask members spills MORE: 564 bytes against 312)
-                                    auto kern = sb::k_fit_rows_g<N>;
-                                    SB_ALLOW_SMEM(kern, S::smem_fit_f);
-                                    SB_LAUNCH(kern, dim3(div_up(Py / 2, S::GP), nsub), dim3(S::threads), S::smem_fit_f,
-                                              pl->stream, g, gp.count, d_slots, (const sb::FitT*)pl->fit.p,
-                                              (const float4*)pl->gbuf.p, bsnr, bamp, bidx, (const float2*)twx,
-                                              gp.err ? (const int4*)pl->cross.p : (const int4*)nullptr, sub_stride);
-                                    return check_launch(pl, "k_fit_rows_g");
+                                    return launch(pl, "k_fit_rows_g", sb::k_fit_rows_g<N>, grid, dim3(S::threads),
+                                                  S::smem_fit_f, g, gp.count, d_slots, (const sb::FitT*)pl->fit.p,
+                                                  (const float4*)pl->gbuf.p, bsnr, bamp, bidx, (const float2*)twx,
+                                                  cross, sub_stride);
                                 }));
-                                if (g.poison) {
-                                    SB_LAUNCH(sb::k_poison_windows, dim3(div_up((long)g.out_ny * g.out_nx, 256)), dim3(256), 0,
-                                              pl->stream, g, gp.count, d_slots, (const sb::FitT*)pl->fit.p, bsnr);
-                                    SB_OK(check_launch(pl, "k_poison_windows"));
-                                }
+                                if (g.poison)
+                                    SB_OK(launch(pl, "k_poison_windows", sb::k_poison_windows,
+                                                 dim3(div_up((long)g.out_ny * g.out_nx, 256)), dim3(256), 0, g,
+                                                 gp.count, d_slots, (const sb::FitT*)pl->fit.p, bsnr));
                                 continue;
                             }
                         }
@@ -1054,29 +964,25 @@ int run_sweep_t(sb_plan* pl, const sb_angle* angles, int n_angles, const sb_temp
                         SB_OK(dispatch_n(Px, [&](auto nn) {
                             constexpr int N = decltype(nn)::value;
                             using S = Shape<N, R>;
-                            auto kern = sb::k_fit_rows<N, R>;
-                            SB_ALLOW_SMEM(kern, S::smem);
                             ProfScope prof(pl, K_FIT_ROWS);
-                            SB_LAUNCH(kern, dim3(div_up(g.out_ny, S::GP)), dim3(S::threads), S::smem,
-                                      pl->stream, g, d_tm, pb, gp.count, d_slots, (const sb::TSum*)pl->sums.p,
-                                      (const C4*)pl->gbuf.p, (const double*)pl->d_x, (const double*)pl->d_y, fo, twx);
-                            return check_launch(pl, "k_fit_rows");
+                            return launch(pl, "k_fit_rows", sb::k_fit_rows<N, R>, dim3(div_up(g.out_ny, S::GP)),
+                                          dim3(S::threads), S::smem, g, d_tm, pb, gp.count, d_slots,
+                                          (const sb::TSum*)pl->sums.p, (const C4*)pl->gbuf.p, (const double*)pl->d_x,
+                                          (const double*)pl->d_y, fo, twx);
                         }));
                     }
                 }
             }
         }
     if (nsub > 1) {
-        SB_LAUNCH(sb::k_best_fold, dim3(div_up(sub_stride, 256)), dim3(256), 0, pl->stream, sub_stride, nsub - 1, sub_stride,
-                  (const float*)pl->d_bsnr + sub_stride, (const float*)pl->d_bamp + sub_stride,
-                  (const int*)pl->d_bidx + sub_stride, pl->d_bsnr, pl->d_bamp, pl->d_bidx);
-        SB_OK(check_launch(pl, "k_best_fold"));
+        SB_OK(launch(pl, "k_best_fold", sb::k_best_fold, dim3(div_up(sub_stride, 256)), dim3(256), 0, sub_stride,
+                     nsub - 1, sub_stride, (const float*)pl->d_bsnr + sub_stride, (const float*)pl->d_bamp + sub_stride,
+                     (const int*)pl->d_bidx + sub_stride, pl->d_bsnr, pl->d_bamp, pl->d_bidx));
     }
     if (masked) {
-        SB_LAUNCH(sb::k_best_clear_nodata, dim3(div_up(bn, 256)), dim3(256), 0, pl->stream, pl->ny, pl->nx, pl->row0,
-                  pl->slab_lo, (int)pl->brows(), pl->n_states, bn, (const double*)pl->d_dem, pl->d_bsnr, pl->d_bamp,
-                  pl->d_bidx);
-        SB_OK(check_launch(pl, "k_best_clear_nodata"));
+        SB_OK(launch(pl, "k_best_clear_nodata", sb::k_best_clear_nodata, dim3(div_up(bn, 256)), dim3(256), 0, pl->ny,
+                     pl->nx, pl->row0, pl->slab_lo, (int)pl->brows(), pl->n_states, bn, (const double*)pl->d_dem,
+                     pl->d_bsnr, pl->d_bamp, pl->d_bidx));
     }
     drain_profile(pl);
     return 0;
@@ -1141,12 +1047,6 @@ int sb_plan_create(sb_plan** plan, int ny, int nx, double dx, double dx2, double
         }
         pl->own_stream = true;
     }
-    if (const char* e = std::getenv("SB_CONV_P")) pl->conv_persist = std::atoi(e);
-    if (const char* e = std::getenv("SB_CONV_R64")) pl->conv_r64 = std::atoi(e);
-    if (const char* e = std::getenv("SB_LINCOMB")) pl->lincomb = std::atoi(e);
-#ifdef SB_ABLATE
-    if (const char* e = std::getenv("SB_DBG")) pl->dbg = std::atoi(e);
-#endif
 #else
     (void)device; (void)stream;
 #endif
@@ -1198,7 +1098,6 @@ int sb_plan_set_option(sb_plan* pl, const char* key, long value) {
     if (k == "fast") { pl->fast = value != 0; return 0; }
     if (k == "conv_persist") { pl->conv_persist = (int)value; return 0; }
     if (k == "conv_r64") { pl->conv_r64 = value != 0; return 0; }
-    if (k == "lincomb") { pl->lincomb = value != 0; return 0; }
     if (k == "fit_substreams") { pl->fit_substreams = (int)std::max(0L, std::min(8L, value)); return 0; }
     if (k == "precision") {
         if (value != 32 && value != 64) return fail("precision must be 32 or 64");
@@ -1346,9 +1245,8 @@ int sb_directional_laplacian(sb_plan* pl, const sb_angle* angle, double* out, in
     }
     sb::Angle a;
     a.ca = angle->cos_a; a.sa = angle->sin_a; a.ca2 = angle->cos2_a; a.sa2 = angle->sin2_a;
-    SB_LAUNCH(sb::k_laplacian, dim3(div_up(n, 256)), dim3(256), 0, pl->stream, pl->ny, pl->nx,
-              (const double*)pl->d_dem, pl->dx, pl->dx2, pl->dy2, a, dst);
-    SB_OK(check_launch(pl, "k_laplacian"));
+    SB_OK(launch(pl, "k_laplacian", sb::k_laplacian, dim3(div_up(n, 256)), dim3(256), 0, pl->ny, pl->nx,
+                 (const double*)pl->d_dem, pl->dx, pl->dx2, pl->dy2, a, dst));
     if (!out_is_device) return copy_out(pl, out, dst, (size_t)n, 0);
     SB_TRY(sb_rt_sync(pl->stream));
     return 0;
@@ -1365,9 +1263,8 @@ int sb_render_template(sb_plan* pl, const sb_template* tmpl, double* out, int ou
     }
     sb::Tmpl t;
     std::memcpy(&t, tmpl, sizeof(t));
-    SB_LAUNCH(sb::k_render_template, dim3(div_up(n, 256)), dim3(256), 0, pl->stream, pl->ny, pl->nx, t,
-              (const double*)pl->d_x, (const double*)pl->d_y, dst);
-    SB_OK(check_launch(pl, "k_render_template"));
+    SB_OK(launch(pl, "k_render_template", sb::k_render_template, dim3(div_up(n, 256)), dim3(256), 0, pl->ny, pl->nx, t,
+                 (const double*)pl->d_x, (const double*)pl->d_y, dst));
     if (!out_is_device) return copy_out(pl, out, dst, (size_t)n, 0);
     SB_TRY(sb_rt_sync(pl->stream));
     return 0;
@@ -1422,9 +1319,8 @@ int sb_match_template_raster(sb_plan* pl, const sb_angle* angle, const double* b
 int sb_best_reset(sb_plan* pl) {
     if (!pl) return fail("null plan");
     const long n = pl->bn() * pl->n_states;
-    SB_LAUNCH(sb::k_best_init, dim3(div_up(n, 256)), dim3(256), 0, pl->stream, n, pl->d_bsnr, pl->d_bamp,
-              pl->d_bidx);
-    return check_launch(pl, "k_best_init");
+    return launch(pl, "k_best_init", sb::k_best_init, dim3(div_up(n, 256)), dim3(256), 0, n, pl->d_bsnr, pl->d_bamp,
+                  pl->d_bidx);
 }
 
 int sb_sweep(sb_plan* pl, const sb_angle* angles, int n_angles, const sb_template* tmpls, int n_tmpls) {
@@ -1455,10 +1351,9 @@ int sb_finalize_ex(sb_plan* pl, int state, int row_lo, int row_hi, const double*
         SB_OK(ensure(pl->raw, (size_t)n * 4 * sizeof(double)));
         dst = (double*)pl->raw.p;
     }
-    SB_LAUNCH(sb::k_finalize, dim3(div_up(n, 256)), dim3(256), 0, pl->stream, n, (const float*)pl->d_bsnr + off,
-              (const float*)pl->d_bamp + off, (const int*)pl->d_bidx + off, (const double*)d_age, (const double*)d_ang,
-              n_idx, dst);
-    SB_OK(check_launch(pl, "k_finalize"));
+    SB_OK(launch(pl, "k_finalize", sb::k_finalize, dim3(div_up(n, 256)), dim3(256), 0, n,
+                 (const float*)pl->d_bsnr + off, (const float*)pl->d_bamp + off, (const int*)pl->d_bidx + off,
+                 (const double*)d_age, (const double*)d_ang, n_idx, dst));
     if (!out_is_device) return copy_out(pl, out4, dst, (size_t)n * 4, 0);
     SB_TRY(sb_rt_sync(pl->stream));
     return 0;
@@ -1491,33 +1386,29 @@ int sb_best_merge(sb_plan* pl, int state, int row_lo, int row_hi, int n_cands, c
     if (row_lo < pl->slab_lo || row_hi > pl->slab_hi || row_lo >= row_hi) return fail("sb_best_merge: rows outside the plan");
     const long n = (long)(row_hi - row_lo) * pl->nx;
     const long off = (long)state * pl->bn() + (long)(row_lo - pl->slab_lo) * pl->nx;
-    SB_LAUNCH(sb::k_best_merge, dim3(div_up(n, 256)), dim3(256), 0, pl->stream, n, n_cands, snr_c, amp_c, (const int*)idx_c,
-              pl->d_bsnr + off, pl->d_bamp + off, pl->d_bidx + off);
-    return check_launch(pl, "k_best_merge");
+    return launch(pl, "k_best_merge", sb::k_best_merge, dim3(div_up(n, 256)), dim3(256), 0, n, n_cands, snr_c, amp_c,
+                  (const int*)idx_c, pl->d_bsnr + off, pl->d_bamp + off, pl->d_bidx + off);
 }
 
 int sb_best_pack(sb_plan* pl, unsigned long long* keys_dev) {
     if (!pl || !keys_dev) return fail("sb_best_pack: null");
     const long n = pl->bn();
-    SB_LAUNCH(sb::k_best_pack, dim3(div_up(n, 256)), dim3(256), 0, pl->stream, n, (const float*)pl->d_bsnr,
-              (const int*)pl->d_bidx, keys_dev);
-    return check_launch(pl, "k_best_pack");
+    return launch(pl, "k_best_pack", sb::k_best_pack, dim3(div_up(n, 256)), dim3(256), 0, n, (const float*)pl->d_bsnr,
+                  (const int*)pl->d_bidx, keys_dev);
 }
 
 int sb_best_select(sb_plan* pl, const unsigned long long* gkeys_dev, float* amp_out_dev) {
     if (!pl || !gkeys_dev || !amp_out_dev) return fail("sb_best_select: null");
     const long n = pl->bn();
-    SB_LAUNCH(sb::k_best_select, dim3(div_up(n, 256)), dim3(256), 0, pl->stream, n, (const float*)pl->d_bsnr,
-              (const float*)pl->d_bamp, (const int*)pl->d_bidx, gkeys_dev, amp_out_dev);
-    return check_launch(pl, "k_best_select");
+    return launch(pl, "k_best_select", sb::k_best_select, dim3(div_up(n, 256)), dim3(256), 0, n,
+                  (const float*)pl->d_bsnr, (const float*)pl->d_bamp, (const int*)pl->d_bidx, gkeys_dev, amp_out_dev);
 }
 
 int sb_best_unpack(sb_plan* pl, const unsigned long long* gkeys_dev, const float* amp_dev) {
     if (!pl || !gkeys_dev || !amp_dev) return fail("sb_best_unpack: null");
     const long n = pl->bn();
-    SB_LAUNCH(sb::k_best_unpack, dim3(div_up(n, 256)), dim3(256), 0, pl->stream, n, gkeys_dev, amp_dev,
-              pl->d_bsnr, pl->d_bamp, pl->d_bidx);
-    return check_launch(pl, "k_best_unpack");
+    return launch(pl, "k_best_unpack", sb::k_best_unpack, dim3(div_up(n, 256)), dim3(256), 0, n, gkeys_dev, amp_dev,
+                  pl->d_bsnr, pl->d_bamp, pl->d_bidx);
 }
 
 int sb_compare_host(sb_plan* pl, double* best4_host, const double* amp, const double* age, const double* angle,
@@ -1533,9 +1424,8 @@ int sb_compare_host(sb_plan* pl, double* best4_host, const double* amp, const do
     const double* d_ang = nullptr;
     if (age) { SB_TRY(sb_rt_h2d(d + 6 * n, age, (size_t)n * sizeof(double), pl->stream)); d_age = d + 6 * n; }
     if (angle) { SB_TRY(sb_rt_h2d(d + 7 * n, angle, (size_t)n * sizeof(double), pl->stream)); d_ang = d + 7 * n; }
-    SB_LAUNCH(sb::k_compare, dim3(div_up(n, 256)), dim3(256), 0, pl->stream, n, d, d + n, d + 2 * n, d + 3 * n,
-              (const double*)(d + 4 * n), d_age, d_ang, (const double*)(d + 5 * n), age_s, angle_s);
-    SB_OK(check_launch(pl, "k_compare"));
+    SB_OK(launch(pl, "k_compare", sb::k_compare, dim3(div_up(n, 256)), dim3(256), 0, n, d, d + n, d + 2 * n, d + 3 * n,
+                 (const double*)(d + 4 * n), d_age, d_ang, (const double*)(d + 5 * n), age_s, angle_s));
     return copy_out(pl, best4_host, d, (size_t)n * 4, 0);
 }
 
@@ -1562,15 +1452,12 @@ int sb_curvature_noise_moments(sb_plan* pl, double sigma, double truncate, doubl
     double* d_low = d_tmp + 4 * n;
     double* d_part = d_low + 4 * n;
     SB_TRY(sb_rt_h2d(d_w, w.data(), w.size() * sizeof(double), pl->stream));
-    SB_LAUNCH(sb::k_gauss_axis0, dim3(div_up(n, 256), 4), dim3(256), 0, pl->stream, ny, nx, radius, (const double*)d_w,
-              (const double*)pl->d_diffs, (const double*)pl->d_dem, d_tmp);
-    SB_OK(check_launch(pl, "k_gauss_axis0"));
-    SB_LAUNCH(sb::k_gauss_axis1, dim3(div_up(n, 256), 4), dim3(256), 0, pl->stream, ny, nx, radius, (const double*)d_w,
-              (const double*)d_tmp, d_low);
-    SB_OK(check_launch(pl, "k_gauss_axis1"));
-    SB_LAUNCH(sb::k_noise_moments, dim3(blocks), dim3(256), 256 * 10 * sizeof(double), pl->stream, n,
-              (const double*)pl->d_diffs, (const double*)pl->d_dem, (const double*)d_low, d_part);
-    SB_OK(check_launch(pl, "k_noise_moments"));
+    SB_OK(launch(pl, "k_gauss_axis0", sb::k_gauss_axis0, dim3(div_up(n, 256), 4), dim3(256), 0, ny, nx, radius,
+                 (const double*)d_w, (const double*)pl->d_diffs, (const double*)pl->d_dem, d_tmp));
+    SB_OK(launch(pl, "k_gauss_axis1", sb::k_gauss_axis1, dim3(div_up(n, 256), 4), dim3(256), 0, ny, nx, radius,
+                 (const double*)d_w, (const double*)d_tmp, d_low));
+    SB_OK(launch(pl, "k_noise_moments", sb::k_noise_moments, dim3(blocks), dim3(256), 256 * 10 * sizeof(double), n,
+                 (const double*)pl->d_diffs, (const double*)pl->d_dem, (const double*)d_low, d_part));
     std::vector<double> part((size_t)blocks * 10);
     SB_TRY(sb_rt_d2h(part.data(), d_part, part.size() * sizeof(double), pl->stream));
     SB_TRY(sb_rt_sync(pl->stream));
@@ -1593,9 +1480,8 @@ int sb_fill_nodata(sb_plan* pl, double* dem_host_inout, double max_search_distan
     SB_TRY(sb_rt_h2d(d_in, dem_host_inout, (size_t)n * sizeof(double), pl->stream));
     SB_TRY(sb_rt_memset(d_cnt, 0, sizeof(long) * 1024, pl->stream));
     const int blocks = div_up(n, 256);
-    SB_LAUNCH(sb::k_fill_nodata, dim3(blocks), dim3(256), 0, pl->stream, pl->ny, pl->nx, (const double*)d_in, d_out,
-              max_search_distance, d_cnt);
-    SB_OK(check_launch(pl, "k_fill_nodata"));
+    SB_OK(launch(pl, "k_fill_nodata", sb::k_fill_nodata, dim3(blocks), dim3(256), 0, pl->ny, pl->nx,
+                 (const double*)d_in, d_out, max_search_distance, d_cnt));
     std::vector<long> cnt(1024);
     SB_TRY(sb_rt_d2h(cnt.data(), d_cnt, sizeof(long) * 1024, pl->stream));
     SB_OK(copy_out(pl, dem_host_inout, d_out, (size_t)n, 0));
@@ -1620,10 +1506,8 @@ int sb_debug_fft(sb_plan* pl, int n, int rows, const float* in_host, float* out_
         const float2* tw64 = nullptr;
         SB_OK(twiddles64(pl, &tw64));
         constexpr size_t smem = (size_t)(4 * sb64::kXchg + sb64::kTwRows * sb64::R) * sizeof(float2);
-        SB_ALLOW_SMEM(sb64::k_fft4096_r64, smem);
-        SB_LAUNCH(sb64::k_fft4096_r64, dim3(div_up(rows, 4)), dim3(256), smem, pl->stream, rows, (const float2*)d_in,
-                  d_out, inverse & 1, tw64);
-        SB_OK(check_launch(pl, "k_fft4096_r64"));
+        SB_OK(launch(pl, "k_fft4096_r64", sb64::k_fft4096_r64, dim3(div_up(rows, 4)), dim3(256), smem, rows,
+                     (const float2*)d_in, d_out, inverse & 1, tw64));
         SB_TRY(sb_rt_d2h(out_host, d_out, bytes, pl->stream));
         SB_TRY(sb_rt_sync(pl->stream));
         return 0;
@@ -1632,10 +1516,8 @@ int sb_debug_fft(sb_plan* pl, int n, int rows, const float* in_host, float* out_
         constexpr int N = decltype(nn)::value;
         using S = Shape<N, float>;
         auto kern = sb::k_fft_rows<N, float>;
-        SB_ALLOW_SMEM(kern, S::smem);
-        SB_LAUNCH(kern, dim3(div_up(rows, S::GP)), dim3(S::threads), S::smem, pl->stream, rows,
-                  (const float2*)d_in, d_out, inverse, tw);
-        return check_launch(pl, "k_fft_rows");
+        return launch(pl, "k_fft_rows", kern, dim3(div_up(rows, S::GP)), dim3(S::threads), S::smem, rows,
+                      (const float2*)d_in, d_out, inverse, tw);
     }));
     SB_TRY(sb_rt_d2h(out_host, d_out, bytes, pl->stream));
     SB_TRY(sb_rt_sync(pl->stream));
@@ -1662,12 +1544,8 @@ int sb_debug_fft_bench(sb_plan* pl, int n, int rows, int reps, int radix64, floa
             rc = twiddles64(pl, &tw64);
             if (rc) break;
             constexpr size_t smem = (size_t)(4 * sb64::kXchg + sb64::kTwRows * sb64::R) * sizeof(float2);
-#ifndef SB_EMU
-            cudaFuncSetAttribute(sb64::k_fft4096_r64, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem);
-#endif
-            SB_LAUNCH(sb64::k_fft4096_r64, dim3(div_up(rows, 4)), dim3(256), smem, pl->stream, rows, (const float2*)d_in,
-                      d_out, 0, tw64);
-            rc = check_launch(pl, "k_fft4096_r64");
+            rc = launch(pl, "k_fft4096_r64", sb64::k_fft4096_r64, dim3(div_up(rows, 4)), dim3(256), smem, rows,
+                        (const float2*)d_in, d_out, 0, tw64);
         } else {
             const float2* tw = nullptr;
             rc = twiddles<float>(pl, n, &tw);
@@ -1676,10 +1554,8 @@ int sb_debug_fft_bench(sb_plan* pl, int n, int rows, int reps, int radix64, floa
                 constexpr int N = decltype(nn)::value;
                 using S = Shape<N, float>;
                 auto kern = sb::k_fft_rows<N, float>;
-                SB_ALLOW_SMEM(kern, S::smem);
-                SB_LAUNCH(kern, dim3(div_up(rows, S::GP)), dim3(S::threads), S::smem, pl->stream, rows,
-                          (const float2*)d_in, d_out, 0, tw);
-                return check_launch(pl, "k_fft_rows");
+                return launch(pl, "k_fft_rows", kern, dim3(div_up(rows, S::GP)), dim3(S::threads), S::smem, rows,
+                              (const float2*)d_in, d_out, 0, tw);
             });
         }
     }

@@ -62,11 +62,8 @@ SB_DEVICE float4 sb_ld_shared_soon(const float4* p) {
     return r;
 }
 // write-once data (the planes handed to the next kernel)
-#ifndef SB_ST_POLICY
-#define SB_ST_POLICY ".L1::no_allocate"
-#endif
 SB_DEVICE void sb_st_stream(float4* p, float4 v) {
-    asm volatile("st.global" SB_ST_POLICY ".v4.f32 [%0], {%1, %2, %3, %4};" ::"l"(p), "f"(v.x), "f"(v.y), "f"(v.z), "f"(v.w) : "memory");
+    asm volatile("st.global.L1::no_allocate.v4.f32 [%0], {%1, %2, %3, %4};" ::"l"(p), "f"(v.x), "f"(v.y), "f"(v.z), "f"(v.w) : "memory");
 }
 // two adjacent values as one full-sector (float) / two-sector (double) store
 SB_DEVICE void sb_st_pair(float4* p, float4 a, float4 b) {
@@ -77,10 +74,7 @@ SB_DEVICE void sb_st_pair(double4* p, double4 a, double4 b) { p[0] = a; p[1] = b
 // one whole 32-byte sector (two adjacent float4) in one request; kept in L1 until its second
 // reader (the thread that needs the mirrored element) has had it, first in line for eviction
 SB_DEVICE void sb_ld_sector(const float4* p, float4& a, float4& b) {
-#ifndef SB_SECTOR_POLICY
-#define SB_SECTOR_POLICY ".L1::evict_first"
-#endif
-    asm("ld.global.nc" SB_SECTOR_POLICY ".v8.f32 {%0, %1, %2, %3, %4, %5, %6, %7}, [%8];"
+    asm("ld.global.nc.L1::evict_first.v8.f32 {%0, %1, %2, %3, %4, %5, %6, %7}, [%8];"
         : "=f"(a.x), "=f"(a.y), "=f"(a.z), "=f"(a.w), "=f"(b.x), "=f"(b.y), "=f"(b.z), "=f"(b.w) : "l"(p));
 }
 // hint: pull one 128-byte line towards L2 ahead of the loads that will need it

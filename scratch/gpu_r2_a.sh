@@ -24,7 +24,7 @@ timeout 1200 ncu --set full --clock-control none --import-source on -k regex:'k_
 ncu -i /tmp/a_prof.ncu-rep --page raw --csv > gpurun_out/a_prof_raw.csv 2>/dev/null
 ncu -i /tmp/a_prof.ncu-rep --page source --csv --print-source sass > gpurun_out/a_prof_source.csv 2>/dev/null
 gzip -f gpurun_out/a_prof_source.csv
-timeout 600 ncu --set full --clock-control none -k regex:'k_curv_rows_f|k_curv_cols|k_tmpl_rows|k_conv_cols_f|k_fit_rows_g' -s 10 -c 5 \
+timeout 600 ncu --set full --clock-control none -k regex:'k_curv_cols|k_tmpl_rows|k_conv_cols_f|k_fit_rows_g' -s 10 -c 5 \
   -o /tmp/a_prof_c1 -f python bench.py --workload c1 --steps 1 --warmup 1 --e2e-steps 1 --no-cpu-baseline --no-dropin > gpurun_out/a_ncu_c1.log 2>&1
 ncu -i /tmp/a_prof_c1.ncu-rep --page raw --csv > gpurun_out/a_prof_c1_raw.csv 2>/dev/null
 du -sh gpurun_out

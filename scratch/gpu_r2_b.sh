@@ -1,12 +1,11 @@
 #!/bin/bash
-# Round 2, GPU call B: radix-64 column kernel on hardware -- tests, bench with and without it, ncu.
+# Round 2, GPU call B: radix-64 column kernel on hardware -- tests, bench, ncu.
 cd "$(dirname "$0")/.."
 mkdir -p gpurun_out/parity
 export SB_PARITY_DIR=gpurun_out/parity
 ( time timeout 1500 python -m pytest tests -m gpu -q ) > gpurun_out/b_tests.log 2>&1
 echo "tests rc=$?" >> gpurun_out/b_tests.log
 timeout 600 python bench.py --steps 3 --warmup 3 --no-cpu-baseline > gpurun_out/b_bench_c3_r64.json 2> gpurun_out/b_bench_c3_r64.err
-SB_CONV_R64=0 timeout 600 python bench.py --steps 3 --warmup 3 --no-cpu-baseline --no-dropin > gpurun_out/b_bench_c3_r16.json 2> gpurun_out/b_bench_c3_r16.err
 timeout 1200 ncu --set full --clock-control none --import-source on -k regex:'k_conv_cols_r' -s 20 -c 1 \
   -o /tmp/b_prof -f python bench.py --steps 1 --warmup 1 --e2e-steps 1 --no-cpu-baseline --no-dropin > gpurun_out/b_ncu.log 2>&1
 ncu -i /tmp/b_prof.ncu-rep --page raw --csv > gpurun_out/b_prof_raw.csv 2>/dev/null

@@ -155,28 +155,24 @@ def test_persistent_column_kernel(emu_lib, scale, ages):
     from scarplet_b200.engine import Plan
     from scarplet_b200.synth import synthetic_dem
     from scarplet_b200.templates import Scarp
-    import os
     ny, nx = 1024, 200
     z = synthetic_dem(ny, seed=21, nx=nx, relief=3.0)
     angles = P.search_angles(-np.pi / 2, np.pi / 2)[[3, 50, 90, 140]]
     outs = {}
-    for persist in ("1", "0"):
-        os.environ["SB_CONV_P"] = persist            # read when the plan is created
-        try:
-            with Plan(ny, nx, 1.0, 1.0) as plan:
-                plan.set_dem(z)
-                a, t, age_of, angle_of = plan.build_sweep(Scarp._sb_spec, scale, ages, angles)
-                plan.reset()
-                plan.sweep(a, t)
-                outs[persist] = plan.finalize(age_of, angle_of)
-                assert plan.last_geometry()["Py"] == 1024
-        finally:
-            del os.environ["SB_CONV_P"]
+    for persist in (1, 0):
+        with Plan(ny, nx, 1.0, 1.0) as plan:
+            plan.set_option("conv_persist", persist)
+            plan.set_dem(z)
+            a, t, age_of, angle_of = plan.build_sweep(Scarp._sb_spec, scale, ages, angles)
+            plan.reset()
+            plan.sweep(a, t)
+            outs[persist] = plan.finalize(age_of, angle_of)
+            assert plan.last_geometry()["Py"] == 1024
     # same arithmetic in the same order as the per-template kernel
-    assert np.array_equal(outs["1"], outs["0"])
+    assert np.array_equal(outs[1], outs[0])
     ref = O.compare((O.match_template(z, 1.0, 1.0, O.SCARP, scale, age, ang)
                      for age in ages for ang in angles), ny, nx)
-    rep = stack_report(outs["1"], np.stack(ref))
+    rep = stack_report(outs[1], np.stack(ref))
     assert rep["mask_mismatch_unexplained"] == 0 and rep["index_agreement"] >= 0.999, rep
     # a 200-column strip holds nothing a scale-70 scarp fits (median SNR 0.07): the bound applies
     # to the upper half of the SNR range, the rest is noise-level

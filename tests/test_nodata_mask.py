@@ -234,12 +234,12 @@ def test_nodata_errors(emu_lib):
         with pytest.raises(SbError, match="match_template"):
             plan.match_template_raster(plan.render_template(T.Scarp._sb_spec, 8, 3.0, 0.1), 0.1)
         a, t, _, _ = plan.build_sweep(T.Scarp._sb_spec, 8, [3.0], angles)
-        for key, value in (("fast", 0), ("precision", 64), ("lincomb", 0)):
+        for key, value in (("fast", 0), ("precision", 64)):
             plan.set_option(key, value)
             plan.reset()
             with pytest.raises(SbError, match="nodata mask"):
                 plan.sweep(a, t)
-            plan.set_option(key, {"fast": 1, "precision": 32, "lincomb": 1}[key])
+            plan.set_option(key, {"fast": 1, "precision": 32}[key])
     with pytest.raises(ValueError):
         sl.match(sl.DEMGrid(z, 1.0), T.Scarp, scale=8, age=3.0, nodata="bogus")
     sl.release()
