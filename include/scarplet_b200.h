@@ -159,6 +159,27 @@ int sb_match_template_raster(sb_plan* plan, const sb_angle* angle, const double*
                              int sy_lo, int sy_hi, int sx_lo, int sx_hi, double tscale,
                              double* amp, double* snr, int out_is_device);
 
+/* Fit surfaces at chosen pixels: post-mask amp / snr of every template at every pixel by direct
+ * float64 correlation (DESIGN §12).  out[p * n_tmpls + k] for pixel p, record k.
+ * For pixel p = (rows_host[p], cols_host[p]) and record k the values core.match_template returns
+ * there (core.py:359-375, get_err_mask and get_window_limits applied), with the FFTs replaced by
+ * sums over the template's support box in float64:
+ *   xcorr = sum t[a0 + u, b0 + v] * curv[(i - u + ny % 2) mod ny, (j - v + nx % 2) mod nx],
+ *   T3 = the same sum of M * curv**2, (a0, b0) = (ny / 2, nx / 2);
+ * t, M, curv are the library's float64 values; n and ts are fixed-order sums over the box.  A
+ * pixel's result does not depend on the other pixels of the call, their order or count, nor on
+ * the options "precision", "fast" or the FFT tiling: every sum runs in one fixed order.
+ * Nodata: SB_NODATA_PROPAGATE with a non-finite DEM cell anywhere -> NaN wherever the masks leave
+ * an entry (the reference's full-raster fft2); SB_NODATA_MASK -> the masked fit of
+ * sb_plan_set_nodata with the sums taken over the cells with V = 1.
+ * Fails without a DEM, for a pixel outside the plan's rows (row slabs) or columns, on a row slab
+ * whose halo does not hold a template's support, and for SB_KIND_RASTER records.  Output buffers
+ * are the caller's; device scratch is bounded by working through the pixels in chunks. */
+int sb_fit_surface(sb_plan* plan, const sb_angle* angles, int n_angles,
+                   const sb_template* tmpls, int n_tmpls,
+                   const int32_t* rows_host, const int32_t* cols_host, int n_pix,
+                   double* amp, double* snr, int out_is_device);
+
 /* Best-fit state (running result of core.compare over a sweep). */
 int sb_best_reset(sb_plan* plan);
 

@@ -91,6 +91,8 @@ def _declare(lib):
     lib.sb_debug_fft.argtypes = [P, c_int, c_int, c_void_p, c_void_p, c_int]
     lib.sb_debug_fft_bench.argtypes = [P, c_int, c_int, c_int, c_int, POINTER(c_float)]
     lib.sb_debug_fft_bench.restype = c_int
+    lib.sb_fit_surface.argtypes = [P, POINTER(SbAngle), c_int, POINTER(SbTemplate), c_int, c_void_p, c_void_p,
+                                   c_int, c_void_p, c_void_p, c_int]
     lib.sb_sync.argtypes = [P]
     for name in ("sb_plan_create", "sb_plan_destroy", "sb_plan_set_option",
                  "sb_plan_last_geometry", "sb_plan_profile", "sb_set_dem_host", "sb_set_dem_dev",
@@ -99,7 +101,8 @@ def _declare(lib):
                  "sb_best_state", "sb_best_pack", "sb_best_select", "sb_best_unpack",
                  "sb_compare_host", "sb_debug_fft", "sb_sync", "sb_plan_set_slab", "sb_plan_dem_rows",
                  "sb_plan_curv_stats", "sb_plan_set_curv_stats", "sb_finalize_ex", "sb_best_state_ex",
-                 "sb_best_merge", "sb_curvature_noise_moments", "sb_fill_nodata", "sb_plan_set_nodata"):
+                 "sb_best_merge", "sb_curvature_noise_moments", "sb_fill_nodata", "sb_plan_set_nodata",
+                 "sb_fit_surface"):
         getattr(lib, name).restype = c_int
     return lib
 
@@ -113,7 +116,7 @@ EXPORTED = ("sb_last_error", "sb_build_info", "sb_plan_create", "sb_plan_destroy
             "sb_debug_fft", "sb_sync", "sb_plan_set_slab", "sb_plan_dem_rows", "sb_plan_curv_stats",
             "sb_plan_set_curv_stats", "sb_plan_stream", "sb_plan_device_bytes", "sb_plan_last_fft_area",
             "sb_finalize_ex", "sb_best_state_ex", "sb_best_merge", "sb_curvature_noise_moments",
-            "sb_fill_nodata", "sb_debug_fft_bench", "sb_sweep_ex", "sb_plan_set_nodata")
+            "sb_fill_nodata", "sb_debug_fft_bench", "sb_sweep_ex", "sb_plan_set_nodata", "sb_fit_surface")
 
 
 def library_path():

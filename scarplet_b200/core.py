@@ -15,6 +15,7 @@ Plans (device workspace, twiddle tables, page-locked result buffers) are cached 
 geometry, so that a second ``match`` on a raster of the same shape pays for nothing but the
 DEM upload, the search and the result download; ``release()`` frees them.
 """
+import collections
 import threading
 
 import numpy as np
@@ -241,6 +242,49 @@ def match_scales(data, Template, scales, **kwargs):
     ages, ang_max, ang_min, single = _match_args(kwargs)
     res = _sweep(data, Template, scales, ages, ang_max, ang_min, "age_major", _masking(kwargs))
     return {s: (r if single else (r[0], r[1], r[2], r[3])) for s, r in zip(scales, res)}
+
+
+FitSurface = collections.namedtuple("FitSurface", ["amp", "snr", "ages", "angles"])
+
+
+def fit_surface(data, Template, scale, pixels, ages=None, ang_min=-np.pi / 2, ang_max=np.pi / 2,
+                nodata="propagate", min_coverage=1.0, **kwargs):
+    """Fit surfaces at chosen pixels: for every (age, orientation) template of the search that
+    ``match`` runs with the same arguments, the amplitude and SNR ``match_template`` returns at
+    each pixel (masks applied), in float64 -- how sharply the best fit is constrained in age and
+    orientation.  Computed by direct correlation over each template's support, not by
+    whole-raster FFTs (DESIGN.md section 12).
+
+    ``pixels``: ``(n, 2)`` integers ``(row, col)``.  ``ages=None``: the 35 default ages of
+    ``match``.  Returns ``FitSurface(amp, snr, ages, angles)`` with ``amp``, ``snr`` of shape
+    ``(n, len(ages), len(angles))``; ``snr.reshape(n, -1).argmax(1)`` is the flat index the search
+    picks (up to its float32 near-ties).  ``nodata`` / ``min_coverage``: see
+    ``calculate_best_fit_parameters``.  Only the built-in template classes are supported (the
+    direct path needs their on-device generators): a plugin class or constructor keyword
+    arguments raise ``ValueError``."""
+    if kwargs:
+        raise ValueError("fit_surface takes no template keyword arguments (%s): the direct path needs a "
+                         "built-in template class" % ", ".join(sorted(kwargs)))
+    spec = device_spec(Template)
+    if spec is None:
+        raise ValueError("fit_surface needs a built-in template class; %r has no on-device generator" % (Template,))
+    z, _, _ = _grid_fields(data)
+    ny, nx = np.shape(z)
+    px = np.asarray(pixels)
+    if px.size == 0:
+        px = np.zeros((0, 2), dtype=np.int64)
+    if px.ndim != 2 or px.shape[1] != 2 or px.dtype.kind not in "iu":
+        raise ValueError("pixels must be an (n, 2) integer array of (row, col)")
+    if px.size and ((px[:, 0] < 0).any() or (px[:, 0] >= ny).any() or (px[:, 1] < 0).any() or (px[:, 1] >= nx).any()):
+        raise ValueError("pixels outside the %d x %d raster" % (ny, nx))
+    ages = P.default_ages() if ages is None else np.atleast_1d(np.asarray(ages, dtype=np.float64))
+    angles = P.search_angles(ang_min, ang_max)
+    if len(px) == 0:
+        empty = np.zeros((0, len(ages), len(angles)), dtype=np.float64)
+        return FitSurface(empty, empty.copy(), ages, angles)
+    with _plan_for(data, nodata=nodata, min_coverage=min_coverage) as plan:
+        amp, snr = plan.fit_surface(spec, scale, ages, angles, px[:, 0], px[:, 1])
+    return FitSurface(amp, snr, ages, angles)
 
 
 def compare(results, ny, nx):

@@ -1073,6 +1073,135 @@ SB_GLOBAL k_render_template(int ny, int nx, Tmpl p, const double* SB_RESTRICT xv
     out[i] = w;
 }
 
+// ---------------------------------------------------------------------------
+// Fit surfaces at chosen pixels (sb_fit_surface, DESIGN.md section 12): the post-mask amp / snr of
+// core.py:359-375 of every template at every pixel, by direct float64 sums over the template's
+// support box instead of FFTs:
+//     xcorr(i, j) = sum_{u,v} t[a0 + u, b0 + v] * curv[(i - u + ny % 2) mod ny, (j - v + nx % 2) mod nx]
+//     T3(i, j)    = the same sum of M * curv**2
+// A job is up to kFsAges templates of ONE search angle (the ages of an orientation); grid
+// (jobs, groups of kFsPix pixels), warp w = template w of the job, lane l = pixel l of the group.
+// The union of the job's support boxes is walked in row-major tiles of kFsTile cells: the
+// curvature of the group's pixels over a tile is staged in shared memory once for all the
+// job's templates, the values of a template once for all pixels.  Each (pixel, template) pair
+// is summed by ONE thread, sequentially, in row-major order over the template's own box (cells
+// outside it have t = 0 and are skipped), so its bits do not depend on the other pixels or
+// templates of the call, on their order or on the batching.  n = sum(M) and ts = sum(t**2) are
+// summed the same way by every lane.
+// MASKED (SB_NODATA_MASK): the sums run over the cells with V = 1 only (selected, never
+// multiplied: the float64 curvature is not finite there); n_valid and ts_m are summed alongside.
+// ---------------------------------------------------------------------------
+constexpr int kFsAges = 8;                // templates per job = warps per CTA
+constexpr int kFsPix = 32;                // pixels per CTA = lanes
+constexpr int kFsTile = 128;              // support cells per shared-memory tile
+constexpr int kFsPitch = kFsPix + 1;      // curvature tile row pitch (doubles): conflict-free both ways
+constexpr size_t kFsSmem = (size_t)(kFsTile * kFsPitch + kFsAges * kFsTile) * sizeof(double);
+
+struct FsJob {
+    int first, count;             // templates order[first .. first + count - 1], all of one angle
+    int uy_lo, ux_lo, uw, cells;  // union of their support boxes: top-left offset, width, cells
+};
+
+template <bool MASKED>
+SB_GLOBAL SB_LAUNCH_BOUNDS(kFsAges * kFsPix, 1)
+k_fit_surface(int ny, int nx, int row0, int drows, const double* SB_RESTRICT diffs, const double* SB_RESTRICT dem,
+              const Angle* SB_RESTRICT angles, const Tmpl* SB_RESTRICT tmpls, const int* SB_RESTRICT order,
+              const FsJob* SB_RESTRICT jobs, int n_tmpls, const int* SB_RESTRICT rows, const int* SB_RESTRICT cols, int n_pix,
+              const double* SB_RESTRICT xvec, const double* SB_RESTRICT yvec, int poison, double min_coverage,
+              double* SB_RESTRICT amp, double* SB_RESTRICT snr) {
+    double* cv = (double*)sb_shared();                 // [cell][kFsPitch]: curvature of the group's pixels
+    double* tv = cv + kFsTile * kFsPitch;              // [template][cell]: template values
+    const FsJob job = jobs[sb_bx()];
+    const int w = sb_tid() / kFsPix, lane = sb_tid() % kFsPix;
+    const int p0 = sb_by() * kFsPix;
+    const bool has_t = w < job.count;
+    const int k = has_t ? order[job.first + w] : order[job.first];
+    const Tmpl p = tmpls[k];
+    const Angle ang = angles[p.angle_id];
+    const long plane = (long)drows * nx;
+    const int a0 = ny / 2, b0 = nx / 2, oy = ny & 1, ox = nx & 1;
+
+    double xc = 0.0, t3 = 0.0, ts = 0.0, tsm = 0.0;
+    int n = 0, nv = 0;
+#pragma unroll 1
+    for (int f0 = 0; f0 < job.cells; f0 += kFsTile) {
+        // curvature at (pixel - offset) for every cell of the tile: consecutive threads take
+        // consecutive cells of one pixel (adjacent DEM columns)
+#pragma unroll 1
+        for (int e = sb_tid(); e < kFsTile * kFsPix; e += kFsAges * kFsPix) {
+            const int c = e % kFsTile, q = e / kFsTile, f = f0 + c;
+            double val = 0.0;
+            if (f < job.cells && p0 + q < n_pix) {
+                const int gi = wrap_near(rows[p0 + q] - (job.uy_lo + f / job.uw) + oy, ny);
+                const int gj = wrap_near(cols[p0 + q] - (job.ux_lo + f % job.uw) + ox, nx);
+                const int li = gi - row0 < 0 ? gi - row0 + ny : gi - row0;
+                const long o = (long)li * nx + gj;
+                val = combine_curvature(sb_ldg(diffs + o), sb_ldg(diffs + plane + o), sb_ldg(diffs + 2 * plane + o), ang);
+                if (MASKED && !stencil_finite(dem, ny, nx, gi, li, drows, gj)) val = NAN;   // V = 0
+            }
+            cv[c * kFsPitch + q] = val;
+        }
+        // rows of the tile; a template whose box misses them has nothing here
+        const int r_lo = job.uy_lo + f0 / job.uw;
+        const int f1 = f0 + kFsTile < job.cells ? f0 + kFsTile : job.cells;       // tile end
+        const int r_hi = job.uy_lo + (f1 - 1) / job.uw;
+        const bool live = has_t && r_hi >= p.sy_lo && r_lo <= p.sy_hi;
+        if (live) {
+            for (int c = lane; c < kFsTile; c += kFsPix) {
+                const int f = f0 + c;
+                const int u = job.uy_lo + f / job.uw, v = job.ux_lo + f % job.uw;
+                double t = 0.0;
+                if (f < job.cells && u >= p.sy_lo && u <= p.sy_hi && v >= p.sx_lo && v <= p.sx_hi)
+                    t = template_at(p, sb_ldg(xvec + b0 + v), sb_ldg(yvec + a0 + u));
+                tv[w * kFsTile + c] = t;
+            }
+        }
+        sb_sync();
+        if (live) {
+#pragma unroll 4
+            for (int c = 0; c < f1 - f0; ++c) {
+                const double t = tv[w * kFsTile + c];
+                if (t == 0.0) continue;                               // M = t != 0 (core.py:348)
+                const double cc = cv[c * kFsPitch + lane];
+                n += 1;
+                ts = fma(t, t, ts);
+                if (MASKED && cc != cc) continue;                     // V = 0: not part of the fit
+                xc = fma(t, cc, xc);                                  // core.py:359
+                t3 = t3 + sb_mul(cc, cc);                             // core.py:355, 363
+                if (MASKED) {
+                    nv += 1;
+                    tsm = fma(t, t, tsm);
+                }
+            }
+        }
+        sb_sync();
+    }
+    const int px = p0 + lane;
+    if (!has_t || px >= n_pix) return;
+    const int i = rows[px], j = cols[px];
+    double nn = sb_add((double)n, kEps), tss = ts;                  // core.py:350, 356
+    bool cand = true;
+    if (MASKED) {
+        const int li = i - row0 < 0 ? i - row0 + ny : i - row0;
+        cand = finite_cell(sb_ldg(dem + (long)li * nx + j)) && nv >= (int)ceil(min_coverage * (double)n);
+        if (nv != n) { nn = sb_add((double)nv, kEps); tss = tsm; }
+    }
+    // core.py:360-367, operation for operation
+    double a = sb_div(xc, tss);
+    const double t1 = sb_mul(tss, sb_mul(a, a));
+    const double err = sb_add(sb_mul(sb_div(1.0, nn), sb_add(sb_sub(t1, sb_mul(sb_mul(2.0, a), xc)), t3)), kEps);
+    double s = fabs(sb_div(t1, err));
+    if (poison) { a = NAN; s = NAN; }                               // a NaN in the DEM reaches every pixel (section 4)
+    if (!cand) { a = 0.0; s = 0.0; }
+    if (p.errmode != 0) {                                             // core.py:369-371
+        const double xr = sb_add(sb_mul(sb_ldg(xvec + j), p.ca), sb_mul(sb_ldg(yvec + i), p.sa));
+        if ((p.errmode == 1 && xr <= 0.0) || (p.errmode == 2 && xr >= 0.0)) s = 0.0;
+    }
+    if (i < p.i_lo || i > p.i_hi || j < p.j_lo || j > p.j_hi) { a = 0.0; s = 0.0; }   // core.py:373-375
+    amp[(long)px * n_tmpls + k] = a;
+    snr[(long)px * n_tmpls + k] = s;
+}
+
 // core.compare (core.py:198-243) on full planes with the reference's exact
 // semantics (strict compares; an exact tie zeroes the pixel).  this_age / this_angle
 // are scalars when the pointers are null.

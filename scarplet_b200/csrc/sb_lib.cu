@@ -112,6 +112,7 @@ struct sb_plan {
     int nodata_req = SB_NODATA_PROPAGATE, nodata = SB_NODATA_PROPAGATE;
     double min_cov_req = 1.0, min_cov = 1.0;
     Buf fitm;
+    Buf fs_idx, fs_out;            // sb_fit_surface: jobs, template order and pixels; output chunk
     int profile = 0;
     std::vector<sb_event_t> ev_pool;
     struct EvPair { int kind; sb_event_t a, b; };
@@ -1073,7 +1074,7 @@ int sb_plan_destroy(sb_plan* pl) {
     for (auto e : pl->ev_pool) sb_rt_event_destroy(e);
     for (Buf* b : {&pl->cr, &pl->fct, &pl->trt, &pl->part, &pl->gbuf, &pl->sums, &pl->fit, &pl->tmpls, &pl->angles,
                    &pl->tables, &pl->raw, &pl->tbox, &pl->slots, &pl->cross, &pl->casa, &pl->aux, &pl->spec9, &pl->coef,
-                   &pl->fitm})
+                   &pl->fitm, &pl->fs_idx, &pl->fs_out})
         release(*b);
 #ifndef SB_EMU
     if (pl->own_stream) cudaStreamDestroy(pl->stream);
@@ -1178,7 +1179,7 @@ long sb_plan_device_bytes(const sb_plan* pl) {
     b += (size_t)pl->bn() * pl->n_states * pl->best_copies * 12;
     for (const Buf* q : {&pl->cr, &pl->fct, &pl->trt, &pl->part, &pl->gbuf, &pl->sums, &pl->fit, &pl->tmpls, &pl->angles,
                          &pl->tables, &pl->raw, &pl->tbox, &pl->slots, &pl->cross, &pl->casa, &pl->aux, &pl->spec9, &pl->coef,
-                         &pl->fitm})
+                         &pl->fitm, &pl->fs_idx, &pl->fs_out})
         b += q->cap;
     return (long)b;
 }
@@ -1314,6 +1315,107 @@ int sb_match_template_raster(sb_plan* pl, const sb_angle* angle, const double* b
     t.sy_lo = sy_lo; t.sy_hi = sy_hi; t.sx_lo = sx_lo; t.sx_hi = sx_hi;
     t.i_lo = 0; t.i_hi = pl->ny - 1; t.j_lo = 0; t.j_hi = pl->nx - 1;     // masks are the caller's
     return sb_match_template(pl, angle, &t, amp, snr, out_is_device);
+}
+
+int sb_fit_surface(sb_plan* pl, const sb_angle* angles, int n_angles, const sb_template* tmpls, int n_tmpls,
+                   const int32_t* rows_host, const int32_t* cols_host, int n_pix, double* amp, double* snr,
+                   int out_is_device) {
+    if (!pl || !angles || !tmpls || (n_pix > 0 && (!rows_host || !cols_host || !amp || !snr)))
+        return fail("sb_fit_surface: null");
+    if (!pl->d_dem) return fail("sb_fit_surface: no DEM set (sb_set_dem_host / sb_set_dem_dev)");
+    if (!pl->d_x || !pl->d_y) return fail("sb_fit_surface: no axis vectors set (sb_set_axes_host)");
+    if (n_angles <= 0 || n_tmpls <= 0 || n_pix < 0) return fail("sb_fit_surface: bad counts");
+    int lo_y = 0, hi_y = 0;
+    for (int k = 0; k < n_tmpls; ++k) {
+        const sb_template& t = tmpls[k];
+        if (t.kind != SB_KIND_SCARP && t.kind != SB_KIND_RICKER)
+            return fail("sb_fit_surface: template " + std::to_string(k) +
+                        " has no on-device generator (raster / plugin templates are not supported)");
+        if (t.angle_id < 0 || t.angle_id >= n_angles) return fail("sb_fit_surface: template angle_id out of range");
+        if (t.sy_hi < t.sy_lo || t.sx_hi < t.sx_lo) return fail("sb_fit_surface: empty template support box");
+        if (t.sy_lo < -(pl->ny / 2) || t.sy_hi > pl->ny - 1 - pl->ny / 2 || t.sx_lo < -(pl->nx / 2) ||
+            t.sx_hi > pl->nx - 1 - pl->nx / 2)
+            return fail("sb_fit_surface: template support box exceeds the raster");
+        lo_y = std::min(lo_y, t.sy_lo);
+        hi_y = std::max(hi_y, t.sy_hi);
+    }
+    // pixels: the plan's own rows; on a row slab the curvature rows (+ 1 for the stencil) of every
+    // template must lie inside the DEM rows the plan holds (as run_sweep_t requires of its tiles)
+    const long have_lo = (long)pl->slab_lo - (pl->slab_lo - pl->row0 + (pl->slab_lo < pl->row0 ? pl->ny : 0));
+    for (int q = 0; q < n_pix; ++q) {
+        const int r = rows_host[q], c = cols_host[q];
+        if (c < 0 || c >= pl->nx || r < pl->slab_lo || r >= pl->slab_hi)
+            return fail("sb_fit_surface: pixel " + std::to_string(q) + " (" + std::to_string(r) + ", " +
+                        std::to_string(c) + ") outside rows " + std::to_string(pl->slab_lo) + ".." +
+                        std::to_string(pl->slab_hi - 1) + " / columns 0.." + std::to_string(pl->nx - 1) + " of the plan");
+        const long first = (long)r + (pl->ny & 1) - hi_y - 1, last = (long)r + (pl->ny & 1) - lo_y + 1;
+        if (pl->drows < pl->ny && (first < have_lo || last >= have_lo + pl->drows))
+            return fail("row slab: halo too small for the template support (pixel row " + std::to_string(r) +
+                        " needs rows " + std::to_string(first) + ".." + std::to_string(last) + ", have " +
+                        std::to_string(have_lo) + ".." + std::to_string(have_lo + pl->drows - 1) + ")");
+    }
+    if (n_pix == 0) return 0;
+
+    // jobs: up to kFsAges templates of one angle (caller order within the angle), with the union of their boxes
+    std::vector<int> order(n_tmpls);
+    for (int k = 0; k < n_tmpls; ++k) order[k] = k;
+    std::stable_sort(order.begin(), order.end(), [&](int a, int b) { return tmpls[a].angle_id < tmpls[b].angle_id; });
+    std::vector<sb::FsJob> jobs;
+    for (int s = 0; s < n_tmpls;) {
+        int e = s + 1;
+        while (e < n_tmpls && e - s < sb::kFsAges && tmpls[order[e]].angle_id == tmpls[order[s]].angle_id) ++e;
+        int y0 = tmpls[order[s]].sy_lo, y1 = tmpls[order[s]].sy_hi, x0 = tmpls[order[s]].sx_lo, x1 = tmpls[order[s]].sx_hi;
+        for (int k = s + 1; k < e; ++k) {
+            const sb_template& t = tmpls[order[k]];
+            y0 = std::min(y0, t.sy_lo); y1 = std::max(y1, t.sy_hi);
+            x0 = std::min(x0, t.sx_lo); x1 = std::max(x1, t.sx_hi);
+        }
+        const long cells = (long)(y1 - y0 + 1) * (x1 - x0 + 1);
+        if (cells > 0x7fffffffL) return fail("sb_fit_surface: template support box too large");
+        jobs.push_back({s, e - s, y0, x0, x1 - x0 + 1, (int)cells});
+        s = e;
+    }
+    const int n_jobs = (int)jobs.size();
+    const size_t jobs_b = jobs.size() * sizeof(sb::FsJob), ints_b = sizeof(int32_t) * ((size_t)n_tmpls + 2 * (size_t)n_pix);
+    SB_OK(ensure(pl->fs_idx, jobs_b + ints_b));
+    SB_OK(ensure(pl->tmpls, (size_t)n_tmpls * sizeof(sb::Tmpl)));
+    SB_OK(ensure(pl->angles, (size_t)n_angles * sizeof(sb::Angle)));
+    char* base = (char*)pl->fs_idx.p;
+    const sb::FsJob* d_jobs = (const sb::FsJob*)base;
+    const int* d_order = (const int*)(base + jobs_b);
+    const int* d_rows = d_order + n_tmpls;
+    const int* d_cols = d_rows + n_pix;
+    SB_TRY(sb_rt_h2d(base, jobs.data(), jobs_b, pl->stream));
+    SB_TRY(sb_rt_h2d((void*)d_order, order.data(), (size_t)n_tmpls * sizeof(int), pl->stream));
+    SB_TRY(sb_rt_h2d((void*)d_rows, rows_host, (size_t)n_pix * sizeof(int32_t), pl->stream));
+    SB_TRY(sb_rt_h2d((void*)d_cols, cols_host, (size_t)n_pix * sizeof(int32_t), pl->stream));
+    SB_TRY(sb_rt_h2d(pl->tmpls.p, tmpls, (size_t)n_tmpls * sizeof(sb::Tmpl), pl->stream));
+    SB_TRY(sb_rt_h2d(pl->angles.p, angles, (size_t)n_angles * sizeof(sb::Angle), pl->stream));
+    SB_OK(ensure_diffs64(pl));
+
+    // pixel chunks: at most 256 MB of output per launch (2 doubles per pixel and template)
+    long chunk = ((256L << 20) / (16L * n_tmpls)) / sb::kFsPix * sb::kFsPix;
+    chunk = std::max<long>(sb::kFsPix, std::min<long>(chunk, 1L << 20));
+    if (!out_is_device) SB_OK(ensure(pl->fs_out, (size_t)std::min<long>(chunk, n_pix) * n_tmpls * 2 * sizeof(double)));
+    const bool masked = pl->nodata == SB_NODATA_MASK;
+    auto kern = masked ? sb::k_fit_surface<true> : sb::k_fit_surface<false>;
+    for (long p0 = 0; p0 < n_pix; p0 += chunk) {
+        const int cnt = (int)std::min<long>(chunk, n_pix - p0);
+        const size_t off = (size_t)p0 * n_tmpls, vals = (size_t)cnt * n_tmpls;
+        double* d_amp = out_is_device ? amp + off : (double*)pl->fs_out.p;
+        double* d_snr = out_is_device ? snr + off : d_amp + vals;
+        SB_OK(launch(pl, "k_fit_surface", kern, dim3(n_jobs, div_up(cnt, sb::kFsPix)), dim3(sb::kFsAges * sb::kFsPix),
+                     sb::kFsSmem, pl->ny, pl->nx, pl->row0, pl->drows, (const double*)pl->d_diffs,
+                     (const double*)pl->d_dem, (const sb::Angle*)pl->angles.p, (const sb::Tmpl*)pl->tmpls.p, d_order,
+                     d_jobs, n_tmpls, d_rows + p0, d_cols + p0, cnt, (const double*)pl->d_x, (const double*)pl->d_y,
+                     pl->dem_nonfinite ? 1 : 0, pl->min_cov, d_amp, d_snr));
+        if (!out_is_device) {
+            SB_TRY(sb_rt_d2h(amp + off, d_amp, vals * sizeof(double), pl->stream));
+            SB_TRY(sb_rt_d2h(snr + off, d_snr, vals * sizeof(double), pl->stream));
+        }
+    }
+    SB_TRY(sb_rt_sync(pl->stream));
+    return 0;
 }
 
 int sb_best_reset(sb_plan* pl) {

@@ -253,6 +253,32 @@ class Plan(object):
             int(cols[0]) - b0, int(cols[-1]) - b0, tscale, amp.ctypes.data, snr.ctypes.data, 0))
         return amp, snr
 
+    def fit_surface(self, spec, scale, ages, angles, rows, cols):
+        """Fit surfaces at pixels ``(rows[p], cols[p])`` (``sb_fit_surface``, DESIGN.md section 12):
+        float64 ``(amp, snr)`` of shape ``(n_pix, len(ages), len(angles))``, the post-mask values
+        ``match_template`` returns there for every (age, angle), by direct correlation.  The records
+        are in the sweep's ``age_major`` order, so ``snr.reshape(n_pix, -1)`` is indexed by the flat
+        index a search over the same ages and angles decodes."""
+        ages = np.atleast_1d(np.asarray(ages, dtype=np.float64))
+        angles = np.atleast_1d(np.asarray(angles, dtype=np.float64))
+        rows = np.ascontiguousarray(rows, dtype=np.int32)
+        cols = np.ascontiguousarray(cols, dtype=np.int32)
+        if rows.shape != cols.shape or rows.ndim != 1:
+            raise ValueError("rows and cols must be 1-D and of equal length")
+        A, G, n = len(angles), len(ages), len(rows)
+        arr_a = (SbAngle * max(A, 1))()
+        for k, a in enumerate(angles):
+            arr_a[k] = P.angle_record(a)
+        ai, gi = np.meshgrid(np.arange(A), np.arange(G), indexing="ij")
+        recs = P.template_records(spec, scale, ages, angles, self.nx, self.ny, self.dx, self.x, self.y,
+                                  np.arange(A), gi * A + ai)                       # [A, G]
+        arr_t = P.records_to_ctypes(np.ascontiguousarray(recs.T))               # k = age * A + angle
+        amp = np.empty((n, G, A), dtype=np.float64)
+        snr = np.empty((n, G, A), dtype=np.float64)
+        check(self.lib, self.lib.sb_fit_surface(self._h, arr_a, A, arr_t, A * G, rows.ctypes.data, cols.ctypes.data,
+                                                n, amp.ctypes.data, snr.ctypes.data, 0))
+        return amp, snr
+
     # -- sweeps ------------------------------------------------------------------
     def build_sweep(self, spec, scale, ages, angles, order="age_major", angle_slice=None, template_share=None):
         """Records for the fan-out over ``angles`` x ``ages``.
