@@ -207,6 +207,21 @@ int sb_finalize(sb_plan* plan, const double* age_of_host, const double* angle_of
 int sb_finalize_ex(sb_plan* plan, int state, int row_lo, int row_hi, const double* age_of_host,
                    const double* angle_of_host, int n_idx, double* out4, int out_is_device);
 
+/* Age-resolved search (DESIGN §13): best states 0 .. n_states-1 hold one age each (state s = the
+ * templates of ages[s]).  For raster rows row_lo .. row_hi-1 writes out6 = float64[6][rows][nx]:
+ *   [0..3] amp, age, angle, snr of the fold over the states (highest SNR, then lowest flat index,
+ *          a NaN SNR sticks), decoded as sb_finalize_ex decodes a state;
+ *   [4], [5] age_lo, age_hi: the smallest / largest age_of[idx_s] over the states s with
+ *          snr_s > 0 and (double)snr_s >= snr_ratio * (double)snr_best; 0 where the fold's snr is
+ *          0 or NaN (like its age plane).
+ * The fold is the one the single-state sweep runs over the same templates, so planes 0..3 equal
+ * sb_finalize_ex after a sweep with every record in state 0.  The states are read, not modified.
+ * Fails for snr_ratio outside (0, 1], n_states outside 1 .. option "states", and rows outside the
+ * plan's rows. */
+int sb_age_range(sb_plan* plan, int n_states, int row_lo, int row_hi, double snr_ratio,
+                 const double* age_of_host, const double* angle_of_host, int n_idx,
+                 double* out6, int out_is_device);
+
 /* Raw best state for a cross-GPU merge: device pointers into the plan, one value per pixel of
  * the plan's rows. */
 int sb_best_state(sb_plan* plan, float** snr_dev, float** amp_dev, int32_t** idx_dev);

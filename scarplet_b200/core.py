@@ -287,6 +287,69 @@ def fit_surface(data, Template, scale, pixels, ages=None, ang_min=-np.pi / 2, an
     return FitSurface(amp, snr, ages, angles)
 
 
+def _age_search(name, Template, ages, kwargs, snr_ratio=None):
+    """(device spec, float64 ages) of an age-resolved search; ``ValueError`` for what it does not take."""
+    if kwargs:
+        raise ValueError("%s takes no template keyword arguments (%s): the per-age states need a built-in "
+                         "template class" % (name, ", ".join(sorted(kwargs))))
+    spec = device_spec(Template)
+    if spec is None:
+        raise ValueError("%s needs a built-in template class; %r has no on-device generator" % (name, Template))
+    ages = P.default_ages() if ages is None else np.atleast_1d(np.asarray(ages, dtype=np.float64))
+    if ages.ndim != 1 or not 1 <= len(ages) <= 64:
+        raise ValueError("%s takes 1 .. 64 ages (one best state each), not %d" % (name, ages.size))
+    if len(np.unique(ages)) != len(ages):
+        raise ValueError("%s: duplicate ages" % name)
+    if snr_ratio is not None and not (np.isfinite(snr_ratio) and 0.0 < snr_ratio <= 1.0):
+        raise ValueError("snr_ratio must be in (0, 1], not %r" % (snr_ratio,))
+    return spec, ages
+
+
+def _age_sweep(plan, spec, scale, ages, ang_min, ang_max):
+    angles = P.search_angles(ang_min, ang_max)
+    a_rec, t_rec, age_of, angle_of = plan.build_sweep(spec, scale, ages, angles, "age_major", state_per_age=True)
+    plan.reset()
+    plan.sweep(a_rec, t_rec)
+    return age_of, angle_of
+
+
+def match_ages(data, Template, scale, ages=None, ang_min=-np.pi / 2, ang_max=np.pi / 2, nodata="propagate",
+               min_coverage=1.0, **kwargs):
+    """The best fit over orientations at EVERY age, from one device sweep: ``{age: (4, ny, nx)}``,
+    entry ``a`` being what ``calculate_best_fit_parameters(data, Template, scale, a, ...)`` returns
+    (up to the float32 rounding of the FFT pipeline) -- the per-age results ``match`` folds
+    (core.py:288-291), e.g. the SNR as a function of age at every pixel.  Each age folds into its
+    own best state (DESIGN.md section 13); the values are views into one (len(ages), 4, ny, nx)
+    array.  ``ages=None``: the 35 default ages.  Device memory: the best states take 12 B x ages per
+    pixel (x the fit kernel's sub-stream copies on small rasters): 6 GB at 4096^2 with 30 ages.
+    Built-in template classes only, at most 64 distinct ages; ``nodata`` / ``min_coverage``: see
+    ``calculate_best_fit_parameters``."""
+    spec, ages = _age_search("match_ages", Template, ages, kwargs)
+    z, _, _ = _grid_fields(data)
+    ny, nx = np.shape(z)
+    with _plan_for(data, states=len(ages), nodata=nodata, min_coverage=min_coverage) as plan:
+        age_of, angle_of = _age_sweep(plan, spec, scale, ages, ang_min, ang_max)
+        out = np.empty((len(ages), 4, ny, nx), dtype=np.float64)
+        for s in range(len(ages)):
+            plan.finalize(age_of, angle_of, state=s, out=out[s])
+    return {float(a): out[s] for s, a in enumerate(ages)}
+
+
+def age_range(data, Template, scale, snr_ratio, ages=None, ang_min=-np.pi / 2, ang_max=np.pi / 2,
+              nodata="propagate", min_coverage=1.0, **kwargs):
+    """The age range each pixel's SNR supports: (6, ny, nx) float64 [amp, age, angle, snr, age_lo,
+    age_hi].  Planes 0..3 are exactly ``match(data, Template, scale=scale, ages=ages, ...)``;
+    ``age_lo`` / ``age_hi`` are the smallest / largest age whose best fit over the orientations has
+    an SNR of at least ``snr_ratio`` (in (0, 1]) times the pixel's best (compared in float64), 0
+    where the pixel has no fit.  One device sweep with one best state per age, reduced on the
+    device: 48 B per pixel cross PCIe whatever the number of ages.  Arguments, limits and device
+    memory as ``match_ages``."""
+    spec, ages = _age_search("age_range", Template, ages, kwargs, snr_ratio)
+    with _plan_for(data, states=len(ages), nodata=nodata, min_coverage=min_coverage) as plan:
+        age_of, angle_of = _age_sweep(plan, spec, scale, ages, ang_min, ang_max)
+        return plan.age_range(age_of, angle_of, snr_ratio)
+
+
 def compare(results, ny, nx):
     """Per-pixel best-SNR select over an iterable of ``(amp, age, angle, snr)``
     (core.py:198-243), with the reference's exact semantics (strict compares, an

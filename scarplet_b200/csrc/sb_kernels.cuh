@@ -1005,23 +1005,88 @@ SB_GLOBAL k_best_fold(long n, int n_extra, long stride, const float* SB_RESTRICT
     if (changed) { snr[i] = bs; amp[i] = ba; idx[i] = bi; }
 }
 
+// One pixel of a best state (SNR s, flat index k, amplitude *amp -- read only for a hit) as the
+// reference's [amp, age, angle, snr] float64 values (core.py:190-193)
+SB_DEVICE void decode_best(float s, int k, const float* SB_RESTRICT amp, const double* SB_RESTRICT age_of,
+                           const double* SB_RESTRICT angle_of, int n_idx, double (&o)[4]) {
+    const bool hit = s > 0.f && k >= 0 && k < n_idx;
+    // NaN in the DEM (dem.py:105): compare's select leaves NaN in amp and snr and 0 in age and
+    // angle wherever some template was un-masked (SURVEY 8a-5)
+    const bool nan = s != s;
+    const double qnan = (double)s;
+    o[0] = nan ? qnan : hit ? (double)*amp : 0.0;
+    o[1] = hit ? age_of[k] : 0.0;
+    o[2] = hit ? angle_of[k] : 0.0;
+    o[3] = nan ? qnan : hit ? (double)s : 0.0;
+}
+
 // decode the best state into the reference's [amp, age, angle, snr] float64 planes
 SB_GLOBAL k_finalize(long n, const float* SB_RESTRICT snr, const float* SB_RESTRICT amp,
                      const int* SB_RESTRICT idx, const double* SB_RESTRICT age_of,
                      const double* SB_RESTRICT angle_of, int n_idx, double* SB_RESTRICT out4) {
     const long i = (long)sb_bx() * 256 + sb_tid();
     if (i >= n) return;
-    const float s = snr[i];
-    const int k = idx[i];
-    const bool hit = s > 0.f && k >= 0 && k < n_idx;
-    // NaN in the DEM (dem.py:105): compare's select leaves NaN in amp and snr and 0 in age and
-    // angle wherever some template was un-masked (SURVEY 8a-5)
-    const bool nan = s != s;
-    const double qnan = (double)s;
-    out4[i] = nan ? qnan : hit ? (double)amp[i] : 0.0;
-    out4[n + i] = hit ? age_of[k] : 0.0;
-    out4[2 * n + i] = hit ? angle_of[k] : 0.0;
-    out4[3 * n + i] = nan ? qnan : hit ? (double)s : 0.0;
+    double o[4];
+    decode_best(snr[i], idx[i], amp + i, age_of, angle_of, n_idx, o);
+    out4[i] = o[0];
+    out4[n + i] = o[1];
+    out4[2 * n + i] = o[2];
+    out4[3 * n + i] = o[3];
+}
+
+// Age-resolved search (sb_age_range): best state s (pixel i at [s * stride + i]) holds the best fit
+// over the orientations at age s.  Folds the n_states states with k_best_merge's rule -- the fold
+// the single-state sweep runs in the fit kernel, so planes 0..3 are what k_finalize gives for it --
+// and writes [amp, age, angle, snr, age_lo, age_hi]: age_lo / age_hi are the smallest / largest
+// decoded age over the states with snr_s > 0 and (double)snr_s >= ratio * (double)snr_best, 0 where
+// the fold has no hit (SNR 0 or NaN).  SNRs are read per state (coalesced); idx only to break an SNR tie and
+// for the states that count, amp only for the winner.
+SB_GLOBAL k_age_range(long n, long stride, int n_states, const float* SB_RESTRICT snr, const float* SB_RESTRICT amp,
+                      const int* SB_RESTRICT idx, const double* SB_RESTRICT age_of,
+                      const double* SB_RESTRICT angle_of, int n_idx, double ratio, double* SB_RESTRICT out6) {
+    const long i = (long)sb_bx() * 256 + sb_tid();
+    if (i >= n) return;
+    float bs = snr[i];
+    int bst = 0, bi = 0;
+    bool have_bi = false;                       // bi = idx of state bst (read on the first tie)
+    for (int s = 1; s < n_states; ++s) {
+        if (bs != bs) break;
+        const float v = snr[(long)s * stride + i];
+        bool take = v != v || v > bs;
+        if (!take && v == bs) {
+            if (!have_bi) { bi = idx[(long)bst * stride + i]; have_bi = true; }
+            const int k = idx[(long)s * stride + i];
+            take = k < bi;
+            if (take) bi = k;
+        } else if (take) {
+            have_bi = false;
+        }
+        if (take) { bs = v; bst = s; }
+    }
+    const long b = (long)bst * stride + i;
+    const int kb = bs > 0.f ? (have_bi ? bi : idx[b]) : -1;
+    double o[4];
+    decode_best(bs, kb, amp + b, age_of, angle_of, n_idx, o);
+    double lo = 0.0, hi = 0.0;
+    if (bs > 0.f && kb >= 0 && kb < n_idx) {
+        const double floor = ratio * (double)bs;
+        lo = o[1]; hi = o[1];
+        for (int s = 0; s < n_states; ++s) {
+            const float v = snr[(long)s * stride + i];
+            if (!(v > 0.f && (double)v >= floor)) continue;
+            const int k = idx[(long)s * stride + i];
+            if (k < 0 || k >= n_idx) continue;
+            const double a = age_of[k];
+            lo = a < lo ? a : lo;
+            hi = a > hi ? a : hi;
+        }
+    }
+    out6[i] = o[0];
+    out6[n + i] = o[1];
+    out6[2 * n + i] = o[2];
+    out6[3 * n + i] = o[3];
+    out6[4 * n + i] = lo;
+    out6[5 * n + i] = hi;
 }
 
 // sum over the raster of dxx**2 + dyy**2 (per-block partials, fixed order): gives the

@@ -1461,6 +1461,32 @@ int sb_finalize_ex(sb_plan* pl, int state, int row_lo, int row_hi, const double*
     return 0;
 }
 
+int sb_age_range(sb_plan* pl, int n_states, int row_lo, int row_hi, double snr_ratio, const double* age_of_host,
+                 const double* angle_of_host, int n_idx, double* out6, int out_is_device) {
+    if (!pl || !age_of_host || !angle_of_host || !out6 || n_idx <= 0) return fail("sb_age_range: bad arguments");
+    if (!(snr_ratio > 0.0 && snr_ratio <= 1.0)) return fail("sb_age_range: snr_ratio must be in (0, 1]");
+    if (n_states < 1 || n_states > pl->n_states) return fail("sb_age_range: n_states outside 1 .. option \"states\"");
+    if (row_lo < pl->slab_lo || row_hi > pl->slab_hi || row_lo >= row_hi) return fail("sb_age_range: rows outside the plan");
+    const long n = (long)(row_hi - row_lo) * pl->nx;
+    const long off = (long)(row_lo - pl->slab_lo) * pl->nx;
+    SB_OK(ensure(pl->tables, (size_t)2 * n_idx * sizeof(double)));
+    double* d_age = (double*)pl->tables.p;
+    double* d_ang = d_age + n_idx;
+    SB_TRY(sb_rt_h2d(d_age, age_of_host, (size_t)n_idx * sizeof(double), pl->stream));
+    SB_TRY(sb_rt_h2d(d_ang, angle_of_host, (size_t)n_idx * sizeof(double), pl->stream));
+    double* dst = out6;
+    if (!out_is_device) {
+        SB_OK(ensure(pl->raw, (size_t)n * 6 * sizeof(double)));
+        dst = (double*)pl->raw.p;
+    }
+    SB_OK(launch(pl, "k_age_range", sb::k_age_range, dim3(div_up(n, 256)), dim3(256), 0, n, pl->bn(), n_states,
+                 (const float*)pl->d_bsnr + off, (const float*)pl->d_bamp + off, (const int*)pl->d_bidx + off,
+                 (const double*)d_age, (const double*)d_ang, n_idx, snr_ratio, dst));
+    if (!out_is_device) return copy_out(pl, out6, dst, (size_t)n * 6, 0);
+    SB_TRY(sb_rt_sync(pl->stream));
+    return 0;
+}
+
 int sb_finalize(sb_plan* pl, const double* age_of_host, const double* angle_of_host, int n_idx, double* out4,
                 int out_is_device) {
     if (!pl) return fail("null plan");

@@ -280,7 +280,8 @@ class Plan(object):
         return amp, snr
 
     # -- sweeps ------------------------------------------------------------------
-    def build_sweep(self, spec, scale, ages, angles, order="age_major", angle_slice=None, template_share=None):
+    def build_sweep(self, spec, scale, ages, angles, order="age_major", angle_slice=None, template_share=None,
+                    state_per_age=False):
         """Records for the fan-out over ``angles`` x ``ages``.
 
         ``order`` fixes the flat result index (the tie priority of ``compare``):
@@ -295,16 +296,21 @@ class Plan(object):
         ``scale`` may be a sequence: one best state per scale (``Plan(states=len(scale))``),
         all scales of an orientation in the same sweep so that they share its curvature
         spectra; every state uses the same flat index space.
+        ``state_per_age``: the templates of ``ages[g]`` fold into best state ``g``
+        (``Plan(states=len(ages))``, read with ``age_range`` or ``finalize(state=g)``); one scale,
+        ``"age_major"`` order and at most 64 ages.  The flat indices stay those of ``match``.
         Returns ``(angle_records, template_records, age_of, angle_of)``.
         """
         ages = np.atleast_1d(np.asarray(ages, dtype=np.float64))
         angles = np.asarray(angles, dtype=np.float64)
         scales = [scale] if np.ndim(scale) == 0 else list(scale)
+        if state_per_age and (len(scales) != 1 or order != "age_major" or not 1 <= len(ages) <= 64):
+            raise ValueError("state_per_age needs one scale, age_major order and 1 .. 64 ages")
         # the records depend on the arguments and the plan's geometry only: a repeated search
         # (the same templates on the next raster of this shape) reuses them (read-only)
         key = (id(spec), tuple(float(s) for s in scales), ages.tobytes(), angles.tobytes(), order,
                None if angle_slice is None else tuple(angle_slice),
-               None if template_share is None else tuple(template_share))
+               None if template_share is None else tuple(template_share), bool(state_per_age))
         memo = getattr(self, "_sweep_memo", None)
         if memo is None:
             memo = []
@@ -312,12 +318,12 @@ class Plan(object):
         for k, sp, val in memo:
             if k == key and sp is spec:
                 return val
-        val = Plan._build_sweep(self, spec, scales, ages, angles, order, angle_slice, template_share)
+        val = Plan._build_sweep(self, spec, scales, ages, angles, order, angle_slice, template_share, state_per_age)
         memo.append((key, spec, val))
         del memo[:-4]
         return val
 
-    def _build_sweep(self, spec, scales, ages, angles, order, angle_slice, template_share):
+    def _build_sweep(self, spec, scales, ages, angles, order, angle_slice, template_share, state_per_age=False):
         A, G = len(angles), len(ages)
         lo, hi = (0, A) if angle_slice is None else angle_slice
         t_lo = t_hi = None
@@ -341,6 +347,8 @@ class Plan(object):
         recs = [P.template_records(spec, sc, ages, angles[lo:hi], self.nx, self.ny, self.dx,
                                    self.x, self.y, np.arange(hi - lo), idx[lo:hi], state=k)
                 for k, sc in enumerate(scales)]
+        if state_per_age:
+            recs[0]["state"] = np.arange(G, dtype=np.int32)[None, :]
         recs = np.stack(recs, axis=1).reshape(-1) if hi > lo else np.zeros(0, dtype=P.TEMPLATE_DTYPE)   # [angle][scale][age]
         if t_lo is not None:
             recs = recs[t_lo - lo * G * len(scales): t_hi - lo * G * len(scales)]
@@ -444,6 +452,20 @@ class Plan(object):
             raise ValueError("out must be a C-contiguous float64 array of shape %r" % ((4, hi - lo, self.nx),))
         check(self.lib, self.lib.sb_finalize_ex(self._h, int(state), lo, hi, age_of.ctypes.data,
                                                 angle_of.ctypes.data, len(age_of), out.ctypes.data, 0))
+        return out
+
+    def age_range(self, age_of, angle_of, snr_ratio, rows=None):
+        """Age-resolved search (``sb_age_range``, DESIGN.md section 13) after a sweep built with
+        ``state_per_age``: (6, rows, nx) float64 [amp, age, angle, snr, age_lo, age_hi].  Planes
+        0..3 fold the per-age states as the single-state sweep folds its templates (bit-identical
+        to ``finalize`` of that sweep); ``age_lo`` / ``age_hi`` are the smallest / largest age
+        whose best SNR is at least ``snr_ratio`` (in (0, 1]) times the pixel's best, 0 where the
+        pixel has no fit.  ``rows=(lo, hi)``: a band of the plan's rows (default: all of them)."""
+        age_of, angle_of = _as_f64(age_of), _as_f64(angle_of)
+        lo, hi = (self.row_lo, self.row_hi) if rows is None else (int(rows[0]), int(rows[1]))
+        out = np.empty((6, max(hi - lo, 0), self.nx), dtype=np.float64)
+        check(self.lib, self.lib.sb_age_range(self._h, self.states, lo, hi, float(snr_ratio), age_of.ctypes.data,
+                                              angle_of.ctypes.data, len(age_of), out.ctypes.data, 0))
         return out
 
     def finalize_device(self, age_of, angle_of, out_ptr, state=0, rows=None):
