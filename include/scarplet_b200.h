@@ -222,6 +222,37 @@ int sb_age_range(sb_plan* plan, int n_states, int row_lo, int row_hi, double snr
                  const double* age_of_host, const double* angle_of_host, int n_idx,
                  double* out6, int out_is_device);
 
+/* Fit confidence region (DESIGN §14), pass 2 of 2: best state 0 must hold the result of a sweep
+ * (sb_sweep / sb_sweep_ex) over the same records.  Runs that sweep again with the region variant
+ * of the fit kernel, which writes no best state: a record with flat index k qualifies at a pixel
+ * when the masks (window, get_err_mask, min_coverage) leave it a candidate there and its float32
+ * SNR s satisfies s > 0 and (double)s >= snr_ratio * (double)best, best = state 0's SNR.  The
+ * plan's region planes (cleared first; 4 * (3 + ceil(n_pos / 32)) bytes per pixel of the plan's
+ * rows, allocated on first use) receive per pixel the count of qualifying records, the lowest and
+ * highest age_rank_host[k] and the bits angle_pos_host[k] (in 0 .. n_pos - 1) of them.  Integer
+ * atomics: the result does not depend on batches, sub-streams or launch order.
+ * Fails for snr_ratio outside (0, 1], n_pos outside 1 .. 256, ranks / positions out of range, a
+ * record whose idx is outside 0 .. n_idx - 1 or whose state is not 0, and precision 64 or fast = 0. */
+int sb_region_sweep(sb_plan* plan, const sb_angle* angles, int n_angles, const sb_template* tmpls, int n_tmpls,
+                    const int32_t* whole_search5, double snr_ratio, const int32_t* age_rank_host,
+                    const int32_t* angle_pos_host, int n_idx, int n_pos);
+
+/* Decode the region planes for raster rows row_lo .. row_hi-1: out9 = float64[9][rows][nx]
+ *   [0..3] amp, age, angle, snr of best state 0 (as sb_finalize_ex);
+ *   [4], [5] age_lo, age_hi = rank_age_host[lowest / highest rank];
+ *   [6], [7] angle_lo, angle_hi: the shortest arc of orientation positions holding every
+ *            qualifying one.  periodic = 0: pos_angle_host[first], pos_angle_host[last].
+ *            periodic = 1 (positions 0 .. n_pos - 1 close into a circle of pi): the complement of
+ *            the largest circular gap between consecutive qualifying positions (equal gaps: the
+ *            lowest p_lo), angle_hi = pos_angle_host[p_hi] + pi when the arc wraps (p_hi < p_lo);
+ *   [8] the number of qualifying records.
+ * Planes 4..8 are 0 where state 0's SNR is 0 or NaN.  Fails without a region sweep since the best
+ * state was last allocated (option "states", sb_plan_set_slab), for n_pos other than the sweep's,
+ * fewer ranks than the sweep used, and rows outside the plan. */
+int sb_region_finalize(sb_plan* plan, int row_lo, int row_hi, const double* age_of_host,
+                       const double* angle_of_host, int n_idx, const double* rank_age_host, int n_ranks,
+                       const double* pos_angle_host, int n_pos, int periodic, double* out9, int out_is_device);
+
 /* Raw best state for a cross-GPU merge: device pointers into the plan, one value per pixel of
  * the plan's rows. */
 int sb_best_state(sb_plan* plan, float** snr_dev, float** amp_dev, int32_t** idx_dev);

@@ -287,7 +287,7 @@ def fit_surface(data, Template, scale, pixels, ages=None, ang_min=-np.pi / 2, an
     return FitSurface(amp, snr, ages, angles)
 
 
-def _age_search(name, Template, ages, kwargs, snr_ratio=None):
+def _age_search(name, Template, ages, kwargs, snr_ratio=None, max_ages=64):
     """(device spec, float64 ages) of an age-resolved search; ``ValueError`` for what it does not take."""
     if kwargs:
         raise ValueError("%s takes no template keyword arguments (%s): the per-age states need a built-in "
@@ -296,8 +296,11 @@ def _age_search(name, Template, ages, kwargs, snr_ratio=None):
     if spec is None:
         raise ValueError("%s needs a built-in template class; %r has no on-device generator" % (name, Template))
     ages = P.default_ages() if ages is None else np.atleast_1d(np.asarray(ages, dtype=np.float64))
-    if ages.ndim != 1 or not 1 <= len(ages) <= 64:
-        raise ValueError("%s takes 1 .. 64 ages (one best state each), not %d" % (name, ages.size))
+    if max_ages is None:
+        if ages.ndim != 1 or len(ages) < 1:
+            raise ValueError("%s takes at least one age" % name)
+    elif ages.ndim != 1 or not 1 <= len(ages) <= max_ages:
+        raise ValueError("%s takes 1 .. %d ages (one best state each), not %d" % (name, max_ages, ages.size))
     if len(np.unique(ages)) != len(ages):
         raise ValueError("%s: duplicate ages" % name)
     if snr_ratio is not None and not (np.isfinite(snr_ratio) and 0.0 < snr_ratio <= 1.0):
@@ -348,6 +351,39 @@ def age_range(data, Template, scale, snr_ratio, ages=None, ang_min=-np.pi / 2, a
     with _plan_for(data, states=len(ages), nodata=nodata, min_coverage=min_coverage) as plan:
         age_of, angle_of = _age_sweep(plan, spec, scale, ages, ang_min, ang_max)
         return plan.age_range(age_of, angle_of, snr_ratio)
+
+
+def fit_region(data, Template, scale, snr_ratio, ages=None, ang_min=-np.pi / 2, ang_max=np.pi / 2,
+               nodata="propagate", min_coverage=1.0, **kwargs):
+    """Fit confidence region of every pixel: the (age, orientation) templates whose SNR is at least
+    ``snr_ratio`` (in (0, 1]) times the pixel's best (compared in float64).  Returns (9, ny, nx)
+    float64 [amp, age, angle, snr, age_lo, age_hi, angle_lo, angle_hi, n_fits]:
+
+    * planes 0..3 are exactly ``match(data, Template, scale=scale, ages=ages, ...)``;
+    * ``age_lo`` / ``age_hi``: the smallest / largest age among the qualifying templates (what
+      ``age_range`` gives, without its 64-age limit);
+    * ``angle_lo`` / ``angle_hi``: the shortest orientation arc holding every qualifying
+      orientation.  A search spanning pi (the default) is periodic: -pi/2 and pi/2 are one line,
+      and an arc across it has ``angle_hi = angle + pi``, so ``angle_lo <= angle_hi < angle_lo + pi``
+      -- the strike uncertainty of the fit;
+    * ``n_fits``: the number of qualifying templates;
+
+    planes 4..8 are 0 where the pixel has no fit.  Two device sweeps on one plan: ``match``'s, then
+    a threshold pass (DESIGN.md section 14) that records the qualifying templates in 4 * (3 +
+    ceil(orientations / 32)) B per pixel of device memory, whatever the number of ages (36 B for
+    181 orientations).  Built-in template classes only, at most 256 orientations, distinct ages;
+    ``nodata`` / ``min_coverage``: see ``calculate_best_fit_parameters``."""
+    spec, ages = _age_search("fit_region", Template, ages, kwargs, snr_ratio, max_ages=None)
+    angles = P.search_angles(ang_min, ang_max)
+    if len(angles) > 256:
+        raise ValueError("fit_region takes at most 256 orientations, not %d" % len(angles))
+    tables = P.region_tables(ages, angles)
+    with _plan_for(data, nodata=nodata, min_coverage=min_coverage) as plan:
+        a_rec, t_rec, age_of, angle_of = plan.build_sweep(spec, scale, ages, angles, "age_major")
+        plan.reset()
+        plan.sweep(a_rec, t_rec)
+        plan.region_sweep(a_rec, t_rec, snr_ratio, tables)
+        return plan.region_finalize(age_of, angle_of, tables)
 
 
 def compare(results, ny, nx):

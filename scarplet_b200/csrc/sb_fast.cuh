@@ -401,6 +401,73 @@ SB_DEVICE void fit_pixel_masked(float X, float T, const FitT& k, const FitM& m, 
 }
 
 // ---------------------------------------------------------------------------
+// Fit confidence region (DESIGN.md 14): a second sweep of the same templates against best state 0
+// (the first sweep's result) records, per pixel, the templates whose SNR s satisfies s > 0 and
+// (double)s >= ratio * (double)best -- their count, the lowest and highest age rank, and a bitmask
+// of orientation positions.  Integer atomics: the planes do not depend on the order in which
+// sub-streams, batches or launches reach a pixel.
+// ---------------------------------------------------------------------------
+struct RegionOut {
+    const float* best;        // best state 0, addressed by raster row (gi * nx + gj), read only
+    int* count;               // planes of the plan's rows, addressed like `best`
+    int* rank_lo;
+    int* rank_hi;
+    unsigned* bits;           // [words][plane]: orientation position p is bit p & 31 of word p >> 5
+    const int* age_rank;      // per flat index: rank of its age among the search's ages
+    const int* angle_pos;     // per flat index: orientation position
+    long plane;               // elements of one plane
+    double ratio;
+};
+
+template <bool REGION> struct RegionSlot {};
+template <> struct RegionSlot<true> { RegionOut rg; };
+
+SB_DEVICE void sb_atomic_add(int* p, int v) {
+#ifdef SB_EMU
+    __atomic_fetch_add(p, v, __ATOMIC_RELAXED);
+#else
+    atomicAdd(p, v);
+#endif
+}
+SB_DEVICE void sb_atomic_min(int* p, int v) {
+#ifdef SB_EMU
+    int cur = __atomic_load_n(p, __ATOMIC_RELAXED);
+    while (v < cur && !__atomic_compare_exchange_n(p, &cur, v, true, __ATOMIC_RELAXED, __ATOMIC_RELAXED)) {}
+#else
+    atomicMin(p, v);
+#endif
+}
+SB_DEVICE void sb_atomic_max(int* p, int v) {
+#ifdef SB_EMU
+    int cur = __atomic_load_n(p, __ATOMIC_RELAXED);
+    while (v > cur && !__atomic_compare_exchange_n(p, &cur, v, true, __ATOMIC_RELAXED, __ATOMIC_RELAXED)) {}
+#else
+    atomicMax(p, v);
+#endif
+}
+SB_DEVICE void sb_atomic_or(unsigned* p, unsigned v) {
+#ifdef SB_EMU
+    __atomic_fetch_or(p, v, __ATOMIC_RELAXED);
+#else
+    atomicOr(p, v);
+#endif
+}
+
+// the pixel's threshold in the running-best registers: the largest float <= ratio * best (so that
+// s >= it is implied by (double)s >= ratio * best), +inf where there is no fit (best <= 0 or NaN)
+SB_DEVICE float region_threshold(float best, double ratio) {
+    if (!(best > 0.f)) return INFINITY;
+    const double x = ratio * (double)best;
+#ifdef SB_EMU
+    float f = (float)x;
+    if ((double)f > x) f = std::nextafter(f, -INFINITY);
+    return f;
+#else
+    return __double2float_rd(x);
+#endif
+}
+
+// ---------------------------------------------------------------------------
 // k_fit_rows_g<Px>: grid (Py / 2 / GP).  The two transforms
 // a thread group pipelines are the two raster rows that share every 32-byte sector of the
 // interleaved planes (gbuf_index), of ONE template: a thread fetches whole sectors with
@@ -411,8 +478,10 @@ SB_DEVICE void fit_pixel_masked(float X, float T, const FitT& k, const FitM& m, 
 // ---------------------------------------------------------------------------
 // MASKED (k_fit_rows_gm): per template, the companion's row pair runs first (comp) and parks its
 // outputs in `park`, every thread in the slots only it reads back; then the template's own.
-template <int N, bool MASKED = false>
-struct FitPairCtx {
+// REGION (k_fit_rows_gr / _gmr): bsA / bsB hold each pixel's region threshold (region_threshold) and
+// never change; a candidate is confirmed in float64 and recorded in the region planes (region_hit).
+template <int N, bool MASKED = false, bool REGION = false>
+struct FitPairCtx : RegionSlot<REGION> {
     static constexpr int K = sbfft::num_stages(N);
     static constexpr int T = N / E;
     static constexpr int LOG2T = ilog2(T);
@@ -466,6 +535,19 @@ struct FitPairCtx {
         return direct ? make_float2(g4.x, g4.y) : make_float2(g4.z, g4.w);
     }
 
+    // REGION: template `idx` has SNR `snr` >= the threshold at pixel `pix` (gi * nx + gj)
+    SB_DEVICE void region_hit(long pix, float snr, int idx) const {
+        const RegionOut& r = this->rg;
+        const float best = r.best[pix];
+        if (!(best > 0.f && (double)snr >= r.ratio * (double)best)) return;
+        sb_atomic_add(r.count + pix, 1);
+        const int rank = r.age_rank[idx];
+        sb_atomic_min(r.rank_lo + pix, rank);
+        sb_atomic_max(r.rank_hi + pix, rank);
+        const int p = r.angle_pos[idx];
+        sb_atomic_or(r.bits + (long)(p >> 5) * r.plane + pix, 1u << (p & 31));
+    }
+
     template <int F> SB_DEVICE void epilogue(const float2 (&v)[E], float (&bs)[E]) {
         const int gi = F == 0 ? giA : giB;
         const FitT k = s_fit[slot];
@@ -483,6 +565,10 @@ struct FitPairCtx {
             // (A branch-free select over the 16 pixels was measured 3 % slower: it spills.)
             if (snr >= bs[q] && snr > 0.f) {
                 const int jo = (m0 + q * T) & (N - 1);
+                if constexpr (REGION) {
+                    region_hit((long)gi * nx + ox + jo, snr, k.idx);
+                    continue;
+                }
                 if (snr > bs[q] || k.idx < pi[jo]) {
                     bs[q] = snr;
                     pa[jo] = amp;
@@ -537,6 +623,10 @@ struct FitPairCtx {
                     const float snr = q < 8 ? snr2[q & 7].x : snr2[q & 7].y;
                     const float amp = q < 8 ? amp2[q & 7].x : amp2[q & 7].y;
                     const int jo = (m0 + q * T) & (N - 1);
+                    if constexpr (REGION) {
+                        region_hit((long)gi * nx + ox + jo, snr, k.idx);
+                        continue;
+                    }
                     if (snr > bs[q] || k.idx < pi[jo]) {
                         bs[q] = snr;
                         pa[jo] = amp;
@@ -598,11 +688,12 @@ SB_CONSTEXPR size_t fit_masked_extra_smem() {
     return kFitMaxBatch * sizeof(FitM) + (size_t)((N / E > 256 ? N / E : 256) / (N / E)) * 2 * N * sizeof(float2);
 }
 
-template <int N, bool MASKED>
+template <int N, bool MASKED, bool REGION = false>
 SB_DEVICE void fit_rows_g_body(const Geom& g, int count, const int* SB_RESTRICT slots, const FitT* SB_RESTRICT fit,
                                const FitM* SB_RESTRICT fitm, int comp_off, const float4* SB_RESTRICT gbuf,
                                float* SB_RESTRICT best_snr, float* SB_RESTRICT best_amp, int* best_idx,
-                               const float2* SB_RESTRICT tw, const int4* SB_RESTRICT cross, long sub_stride) {
+                               const float2* SB_RESTRICT tw, const int4* SB_RESTRICT cross, long sub_stride,
+                               const RegionOut& rg = RegionOut()) {
     // grid.y > 1 (small rasters, whose row pairs alone do not fill the GPU): the templates of the
     // launch are dealt round-robin to grid.y sub-streams; sub-stream j folds into copy j of the
     // best state (best_* + j * sub_stride; copy 0 is the state itself) and k_best_fold merges the
@@ -612,11 +703,13 @@ SB_DEVICE void fit_rows_g_body(const Geom& g, int count, const int* SB_RESTRICT 
     // best_*: the state's planes, offset so that raster row gi is at gi * nx (row slabs).
     // `cross` (templates with get_err_mask only): per (angle, raster row) the column ranges
     // with xr > 0 (.x .. .y) and xr < 0 (.z .. .w), k_err_cross.
+    // REGION: best_* are unused; the thresholds come from rg.best (state 0 for every sub-stream)
+    // and nothing writes a best state.
     constexpr int T = N / E;
     constexpr int THREADS = T > 256 ? T : 256;
     constexpr int GP = THREADS / T;
     constexpr int PL = sbfft::padded_len(N);
-    typedef FitPairCtx<N, MASKED> Ctx;
+    typedef FitPairCtx<N, MASKED, REGION> Ctx;
     const int grp = sb_tid() / T, t = sb_tid() % T;
     float2* sm = (float2*)sb_shared();
     FitT* s_fit = (FitT*)(sm + (long)GP * 2 * PL);
@@ -683,9 +776,13 @@ SB_DEVICE void fit_rows_g_body(const Geom& g, int count, const int* SB_RESTRICT 
     c.s_fm = s_fm;
     c.park = park;
     c.comp = false;
-    best_snr += sb_by() * sub_stride;
-    best_amp += sb_by() * sub_stride;
-    best_idx += sb_by() * sub_stride;
+    if constexpr (REGION) {
+        c.rg = rg;
+    } else {
+        best_snr += sb_by() * sub_stride;
+        best_amp += sb_by() * sub_stride;
+        best_idx += sb_by() * sub_stride;
+    }
     c.best_amp = best_amp;
     c.best_idx = best_idx;
     c.cross = cross;
@@ -694,8 +791,13 @@ SB_DEVICE void fit_rows_g_body(const Geom& g, int count, const int* SB_RESTRICT 
     for (int q = 0; q < E; ++q) {
         const int jo = (t + q * T + g.dlx) & (N - 1);
         const bool in = jo < g.out_nx;
-        bsA[q] = (actA && in) ? best_snr[(long)c.giA * g.nx + g.ox + jo] : 0.f;
-        bsB[q] = (actB && in) ? best_snr[(long)c.giB * g.nx + g.ox + jo] : 0.f;
+        if constexpr (REGION) {
+            bsA[q] = (actA && in) ? region_threshold(rg.best[(long)c.giA * g.nx + g.ox + jo], rg.ratio) : INFINITY;
+            bsB[q] = (actB && in) ? region_threshold(rg.best[(long)c.giB * g.nx + g.ox + jo], rg.ratio) : INFINITY;
+        } else {
+            bsA[q] = (actA && in) ? best_snr[(long)c.giA * g.nx + g.ox + jo] : 0.f;
+            bsB[q] = (actB && in) ? best_snr[(long)c.giB * g.nx + g.ox + jo] : 0.f;
+        }
     }
     const long row_off = gbuf_index(2 * pr, 0, g.kpitch);
     const long tmpl_pitch = (long)g.Py * g.kpitch;
@@ -727,11 +829,13 @@ SB_DEVICE void fit_rows_g_body(const Geom& g, int count, const int* SB_RESTRICT 
         // buffer B is next written after the coming template's first barrier
         leapfrog<Ctx::K>(c, va, vb);
     }
+    if constexpr (!REGION) {
 #pragma unroll
-    for (int q = 0; q < E; ++q) {
-        const int jo = (t + q * T + g.dlx) & (N - 1);
-        if ((c.chg >> q) & 1u) best_snr[(long)c.giA * g.nx + g.ox + jo] = bsA[q];
-        if ((c.chg >> (q + 16)) & 1u) best_snr[(long)c.giB * g.nx + g.ox + jo] = bsB[q];
+        for (int q = 0; q < E; ++q) {
+            const int jo = (t + q * T + g.dlx) & (N - 1);
+            if ((c.chg >> q) & 1u) best_snr[(long)c.giA * g.nx + g.ox + jo] = bsA[q];
+            if ((c.chg >> (q + 16)) & 1u) best_snr[(long)c.giB * g.nx + g.ox + jo] = bsB[q];
+        }
     }
 }
 
@@ -754,6 +858,26 @@ k_fit_rows_gm(Geom g, int count, const int* SB_RESTRICT slots, const FitT* SB_RE
               long sub_stride) {
     fit_rows_g_body<N, true>(g, count, slots, fit, fitm, comp_off, gbuf, best_snr, best_amp, best_idx, tw, cross,
                              sub_stride);
+}
+
+// the threshold pass of a fit confidence region (sb_region_sweep): k_fit_rows_g / k_fit_rows_gm with
+// the region planes `rg` in place of the best state; grid.y sub-streams all read state 0
+template <int N>
+SB_GLOBAL SB_LAUNCH_BOUNDS((N / E > 256 ? N / E : 256), (N / E > 256 ? 1 : 2))
+k_fit_rows_gr(Geom g, int count, const int* SB_RESTRICT slots, const FitT* SB_RESTRICT fit,
+              const float4* SB_RESTRICT gbuf, const float2* SB_RESTRICT tw, const int4* SB_RESTRICT cross,
+              RegionOut rg) {
+    fit_rows_g_body<N, false, true>(g, count, slots, fit, nullptr, 0, gbuf, nullptr, nullptr, nullptr, tw, cross, 0,
+                                    rg);
+}
+
+template <int N>
+SB_GLOBAL SB_LAUNCH_BOUNDS((N / E > 256 ? N / E : 256), 1)
+k_fit_rows_gmr(Geom g, int count, const int* SB_RESTRICT slots, const FitT* SB_RESTRICT fit,
+               const FitM* SB_RESTRICT fitm, int comp_off, const float4* SB_RESTRICT gbuf,
+               const float2* SB_RESTRICT tw, const int4* SB_RESTRICT cross, RegionOut rg) {
+    fit_rows_g_body<N, true, true>(g, count, slots, fit, fitm, comp_off, gbuf, nullptr, nullptr, nullptr, tw, cross, 0,
+                                   rg);
 }
 
 // Hermitian split (sb_kernels.cuh) of the spectrum parked in natural order in `sm`

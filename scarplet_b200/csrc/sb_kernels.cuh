@@ -1089,6 +1089,69 @@ SB_GLOBAL k_age_range(long n, long stride, int n_states, const float* SB_RESTRIC
     out6[5 * n + i] = hi;
 }
 
+SB_DEVICE int sb_lowest_bit(unsigned m) {
+#ifdef SB_EMU
+    return __builtin_ctz(m);
+#else
+    return __ffs(m) - 1;
+#endif
+}
+
+// Fit confidence region (sb_region_finalize) over the planes the threshold pass wrote (RegionOut,
+// sb_fast.cuh; plane stride `plane`, `words` orientation words): [amp, age, angle, snr] of best
+// state 0 as k_finalize decodes it, then age_lo / age_hi = rank_age[rank_lo / rank_hi], angle_lo /
+// angle_hi = the shortest arc of positions holding every qualifying one, and the count.  Linear
+// search: [pos_angle[first], pos_angle[last]].  Periodic: the arc is the complement of the largest
+// circular gap between consecutive qualifying positions (equal gaps: the lowest p_lo), and
+// angle_hi = pos_angle[p_hi] + pi when it wraps (p_hi < p_lo).  Planes 4..8 are 0 where the pixel
+// has no fit (best SNR 0 or NaN).
+SB_GLOBAL k_region_finalize(long n, long plane, int words, const float* SB_RESTRICT snr,
+                            const float* SB_RESTRICT amp, const int* SB_RESTRICT idx, const int* SB_RESTRICT count,
+                            const int* SB_RESTRICT rank_lo, const int* SB_RESTRICT rank_hi,
+                            const unsigned* SB_RESTRICT bits, const double* SB_RESTRICT age_of,
+                            const double* SB_RESTRICT angle_of, int n_idx, const double* SB_RESTRICT rank_age,
+                            const double* SB_RESTRICT pos_angle, int n_pos, int periodic, double* SB_RESTRICT out9) {
+    const long i = (long)sb_bx() * 256 + sb_tid();
+    if (i >= n) return;
+    const float s = snr[i];
+    double o[4];
+    decode_best(s, idx[i], amp + i, age_of, angle_of, n_idx, o);
+    const int c = count[i];
+    double age_lo = 0.0, age_hi = 0.0, ang_lo = 0.0, ang_hi = 0.0;
+    if (s > 0.f && c > 0) {
+        age_lo = rank_age[rank_lo[i]];
+        age_hi = rank_age[rank_hi[i]];
+        // qualifying positions in increasing order; the largest gap between two consecutive ones
+        int first = -1, prev = -1, gap = 0, gap_lo = 0, gap_hi = 0;
+        for (int w = 0; w < words; ++w) {
+            unsigned m = bits[(long)w * plane + i];
+            while (m != 0u) {
+                const int p = 32 * w + sb_lowest_bit(m);
+                m &= m - 1u;
+                if (first < 0) first = p;
+                else if (p - prev > gap) { gap = p - prev; gap_lo = p; gap_hi = prev; }
+                prev = p;
+            }
+        }
+        int p_lo = first, p_hi = prev;
+        // periodic: the gap across the wrap has the lowest p_lo (first), so it wins a tie
+        if (periodic && first + n_pos - prev < gap) { p_lo = gap_lo; p_hi = gap_hi; }
+        if (first >= 0) {
+            ang_lo = pos_angle[p_lo];
+            ang_hi = p_hi < p_lo ? pos_angle[p_hi] + 3.141592653589793 : pos_angle[p_hi];
+        }
+    }
+    out9[i] = o[0];
+    out9[n + i] = o[1];
+    out9[2 * n + i] = o[2];
+    out9[3 * n + i] = o[3];
+    out9[4 * n + i] = age_lo;
+    out9[5 * n + i] = age_hi;
+    out9[6 * n + i] = ang_lo;
+    out9[7 * n + i] = ang_hi;
+    out9[8 * n + i] = (s > 0.f) ? (double)c : 0.0;
+}
+
 // sum over the raster of dxx**2 + dyy**2 (per-block partials, fixed order): gives the
 // curvature scale used to balance curv against curv**2 in the packed FFT
 // `dem` holds raster rows row0 .. (slab); the sum runs over its rows own_first .. own_first + own_rows - 1

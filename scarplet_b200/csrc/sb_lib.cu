@@ -113,6 +113,10 @@ struct sb_plan {
     double min_cov_req = 1.0, min_cov = 1.0;
     Buf fitm;
     Buf fs_idx, fs_out;            // sb_fit_surface: jobs, template order and pixels; output chunk
+    // fit confidence region (sb_region_sweep): planes [count][rank_lo][rank_hi][words] over the plan's
+    // rows (allocated on first use), and the per-flat-index age rank / orientation position tables
+    Buf region, rtab;
+    int region_words = 0, region_npos = 0, region_nranks = 0;
     int profile = 0;
     std::vector<sb_event_t> ev_pool;
     struct EvPair { int kind; sb_event_t a, b; };
@@ -298,6 +302,7 @@ int alloc_best(sb_plan* pl) {
         if (p) sb_rt_free(p);
     pl->d_bsnr = nullptr; pl->d_bamp = nullptr; pl->d_bidx = nullptr;
     pl->best_copies = 1;
+    pl->region_npos = 0;           // region planes of the old rows / states are void
     const size_t n = (size_t)pl->bn() * pl->n_states;
     int e = 0;
     e |= sb_rt_malloc((void**)&pl->d_bsnr, n * sizeof(float));
@@ -476,6 +481,9 @@ void fill_axis(const AxisPlan& ax, int n, const TileSpec& t, int* o, int* out_n,
 struct SweepOut {
     double* raw_amp = nullptr;
     double* raw_snr = nullptr;
+    // the threshold pass of a fit confidence region (sb_region_sweep): the fit kernel records the
+    // templates that reach each pixel's threshold in these planes; no best state changes
+    const sb::RegionOut* region = nullptr;
 };
 
 // the templates of one best state inside a chunk (one launch of the column kernel)
@@ -510,6 +518,7 @@ int run_sweep_t(sb_plan* pl, const sb_angle* angles, int n_angles, const sb_temp
     const bool masked = pl->nodata == SB_NODATA_MASK;
     if (masked && so.raw_amp) return fail("nodata mask: sb_match_template keeps the reference's NaN semantics");
     if (masked && !fast) return fail("nodata mask needs precision 32 and the option fast");
+    if (so.region && !fast) return fail("fit region needs precision 32 and the option fast");
     if (!fast) SB_OK(ensure_diffs64(pl));
 
     // order templates by search angle (then best state) so that each curvature spectrum is built once
@@ -524,6 +533,7 @@ int run_sweep_t(sb_plan* pl, const sb_angle* angles, int n_angles, const sb_temp
             return fail("raster templates go through sb_match_template_raster, one at a time");
         if (t.angle_id < 0 || t.angle_id >= n_angles) return fail("template angle_id out of range");
         if (t.state < 0 || t.state >= pl->n_states) return fail("template state out of range (option \"states\")");
+        if (so.region && t.state != 0) return fail("fit region: every record must be in best state 0 (state != 0)");
         if (t.sy_hi < t.sy_lo || t.sx_hi < t.sx_lo) return fail("empty template support box");
         if (t.sy_lo < -(pl->ny / 2) || t.sy_hi > pl->ny - 1 - pl->ny / 2 || t.sx_lo < -(pl->nx / 2) ||
             t.sx_hi > pl->nx - 1 - pl->nx / 2)
@@ -720,7 +730,8 @@ int run_sweep_t(sb_plan* pl, const sb_angle* angles, int n_angles, const sb_temp
         nsub = std::max(1, std::min(nsub, Bt / 2));
     }
     const long sub_stride = bn_all(pl);
-    if (nsub > 1) {
+    // (a region pass keeps the sub-streams, whose templates all compare with state 0: no copies)
+    if (nsub > 1 && !so.region) {
         if (nsub > pl->best_copies) {
             // grow the best-state arrays to nsub copies, keeping copy 0 (the accumulated state)
             float *s2 = nullptr, *a2 = nullptr;
@@ -933,6 +944,24 @@ int run_sweep_t(sb_plan* pl, const sb_angle* angles, int n_angles, const sb_temp
                                     using S = Shape<N, float>;
                                     ProfScope prof(pl, K_FIT_ROWS);
                                     const dim3 grid(div_up(Py / 2, S::GP), nsub);
+                                    if (so.region) {
+                                        if (masked) {
+                                            if constexpr (N <= kMaxFftMasked) {
+                                                return launch(pl, "k_fit_rows_gmr", sb::k_fit_rows_gmr<N>, grid,
+                                                              dim3(S::threads),
+                                                              S::smem_fit_f + sb::fit_masked_extra_smem<N>(), g,
+                                                              gp.count, d_slots, (const sb::FitT*)pl->fit.p,
+                                                              (const sb::FitM*)pl->fitm.p, ch.cnt,
+                                                              (const float4*)pl->gbuf.p, (const float2*)twx, cross,
+                                                              *so.region);
+                                            }
+                                            return fail("internal: masked fit at FFT length " + std::to_string(N));
+                                        }
+                                        return launch(pl, "k_fit_rows_gr", sb::k_fit_rows_gr<N>, grid, dim3(S::threads),
+                                                      S::smem_fit_f, g, gp.count, d_slots, (const sb::FitT*)pl->fit.p,
+                                                      (const float4*)pl->gbuf.p, (const float2*)twx, cross,
+                                                      *so.region);
+                                    }
                                     if (masked) {
                                         // FFT lengths <= 4096 only: the park buffers need 2 N float2 per group
                                         if constexpr (N <= kMaxFftMasked) {
@@ -952,7 +981,7 @@ int run_sweep_t(sb_plan* pl, const sb_angle* angles, int n_angles, const sb_temp
                                                   (const float4*)pl->gbuf.p, bsnr, bamp, bidx, (const float2*)twx,
                                                   cross, sub_stride);
                                 }));
-                                if (g.poison)
+                                if (g.poison && !so.region)
                                     SB_OK(launch(pl, "k_poison_windows", sb::k_poison_windows,
                                                  dim3(div_up((long)g.out_ny * g.out_nx, 256)), dim3(256), 0, g,
                                                  gp.count, d_slots, (const sb::FitT*)pl->fit.p, bsnr));
@@ -975,12 +1004,12 @@ int run_sweep_t(sb_plan* pl, const sb_angle* angles, int n_angles, const sb_temp
                 }
             }
         }
-    if (nsub > 1) {
+    if (nsub > 1 && !so.region) {
         SB_OK(launch(pl, "k_best_fold", sb::k_best_fold, dim3(div_up(sub_stride, 256)), dim3(256), 0, sub_stride,
                      nsub - 1, sub_stride, (const float*)pl->d_bsnr + sub_stride, (const float*)pl->d_bamp + sub_stride,
                      (const int*)pl->d_bidx + sub_stride, pl->d_bsnr, pl->d_bamp, pl->d_bidx));
     }
-    if (masked) {
+    if (masked && !so.region) {
         SB_OK(launch(pl, "k_best_clear_nodata", sb::k_best_clear_nodata, dim3(div_up(bn, 256)), dim3(256), 0, pl->ny,
                      pl->nx, pl->row0, pl->slab_lo, (int)pl->brows(), pl->n_states, bn, (const double*)pl->d_dem,
                      pl->d_bsnr, pl->d_bamp, pl->d_bidx));
@@ -1074,7 +1103,7 @@ int sb_plan_destroy(sb_plan* pl) {
     for (auto e : pl->ev_pool) sb_rt_event_destroy(e);
     for (Buf* b : {&pl->cr, &pl->fct, &pl->trt, &pl->part, &pl->gbuf, &pl->sums, &pl->fit, &pl->tmpls, &pl->angles,
                    &pl->tables, &pl->raw, &pl->tbox, &pl->slots, &pl->cross, &pl->casa, &pl->aux, &pl->spec9, &pl->coef,
-                   &pl->fitm, &pl->fs_idx, &pl->fs_out})
+                   &pl->fitm, &pl->fs_idx, &pl->fs_out, &pl->region, &pl->rtab})
         release(*b);
 #ifndef SB_EMU
     if (pl->own_stream) cudaStreamDestroy(pl->stream);
@@ -1179,7 +1208,7 @@ long sb_plan_device_bytes(const sb_plan* pl) {
     b += (size_t)pl->bn() * pl->n_states * pl->best_copies * 12;
     for (const Buf* q : {&pl->cr, &pl->fct, &pl->trt, &pl->part, &pl->gbuf, &pl->sums, &pl->fit, &pl->tmpls, &pl->angles,
                          &pl->tables, &pl->raw, &pl->tbox, &pl->slots, &pl->cross, &pl->casa, &pl->aux, &pl->spec9, &pl->coef,
-                         &pl->fitm, &pl->fs_idx, &pl->fs_out})
+                         &pl->fitm, &pl->fs_idx, &pl->fs_out, &pl->region, &pl->rtab})
         b += q->cap;
     return (long)b;
 }
@@ -1483,6 +1512,94 @@ int sb_age_range(sb_plan* pl, int n_states, int row_lo, int row_hi, double snr_r
                  (const float*)pl->d_bsnr + off, (const float*)pl->d_bamp + off, (const int*)pl->d_bidx + off,
                  (const double*)d_age, (const double*)d_ang, n_idx, snr_ratio, dst));
     if (!out_is_device) return copy_out(pl, out6, dst, (size_t)n * 6, 0);
+    SB_TRY(sb_rt_sync(pl->stream));
+    return 0;
+}
+
+int sb_region_sweep(sb_plan* pl, const sb_angle* angles, int n_angles, const sb_template* tmpls, int n_tmpls,
+                    const int32_t* whole_search5, double snr_ratio, const int32_t* age_rank_host,
+                    const int32_t* angle_pos_host, int n_idx, int n_pos) {
+    if (!pl || !angles || !tmpls || !age_rank_host || !angle_pos_host || n_idx <= 0)
+        return fail("sb_region_sweep: bad arguments");
+    if (!(snr_ratio > 0.0 && snr_ratio <= 1.0)) return fail("sb_region_sweep: snr_ratio must be in (0, 1]");
+    if (n_pos < 1 || n_pos > 256) return fail("sb_region_sweep: n_pos must be in 1 .. 256");
+    if (pl->precision != 32 || !pl->fast) return fail("sb_region_sweep: fit region needs precision 32 and the option fast");
+    int n_ranks = 0;
+    for (int k = 0; k < n_idx; ++k) {
+        if (age_rank_host[k] < 0 || angle_pos_host[k] < 0 || angle_pos_host[k] >= n_pos)
+            return fail("sb_region_sweep: age rank or orientation position out of range at flat index " + std::to_string(k));
+        n_ranks = std::max(n_ranks, age_rank_host[k] + 1);
+    }
+    for (int k = 0; k < n_tmpls; ++k)
+        if (tmpls[k].idx < 0 || tmpls[k].idx >= n_idx)
+            return fail("sb_region_sweep: template flat index outside 0 .. n_idx - 1");
+    const int words = (n_pos + 31) / 32;
+    const long bn = pl->bn(), boff = (long)pl->slab_lo * pl->nx;
+    SB_OK(ensure(pl->region, (size_t)(3 + words) * bn * sizeof(int)));
+    SB_OK(ensure(pl->rtab, (size_t)2 * n_idx * sizeof(int32_t)));
+    int* planes = (int*)pl->region.p;
+    int* tab = (int*)pl->rtab.p;
+    SB_TRY(sb_rt_h2d(tab, age_rank_host, (size_t)n_idx * sizeof(int32_t), pl->stream));
+    SB_TRY(sb_rt_h2d(tab + n_idx, angle_pos_host, (size_t)n_idx * sizeof(int32_t), pl->stream));
+    // count 0, rank_lo 0x7f7f7f7f (above every rank), rank_hi -1, no orientation bits
+    SB_TRY(sb_rt_memset(planes, 0, (size_t)bn * sizeof(int), pl->stream));
+    SB_TRY(sb_rt_memset(planes + bn, 0x7f, (size_t)bn * sizeof(int), pl->stream));
+    SB_TRY(sb_rt_memset(planes + 2 * bn, 0xff, (size_t)bn * sizeof(int), pl->stream));
+    SB_TRY(sb_rt_memset(planes + 3 * bn, 0, (size_t)words * bn * sizeof(int), pl->stream));
+    sb::RegionOut rg;
+    rg.best = pl->d_bsnr - boff;
+    rg.count = planes - boff;
+    rg.rank_lo = planes + bn - boff;
+    rg.rank_hi = planes + 2 * bn - boff;
+    rg.bits = (unsigned*)(planes + 3 * bn) - boff;
+    rg.age_rank = tab;
+    rg.angle_pos = tab + n_idx;
+    rg.plane = bn;
+    rg.ratio = snr_ratio;
+    pl->region_npos = 0;
+    SweepOut so;
+    so.region = &rg;
+    SB_OK(run_sweep(pl, angles, n_angles, tmpls, n_tmpls, so, whole_search5));
+    SB_TRY(sb_rt_sync(pl->stream));
+    pl->region_words = words;
+    pl->region_npos = n_pos;
+    pl->region_nranks = n_ranks;
+    return 0;
+}
+
+int sb_region_finalize(sb_plan* pl, int row_lo, int row_hi, const double* age_of_host, const double* angle_of_host,
+                       int n_idx, const double* rank_age_host, int n_ranks, const double* pos_angle_host, int n_pos,
+                       int periodic, double* out9, int out_is_device) {
+    if (!pl || !age_of_host || !angle_of_host || !rank_age_host || !pos_angle_host || !out9 || n_idx <= 0)
+        return fail("sb_region_finalize: bad arguments");
+    if (pl->region_npos == 0) return fail("sb_region_finalize: no region sweep since the best state was last allocated");
+    if (n_pos != pl->region_npos) return fail("sb_region_finalize: n_pos differs from the region sweep's");
+    if (n_ranks < pl->region_nranks) return fail("sb_region_finalize: fewer ages than the region sweep's ranks");
+    if (row_lo < pl->slab_lo || row_hi > pl->slab_hi || row_lo >= row_hi) return fail("sb_region_finalize: rows outside the plan");
+    const long n = (long)(row_hi - row_lo) * pl->nx;
+    const long off = (long)(row_lo - pl->slab_lo) * pl->nx;
+    const long bn = pl->bn();
+    SB_OK(ensure(pl->tables, (size_t)(2 * n_idx + n_ranks + n_pos) * sizeof(double)));
+    double* d_age = (double*)pl->tables.p;
+    double* d_ang = d_age + n_idx;
+    double* d_rank_age = d_ang + n_idx;
+    double* d_pos_angle = d_rank_age + n_ranks;
+    SB_TRY(sb_rt_h2d(d_age, age_of_host, (size_t)n_idx * sizeof(double), pl->stream));
+    SB_TRY(sb_rt_h2d(d_ang, angle_of_host, (size_t)n_idx * sizeof(double), pl->stream));
+    SB_TRY(sb_rt_h2d(d_rank_age, rank_age_host, (size_t)n_ranks * sizeof(double), pl->stream));
+    SB_TRY(sb_rt_h2d(d_pos_angle, pos_angle_host, (size_t)n_pos * sizeof(double), pl->stream));
+    double* dst = out9;
+    if (!out_is_device) {
+        SB_OK(ensure(pl->raw, (size_t)n * 9 * sizeof(double)));
+        dst = (double*)pl->raw.p;
+    }
+    const int* planes = (const int*)pl->region.p + off;
+    SB_OK(launch(pl, "k_region_finalize", sb::k_region_finalize, dim3(div_up(n, 256)), dim3(256), 0, n, bn,
+                 pl->region_words, (const float*)pl->d_bsnr + off, (const float*)pl->d_bamp + off,
+                 (const int*)pl->d_bidx + off, planes, planes + bn, planes + 2 * bn, (const unsigned*)(planes + 3 * bn),
+                 (const double*)d_age, (const double*)d_ang, n_idx, (const double*)d_rank_age,
+                 (const double*)d_pos_angle, n_pos, periodic ? 1 : 0, dst));
+    if (!out_is_device) return copy_out(pl, out9, dst, (size_t)n * 9, 0);
     SB_TRY(sb_rt_sync(pl->stream));
     return 0;
 }

@@ -468,6 +468,35 @@ class Plan(object):
                                               angle_of.ctypes.data, len(age_of), out.ctypes.data, 0))
         return out
 
+    def region_sweep(self, angle_records, template_records, snr_ratio, tables):
+        """Pass 2 of a fit confidence region (``sb_region_sweep``, DESIGN.md section 14): best state 0
+        must hold the result of ``sweep`` over the same records.  Sweeps them again and records, per
+        pixel, the templates whose SNR is at least ``snr_ratio`` (in (0, 1]) times the pixel's best;
+        ``tables``: ``params.region_tables`` of the search.  The best state is not modified."""
+        arr_a, na = angle_records
+        arr_t, nt = template_records[0], template_records[1]
+        whole = template_records[2] if len(template_records) > 2 else None
+        rank = np.ascontiguousarray(tables.age_rank, dtype=np.int32)
+        pos = np.ascontiguousarray(tables.angle_pos, dtype=np.int32)
+        check(self.lib, self.lib.sb_region_sweep(self._h, arr_a, na, arr_t, nt, whole, float(snr_ratio),
+                                                 rank.ctypes.data, pos.ctypes.data, len(rank),
+                                                 len(tables.pos_angle)))
+
+    def region_finalize(self, age_of, angle_of, tables, rows=None):
+        """(9, rows, nx) float64 [amp, age, angle, snr, age_lo, age_hi, angle_lo, angle_hi, n_fits] after
+        ``region_sweep`` (``sb_region_finalize``): planes 0..3 are ``finalize``'s, 4..8 the region's
+        extent in age and orientation and its template count, 0 where the pixel has no fit.
+        ``rows=(lo, hi)``: a band of the plan's rows (default: all of them)."""
+        age_of, angle_of = _as_f64(age_of), _as_f64(angle_of)
+        rank_age, pos_angle = _as_f64(tables.rank_age), _as_f64(tables.pos_angle)
+        lo, hi = (self.row_lo, self.row_hi) if rows is None else (int(rows[0]), int(rows[1]))
+        out = np.empty((9, max(hi - lo, 0), self.nx), dtype=np.float64)
+        check(self.lib, self.lib.sb_region_finalize(self._h, lo, hi, age_of.ctypes.data, angle_of.ctypes.data,
+                                                    len(age_of), rank_age.ctypes.data, len(rank_age),
+                                                    pos_angle.ctypes.data, len(pos_angle), int(tables.periodic),
+                                                    out.ctypes.data, 0))
+        return out
+
     def finalize_device(self, age_of, angle_of, out_ptr, state=0, rows=None):
         """``finalize`` into device memory (4 * rows * nx float64 at ``out_ptr``)."""
         age_of, angle_of = _as_f64(age_of), _as_f64(angle_of)

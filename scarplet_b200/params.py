@@ -10,6 +10,8 @@ the CUDA library as plain numbers, so that masks come out bit-exact:
 * a conservative support box of the template (the device evaluates the exact window
   ``(abs(xr) < c) & (abs(yr) < d)`` inside it)   WindowedTemplate.py:61-64
 """
+import collections
+
 import numpy as np
 from scipy.special import erfinv
 
@@ -40,6 +42,31 @@ def search_angles(ang_min, ang_max):
     ang_stepsize = 1
     num_angles = int((180 / np.pi) * (ang_max - ang_min) / ang_stepsize + 1)
     return np.linspace(ang_min, ang_max, num_angles)
+
+
+RegionTables = collections.namedtuple("RegionTables", ["age_rank", "angle_pos", "rank_age", "pos_angle", "periodic"])
+
+
+def region_tables(ages, angles, order="age_major"):
+    """Per flat index of a sweep over ``angles`` x ``ages`` (``order`` as ``Plan.build_sweep``): the
+    rank of its age among the sorted ages and its orientation position, with the inverse tables
+    ``rank_age`` and ``pos_angle``.  When the angles span exactly pi (within 1e-9, e.g. the default
+    -pi/2 .. pi/2) the search is periodic: the last angle is the first one's line and shares its
+    position 0, and positions run 0 .. len(angles) - 2."""
+    ages = np.atleast_1d(np.asarray(ages, dtype=np.float64))
+    angles = np.atleast_1d(np.asarray(angles, dtype=np.float64))
+    A, G = len(angles), len(ages)
+    periodic = A > 1 and abs((angles[-1] - angles[0]) - np.pi) <= 1e-9
+    n_pos = A - 1 if periodic else A
+    rank = np.argsort(np.argsort(ages, kind="stable"), kind="stable")
+    pos = np.arange(A) % n_pos
+    ai, gi = np.meshgrid(np.arange(A), np.arange(G), indexing="ij")
+    idx = gi * A + ai if order == "age_major" else ai * G + gi
+    age_rank = np.empty(A * G, dtype=np.int32)
+    angle_pos = np.empty(A * G, dtype=np.int32)
+    age_rank[idx] = rank[gi]
+    angle_pos[idx] = pos[ai]
+    return RegionTables(age_rank, angle_pos, np.sort(ages), angles[:n_pos].copy(), bool(periodic))
 
 
 def default_ages():
