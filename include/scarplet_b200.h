@@ -264,6 +264,20 @@ int sb_best_state_ex(sb_plan* plan, int state, float** snr_dev, float** amp_dev,
 int sb_best_merge(sb_plan* plan, int state, int row_lo, int row_hi, int n_cands, const float* snr_c,
                   const float* amp_c, const int32_t* idx_c);
 
+/* Raw region planes for a cross-GPU merge of a fit confidence region (DESIGN §15): *planes_dev points
+ * at plane 0 of the plan's region planes, plane p of pixel i (counted over the plan's rows) at
+ * [p * rows * nx + i]; *n_planes = 3 + ceil(n_pos / 32) (count, rank_lo, rank_hi, orientation words).
+ * Fails without a region sweep since the best state was last allocated. */
+int sb_region_planes(sb_plan* plan, int32_t** planes_dev, int* n_planes);
+
+/* Replace the region planes on raster rows row_lo .. row_hi - 1 by the fold of n_cands candidates
+ * (device int32 laid out [plane][candidate][row][nx], e.g. what one all-to-all per plane of the
+ * ranks' region planes delivers): count summed, rank_lo minimum, rank_hi maximum, orientation words
+ * OR-ed.  Replaced, not folded in: the candidates are expected to include this plan's own planes.
+ * Rows outside the band are untouched.  Fails for null pointers, n_cands < 1, rows outside the plan
+ * and without a region sweep since the best state was last allocated. */
+int sb_region_merge(sb_plan* plan, int row_lo, int row_hi, int n_cands, const int32_t* cands_dev);
+
 /* Cross-GPU merge of best states (the parent-side reduce over Pool results,
  * core.py:185, when the search is sharded over ranks).  All buffers are device memory
  * of ny*nx elements owned by the caller (e.g. torch tensors handed to NCCL):

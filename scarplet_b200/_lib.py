@@ -69,6 +69,8 @@ def _declare(lib):
                                        c_int, c_void_p, c_int]
     lib.sb_best_state_ex.argtypes = [P, c_int, POINTER(c_void_p), POINTER(c_void_p), POINTER(c_void_p)]
     lib.sb_best_merge.argtypes = [P, c_int, c_int, c_int, c_int, c_void_p, c_void_p, c_void_p]
+    lib.sb_region_planes.argtypes = [P, POINTER(c_void_p), POINTER(c_int)]
+    lib.sb_region_merge.argtypes = [P, c_int, c_int, c_int, c_void_p]
     lib.sb_curvature_noise_moments.argtypes = [P, c_double, c_double, dp]
     lib.sb_fill_nodata.argtypes = [P, c_void_p, c_double, POINTER(c_long)]
     lib.sb_plan_last_geometry.argtypes = [P, POINTER(c_int)]
@@ -107,7 +109,8 @@ def _declare(lib):
                  "sb_compare_host", "sb_debug_fft", "sb_sync", "sb_plan_set_slab", "sb_plan_dem_rows",
                  "sb_plan_curv_stats", "sb_plan_set_curv_stats", "sb_finalize_ex", "sb_best_state_ex",
                  "sb_best_merge", "sb_curvature_noise_moments", "sb_fill_nodata", "sb_plan_set_nodata",
-                 "sb_fit_surface", "sb_age_range", "sb_region_sweep", "sb_region_finalize"):
+                 "sb_fit_surface", "sb_age_range", "sb_region_sweep", "sb_region_finalize", "sb_region_planes",
+                 "sb_region_merge"):
         getattr(lib, name).restype = c_int
     return lib
 
@@ -122,7 +125,7 @@ EXPORTED = ("sb_last_error", "sb_build_info", "sb_plan_create", "sb_plan_destroy
             "sb_plan_set_curv_stats", "sb_plan_stream", "sb_plan_device_bytes", "sb_plan_last_fft_area",
             "sb_finalize_ex", "sb_best_state_ex", "sb_best_merge", "sb_curvature_noise_moments",
             "sb_fill_nodata", "sb_debug_fft_bench", "sb_sweep_ex", "sb_plan_set_nodata", "sb_fit_surface",
-            "sb_age_range", "sb_region_sweep", "sb_region_finalize")
+            "sb_age_range", "sb_region_sweep", "sb_region_finalize", "sb_region_planes", "sb_region_merge")
 
 
 def library_path():

@@ -287,7 +287,7 @@ def fit_surface(data, Template, scale, pixels, ages=None, ang_min=-np.pi / 2, an
     return FitSurface(amp, snr, ages, angles)
 
 
-def _age_search(name, Template, ages, kwargs, snr_ratio=None, max_ages=64):
+def _age_search(name, Template, ages, kwargs, snr_ratio=None, max_ages=64, angles=None):
     """(device spec, float64 ages) of an age-resolved search; ``ValueError`` for what it does not take."""
     if kwargs:
         raise ValueError("%s takes no template keyword arguments (%s): the per-age states need a built-in "
@@ -295,6 +295,15 @@ def _age_search(name, Template, ages, kwargs, snr_ratio=None, max_ages=64):
     spec = device_spec(Template)
     if spec is None:
         raise ValueError("%s needs a built-in template class; %r has no on-device generator" % (name, Template))
+    return spec, search_args(name, ages, snr_ratio, max_ages, angles)
+
+
+def search_args(name, ages, snr_ratio=None, max_ages=64, angles=None):
+    """Float64 ages of an age-resolved search or a fit region (``None``: the 35 default ages);
+    ``ValueError`` for what ``name`` does not take: no or more than ``max_ages`` ages (``None``: no
+    limit), duplicate ages, ``snr_ratio`` outside (0, 1] and, when ``angles`` is given (a fit region),
+    more than 256 orientations.  Shared by ``core`` and the multi-GPU drivers of ``distributed``,
+    which check before any device work or collective."""
     ages = P.default_ages() if ages is None else np.atleast_1d(np.asarray(ages, dtype=np.float64))
     if max_ages is None:
         if ages.ndim != 1 or len(ages) < 1:
@@ -305,7 +314,9 @@ def _age_search(name, Template, ages, kwargs, snr_ratio=None, max_ages=64):
         raise ValueError("%s: duplicate ages" % name)
     if snr_ratio is not None and not (np.isfinite(snr_ratio) and 0.0 < snr_ratio <= 1.0):
         raise ValueError("snr_ratio must be in (0, 1], not %r" % (snr_ratio,))
-    return spec, ages
+    if angles is not None and len(angles) > 256:
+        raise ValueError("%s takes at most 256 orientations, not %d" % (name, len(angles)))
+    return ages
 
 
 def _age_sweep(plan, spec, scale, ages, ang_min, ang_max):
@@ -373,10 +384,8 @@ def fit_region(data, Template, scale, snr_ratio, ages=None, ang_min=-np.pi / 2, 
     ceil(orientations / 32)) B per pixel of device memory, whatever the number of ages (36 B for
     181 orientations).  Built-in template classes only, at most 256 orientations, distinct ages;
     ``nodata`` / ``min_coverage``: see ``calculate_best_fit_parameters``."""
-    spec, ages = _age_search("fit_region", Template, ages, kwargs, snr_ratio, max_ages=None)
     angles = P.search_angles(ang_min, ang_max)
-    if len(angles) > 256:
-        raise ValueError("fit_region takes at most 256 orientations, not %d" % len(angles))
+    spec, ages = _age_search("fit_region", Template, ages, kwargs, snr_ratio, max_ages=None, angles=angles)
     tables = P.region_tables(ages, angles)
     with _plan_for(data, nodata=nodata, min_coverage=min_coverage) as plan:
         a_rec, t_rec, age_of, angle_of = plan.build_sweep(spec, scale, ages, angles, "age_major")

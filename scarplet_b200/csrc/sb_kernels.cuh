@@ -987,6 +987,28 @@ SB_GLOBAL k_best_merge(long n, int n_cands, const float* SB_RESTRICT snr_c, cons
     snr[i] = bs; amp[i] = ba; idx[i] = bi;
 }
 
+// Fold `n_cands` candidate region planes (e.g. one per rank of an orientation-sharded fit region)
+// for the same `n` pixels into the plan's: plane 0 (count) is summed, plane 1 (rank_lo) the minimum,
+// plane 2 (rank_hi) the maximum, planes 3 .. n_planes - 1 (orientation words) OR-ed.  Candidate c of
+// plane p, pixel i is at [(p * n_cands + c) * n + i]; plane p of the output at [p * plane + i].  The
+// output is replaced, not folded into: the candidates include this rank's own planes.  The cleared
+// planes of sb_region_sweep (0, 0x7f7f7f7f, -1, no bits) are identities of the four folds.  One
+// thread per (plane, pixel).
+SB_GLOBAL k_region_merge(long n, int n_planes, int n_cands, long plane, const int* SB_RESTRICT cands,
+                         int* SB_RESTRICT planes) {
+    const long t = (long)sb_bx() * 256 + sb_tid();
+    if (t >= n * n_planes) return;
+    const int p = (int)(t / n);
+    const long i = t - (long)p * n;
+    const int* c = cands + (long)p * n_cands * n + i;
+    int v = c[0];
+    for (int k = 1; k < n_cands; ++k) {
+        const int w = c[(long)k * n];
+        v = p == 0 ? v + w : p == 1 ? (w < v ? w : v) : p == 2 ? (w > v ? w : v) : (v | w);
+    }
+    planes[(long)p * plane + i] = v;
+}
+
 // Fold `n_extra` further copies of a best state (copy c of pixel i at [c * stride + i]) into the
 // main one in place, with k_best_merge's rule.
 SB_GLOBAL k_best_fold(long n, int n_extra, long stride, const float* SB_RESTRICT snr_x, const float* SB_RESTRICT amp_x,

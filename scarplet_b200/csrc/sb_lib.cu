@@ -1635,6 +1635,25 @@ int sb_best_merge(sb_plan* pl, int state, int row_lo, int row_hi, int n_cands, c
                   (const int*)idx_c, pl->d_bsnr + off, pl->d_bamp + off, pl->d_bidx + off);
 }
 
+int sb_region_planes(sb_plan* pl, int32_t** planes_dev, int* n_planes) {
+    if (!pl || !planes_dev || !n_planes) return fail("sb_region_planes: bad arguments");
+    if (pl->region_npos == 0) return fail("sb_region_planes: no region sweep since the best state was last allocated");
+    *planes_dev = (int32_t*)pl->region.p;
+    *n_planes = 3 + pl->region_words;
+    return 0;
+}
+
+int sb_region_merge(sb_plan* pl, int row_lo, int row_hi, int n_cands, const int32_t* cands_dev) {
+    if (!pl || !cands_dev || n_cands < 1) return fail("sb_region_merge: bad arguments");
+    if (pl->region_npos == 0) return fail("sb_region_merge: no region sweep since the best state was last allocated");
+    if (row_lo < pl->slab_lo || row_hi > pl->slab_hi || row_lo >= row_hi) return fail("sb_region_merge: rows outside the plan");
+    const long n = (long)(row_hi - row_lo) * pl->nx;
+    const long off = (long)(row_lo - pl->slab_lo) * pl->nx;
+    const int n_planes = 3 + pl->region_words;
+    return launch(pl, "k_region_merge", sb::k_region_merge, dim3(div_up(n * n_planes, 256)), dim3(256), 0, n, n_planes,
+                  n_cands, pl->bn(), (const int*)cands_dev, (int*)pl->region.p + off);
+}
+
 int sb_best_pack(sb_plan* pl, unsigned long long* keys_dev) {
     if (!pl || !keys_dev) return fail("sb_best_pack: null");
     const long n = pl->bn();

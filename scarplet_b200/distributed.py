@@ -136,6 +136,99 @@ def merge_best_bands(plan, device, group=None, state=0):
     return lo, hi
 
 
+def merge_region_bands(plan, device, group=None):
+    """Banded merge of the region planes after ``region_sweep`` over this rank's share: rank r
+    receives every rank's planes for row band r (one all-to-all per plane) and replaces its own
+    there by their fold (``Plan.region_merge``: counts summed, age ranks min / max, orientation
+    words OR-ed -- NCCL has no OR reduction, so no all-reduce can do this).  Afterwards this rank's
+    region planes are the merged result on rows ``shard_bounds(ny, world, rank)``; returns that band
+    ``(row_lo, row_hi)``.  Bands, fences and receive buffer as ``merge_best_bands``; the buffer holds
+    4 * (3 + words) B per pixel of the plan's rows."""
+    import torch
+    import torch.distributed as dist
+    world, rank = _world(group)
+    ny, nx = plan.row_hi - plan.row_lo, plan.nx
+    bands = [shard_bounds(ny, world, r) for r in range(world)]
+    lo, hi = bands[rank]
+    lo, hi = lo + plan.row_lo, hi + plan.row_lo
+    if world == 1:
+        return lo, hi
+    fence = _Fence(plan, device)
+    ptr, n_planes = plan.region_planes()
+    n = ny * nx
+    send = [nx * (b - a) for a, b in bands]
+    mine = nx * (hi - lo)
+    recv = [mine] * world
+    src = _as_tensor(ptr, n_planes * n, "i4", device).view(n_planes, n)
+    dst = torch.empty((n_planes, world * mine), dtype=torch.int32, device=device)     # [plane][cand][row][nx]
+    fence.plan_done()                        # the region pass's last writes to the planes
+    for p in range(n_planes):
+        dist.all_to_all_single(dst[p], src[p], output_split_sizes=recv, input_split_sizes=send, group=group)
+    fence.torch_done()
+    plan.region_merge((lo, hi), world, dst.data_ptr())
+    fence.plan_done()                        # the candidate buffer is released on return
+    return lo, hi
+
+
+def _region_args(plan, name, ages, angles, snr_ratio):
+    """Checked float64 ages and the region tables of a fit region; one best state."""
+    from . import params as P
+    from .core import search_args
+    ages = search_args(name, ages, snr_ratio, max_ages=None, angles=angles)
+    if plan.states != 1:
+        plan.set_states(1)
+    return ages, P.region_tables(ages, angles)
+
+
+def _age_range_args(plan, name, ages, snr_ratio):
+    """Checked float64 ages of an age range; one best state per age."""
+    from .core import search_args
+    ages = search_args(name, ages, snr_ratio)
+    if plan.states != len(ages):
+        plan.set_states(len(ages))
+    return ages
+
+
+def sharded_fit_region(plan, spec, scale, ages, angles, snr_ratio, device=None, group=None):
+    """``core.fit_region`` over ranks sharing the orientation x age templates (DESIGN.md section 15),
+    on ``plan`` over the whole raster (DEM already set, e.g. with ``set_dem_sharded``): this rank
+    sweeps its share, the best states are merged replicated (every pixel's threshold needs the
+    merged best), the region pass runs over the same share and the region planes are merged by row
+    band.  Returns ``(row_lo, row_hi, stack)``, ``stack`` the (9, row_hi - row_lo, nx) rows of
+    ``core.fit_region``'s result, bit for bit.  Raises ``core.fit_region``'s ``ValueError`` before any
+    device work or collective."""
+    ages, tables = _region_args(plan, "sharded_fit_region", ages, angles, snr_ratio)
+    world, rank = _world(group)
+    share = (rank, world) if world > 1 else None
+    a_rec, t_rec, age_of, angle_of = plan.build_sweep(spec, scale, ages, angles, "age_major", template_share=share)
+    plan.reset()
+    plan.sweep(a_rec, t_rec)
+    if world > 1:
+        merge_best_state(plan, device, group)
+    plan.region_sweep(a_rec, t_rec, snr_ratio, tables)
+    band = merge_region_bands(plan, device, group)
+    return band + (plan.region_finalize(age_of, angle_of, tables, rows=band),)
+
+
+def sharded_age_range(plan, spec, scale, ages, angles, snr_ratio, device=None, group=None):
+    """``core.age_range`` over ranks sharing the orientation x age templates (DESIGN.md section 15):
+    this rank sweeps its share with one best state per age, every state is merged by row band
+    (``merge_best_bands``) and this rank reduces its band.  Returns ``(row_lo, row_hi, stack)``,
+    ``stack`` the (6, row_hi - row_lo, nx) rows of ``core.age_range``'s result, bit for bit.  Raises
+    ``core.age_range``'s ``ValueError`` before any device work or collective."""
+    ages = _age_range_args(plan, "sharded_age_range", ages, snr_ratio)
+    world, rank = _world(group)
+    share = (rank, world) if world > 1 else None
+    a_rec, t_rec, age_of, angle_of = plan.build_sweep(spec, scale, ages, angles, "age_major", template_share=share,
+                                                     state_per_age=True)
+    plan.reset()
+    plan.sweep(a_rec, t_rec)
+    band = (plan.row_lo, plan.row_hi)
+    for s in range(len(ages)):
+        band = merge_best_bands(plan, device, group, state=s)
+    return band + (plan.age_range(age_of, angle_of, snr_ratio, rows=band),)
+
+
 def set_dem_sharded(plan, z, device, group=None):
     """``plan.set_dem(z)`` for an orientation-sharded search, where every rank needs the whole
     raster: rank r copies only rows ``shard_bounds(ny, world, r)`` host -> device and the ranks
@@ -252,3 +345,26 @@ def spatial_search(plan, spec, scale, ages, angles, order="age_major", finalize=
     if not finalize:
         return plan.row_lo, plan.row_hi, None
     return plan.row_lo, plan.row_hi, plan.finalize(age_of, angle_of)
+
+
+def spatial_fit_region(plan, spec, scale, ages, angles, snr_ratio):
+    """``core.fit_region`` on this rank's band (DEM set, statistics shared): both passes on the slab
+    plan.  Returns ``(row_lo, row_hi, stack)`` with ``stack`` of shape (9, row_hi - row_lo, nx); no
+    data-path collective."""
+    ages, tables = _region_args(plan, "spatial_fit_region", ages, angles, snr_ratio)
+    a_rec, t_rec, age_of, angle_of = plan.build_sweep(spec, scale, ages, angles)
+    plan.reset()
+    plan.sweep(a_rec, t_rec)
+    plan.region_sweep(a_rec, t_rec, snr_ratio, tables)
+    return plan.row_lo, plan.row_hi, plan.region_finalize(age_of, angle_of, tables)
+
+
+def spatial_age_range(plan, spec, scale, ages, angles, snr_ratio):
+    """``core.age_range`` on this rank's band (DEM set, statistics shared; create the plan with
+    ``spatial_plan(..., states=len(ages))`` to avoid a reallocation).  Returns ``(row_lo, row_hi,
+    stack)`` with ``stack`` of shape (6, row_hi - row_lo, nx); no data-path collective."""
+    ages = _age_range_args(plan, "spatial_age_range", ages, snr_ratio)
+    a_rec, t_rec, age_of, angle_of = plan.build_sweep(spec, scale, ages, angles, "age_major", state_per_age=True)
+    plan.reset()
+    plan.sweep(a_rec, t_rec)
+    return plan.row_lo, plan.row_hi, plan.age_range(age_of, angle_of, snr_ratio)

@@ -497,6 +497,21 @@ class Plan(object):
                                                     out.ctypes.data, 0))
         return out
 
+    def region_planes(self):
+        """``(ptr, n_planes)`` of the region planes after ``region_sweep`` (``sb_region_planes``): int32
+        device memory, plane ``p`` of pixel ``i`` of the plan's rows at ``[p * rows * nx + i]``; planes
+        count, rank_lo, rank_hi and ``n_planes - 3`` orientation words."""
+        p, n = c_void_p(), c_int()
+        check(self.lib, self.lib.sb_region_planes(self._h, byref(p), byref(n)))
+        return p.value, n.value
+
+    def region_merge(self, rows, n_cands, cands_ptr):
+        """Replace the region planes on raster rows ``rows`` by the fold of ``n_cands`` candidates
+        (int32 device buffer laid out [plane][candidate][row][nx], ``sb_region_merge``): counts
+        summed, rank_lo minimum, rank_hi maximum, orientation words OR-ed."""
+        check(self.lib, self.lib.sb_region_merge(self._h, int(rows[0]), int(rows[1]), int(n_cands),
+                                                 c_void_p(int(cands_ptr))))
+
     def finalize_device(self, age_of, angle_of, out_ptr, state=0, rows=None):
         """``finalize`` into device memory (4 * rows * nx float64 at ``out_ptr``)."""
         age_of, angle_of = _as_f64(age_of), _as_f64(angle_of)
