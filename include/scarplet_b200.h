@@ -253,6 +253,22 @@ int sb_region_finalize(sb_plan* plan, int row_lo, int row_hi, const double* age_
                        const double* angle_of_host, int n_idx, const double* rank_age_host, int n_ranks,
                        const double* pos_angle_host, int n_pos, int periodic, double* out9, int out_is_device);
 
+/* Secondary fit (DESIGN §16): best state 0 must hold the result of a sweep (sb_sweep / sb_sweep_ex)
+ * over the same records, on a plan with at least 2 best states.  Resets best state 1 and sweeps the
+ * records again into it, folding at each pixel only the records whose orientation position
+ * angle_pos_host[idx] (in 0 .. n_pos - 1) is at least min_sep_pos from the position of state 0's
+ * winner there: distance |p - q|, or min(|p - q|, n_pos - |p - q|) when periodic.  A pixel whose state
+ * 0 SNR is 0 or NaN admits nothing.  Otherwise the fold is the search's (masks, min_coverage, highest
+ * SNR then lowest flat index, NaN windows of a NaN DEM, nodata cleared), so state 1 does not depend on
+ * batches, sub-streams or launch order; sb_finalize_ex(state 1) decodes it.  State 0 is not modified.
+ * Device memory: best state 1 (12 B per pixel) and a 2 B per pixel position plane.
+ * Fails for a plan with fewer than 2 states, precision 64 or fast = 0, n_pos outside 1 .. 256,
+ * min_sep_pos outside 1 .. (periodic ? n_pos / 2 : n_pos - 1), positions out of range, a record whose
+ * idx is outside 0 .. n_idx - 1 or whose state is not 0. */
+int sb_secondary_sweep(sb_plan* plan, const sb_angle* angles, int n_angles, const sb_template* tmpls, int n_tmpls,
+                       const int32_t* whole_search5, const int32_t* angle_pos_host, int n_idx, int n_pos,
+                       int periodic, int min_sep_pos);
+
 /* Raw best state for a cross-GPU merge: device pointers into the plan, one value per pixel of
  * the plan's rows. */
 int sb_best_state(sb_plan* plan, float** snr_dev, float** amp_dev, int32_t** idx_dev);

@@ -8,7 +8,7 @@ Drop-in for the reference's ``import scarplet as sl`` on that path::
 """
 from .core import (age_range, calculate_best_fit_parameters,  # noqa: F401
                    calculate_best_fit_parameters_serial, compare, fit_region, fit_surface, match, match_ages,
-                   match_scales, match_template, release)
+                   match_scales, match_template, release, secondary_fit)
 from .dem import DEMGrid  # noqa: F401
 from .engine import configure  # noqa: F401
 from .geotiff import write_results as save_results  # noqa: F401

@@ -395,6 +395,43 @@ def fit_region(data, Template, scale, snr_ratio, ages=None, ang_min=-np.pi / 2, 
         return plan.region_finalize(age_of, angle_of, tables)
 
 
+def secondary_fit(data, Template, scale, min_separation, ages=None, ang_min=-np.pi / 2, ang_max=np.pi / 2,
+                  nodata="propagate", min_coverage=1.0, **kwargs):
+    """The best fit at every pixel among the templates at least ``min_separation`` (radians) in
+    orientation from the pixel's best -- what else fits where a scarp crosses a channel or two fault
+    sets intersect, and whether a detection fits any strike.  Returns (8, ny, nx) float64
+    [amp, age, angle, snr, amp2, age2, angle2, snr2]:
+
+    * planes 0..3 are exactly ``match(data, Template, scale=scale, ages=ages, ...)``;
+    * planes 4..7 are the template with the highest float32 SNR (ties: the lowest flat index, the
+      search's rule) among those the masks leave a candidate at the pixel, with SNR > 0 and an
+      orientation position at least ``params.separation_positions(min_separation, angles)`` from the
+      best's.  A search spanning pi (the default) is periodic: -pi/2 and pi/2 are one position, and
+      the distance wraps across them.  They are 0 where nothing qualifies or the pixel has no fit,
+      and ``[NaN, 0, 0, NaN]`` where plane 3 is NaN.
+
+    Two device sweeps on one plan (DESIGN.md section 16): ``match``'s into best state 0, then the
+    same templates into best state 1 with the separation test in the fit kernel.  Device memory
+    beyond ``match``'s: 14 B per pixel (best state 1 and a 2-byte position plane; 235 MB at 4096^2).
+    Built-in template classes only, at least 2 and at most 256 orientations, distinct ages (any
+    number); ``nodata`` / ``min_coverage``: see ``calculate_best_fit_parameters``."""
+    angles = P.search_angles(ang_min, ang_max)
+    spec, ages = _age_search("secondary_fit", Template, ages, kwargs, max_ages=None, angles=angles)
+    m = P.separation_positions(min_separation, angles)
+    tables = P.region_tables(ages, angles)
+    z, _, _ = _grid_fields(data)
+    ny, nx = np.shape(z)
+    with _plan_for(data, states=2, nodata=nodata, min_coverage=min_coverage) as plan:
+        a_rec, t_rec, age_of, angle_of = plan.build_sweep(spec, scale, ages, angles, "age_major")
+        plan.reset()
+        plan.sweep(a_rec, t_rec)
+        plan.secondary_sweep(a_rec, t_rec, tables, m)
+        out = np.empty((8, ny, nx), dtype=np.float64)
+        plan.finalize(age_of, angle_of, state=0, out=out[:4])
+        plan.finalize(age_of, angle_of, state=1, out=out[4:])
+        return out
+
+
 def compare(results, ny, nx):
     """Per-pixel best-SNR select over an iterable of ``(amp, age, angle, snr)``
     (core.py:198-243), with the reference's exact semantics (strict compares, an

@@ -468,6 +468,39 @@ SB_DEVICE float region_threshold(float best, double ratio) {
 }
 
 // ---------------------------------------------------------------------------
+// Secondary fit (DESIGN.md 16): a second sweep of the same templates folds into best state 1 only the
+// templates whose orientation position is at least min_sep from the position of the pixel's winner
+// in best state 0 (the `pos` plane, k_secondary_pos).  An inadmissible candidate is skipped before it
+// touches the running best; everything else is the search's fold, so state 1 is the max-fold over
+// the admissible templates whatever the batches, sub-streams or launch order.
+// ---------------------------------------------------------------------------
+constexpr unsigned short kNoPos = 0xffff;          // `pos` of a pixel without a fit: nothing qualifies
+
+struct SecondOut {
+    const unsigned short* pos;    // winner's orientation position per pixel, addressed by raster row
+    const int* angle_pos;         // per flat index: orientation position
+    int n_pos;
+    int min_sep;                  // in positions, >= 1
+    int periodic;                 // positions 0 .. n_pos - 1 close into a circle
+};
+
+template <bool SECOND> struct SecondSlot {};
+template <> struct SecondSlot<true> {
+    SecondOut sec;
+    int tpos;                     // orientation position of the current template
+};
+
+// the `pos` plane of a secondary fit from best state 0: the winner's orientation position where
+// decode_best sees a hit (SNR > 0, index in range), kNoPos elsewhere (no fit, NaN)
+SB_GLOBAL k_secondary_pos(long n, const float* SB_RESTRICT snr, const int* SB_RESTRICT idx,
+                          const int* SB_RESTRICT angle_pos, int n_idx, unsigned short* SB_RESTRICT pos) {
+    const long i = (long)sb_bx() * 256 + sb_tid();
+    if (i >= n) return;
+    const int k = idx[i];
+    pos[i] = (snr[i] > 0.f && k >= 0 && k < n_idx) ? (unsigned short)angle_pos[k] : kNoPos;
+}
+
+// ---------------------------------------------------------------------------
 // k_fit_rows_g<Px>: grid (Py / 2 / GP).  The two transforms
 // a thread group pipelines are the two raster rows that share every 32-byte sector of the
 // interleaved planes (gbuf_index), of ONE template: a thread fetches whole sectors with
@@ -480,8 +513,9 @@ SB_DEVICE float region_threshold(float best, double ratio) {
 // outputs in `park`, every thread in the slots only it reads back; then the template's own.
 // REGION (k_fit_rows_gr / _gmr): bsA / bsB hold each pixel's region threshold (region_threshold) and
 // never change; a candidate is confirmed in float64 and recorded in the region planes (region_hit).
-template <int N, bool MASKED = false, bool REGION = false>
-struct FitPairCtx : RegionSlot<REGION> {
+// SECOND (k_fit_rows_gs / _gms): a candidate the separation rules out (second_ok) is skipped.
+template <int N, bool MASKED = false, bool REGION = false, bool SECOND = false>
+struct FitPairCtx : RegionSlot<REGION>, SecondSlot<SECOND> {
     static constexpr int K = sbfft::num_stages(N);
     static constexpr int T = N / E;
     static constexpr int LOG2T = ilog2(T);
@@ -548,6 +582,16 @@ struct FitPairCtx : RegionSlot<REGION> {
         sb_atomic_or(r.bits + (long)(p >> 5) * r.plane + pix, 1u << (p & 31));
     }
 
+    // SECOND: the current template is at least min_sep positions from the winner at pixel `pix`
+    SB_DEVICE bool second_ok(long pix) const {
+        const SecondOut& s = this->sec;
+        const int ps = s.pos[pix];
+        if (ps == kNoPos) return false;
+        int d = abs(this->tpos - ps);
+        if (s.periodic) d = min(d, s.n_pos - d);
+        return d >= s.min_sep;
+    }
+
     template <int F> SB_DEVICE void epilogue(const float2 (&v)[E], float (&bs)[E]) {
         const int gi = F == 0 ? giA : giB;
         const FitT k = s_fit[slot];
@@ -568,6 +612,9 @@ struct FitPairCtx : RegionSlot<REGION> {
                 if constexpr (REGION) {
                     region_hit((long)gi * nx + ox + jo, snr, k.idx);
                     continue;
+                }
+                if constexpr (SECOND) {
+                    if (!second_ok((long)gi * nx + ox + jo)) continue;
                 }
                 if (snr > bs[q] || k.idx < pi[jo]) {
                     bs[q] = snr;
@@ -626,6 +673,9 @@ struct FitPairCtx : RegionSlot<REGION> {
                     if constexpr (REGION) {
                         region_hit((long)gi * nx + ox + jo, snr, k.idx);
                         continue;
+                    }
+                    if constexpr (SECOND) {
+                        if (!second_ok((long)gi * nx + ox + jo)) continue;
                     }
                     if (snr > bs[q] || k.idx < pi[jo]) {
                         bs[q] = snr;
@@ -688,12 +738,12 @@ SB_CONSTEXPR size_t fit_masked_extra_smem() {
     return kFitMaxBatch * sizeof(FitM) + (size_t)((N / E > 256 ? N / E : 256) / (N / E)) * 2 * N * sizeof(float2);
 }
 
-template <int N, bool MASKED, bool REGION = false>
+template <int N, bool MASKED, bool REGION = false, bool SECOND = false>
 SB_DEVICE void fit_rows_g_body(const Geom& g, int count, const int* SB_RESTRICT slots, const FitT* SB_RESTRICT fit,
                                const FitM* SB_RESTRICT fitm, int comp_off, const float4* SB_RESTRICT gbuf,
                                float* SB_RESTRICT best_snr, float* SB_RESTRICT best_amp, int* best_idx,
                                const float2* SB_RESTRICT tw, const int4* SB_RESTRICT cross, long sub_stride,
-                               const RegionOut& rg = RegionOut()) {
+                               const RegionOut& rg = RegionOut(), const SecondOut& sec = SecondOut()) {
     // grid.y > 1 (small rasters, whose row pairs alone do not fill the GPU): the templates of the
     // launch are dealt round-robin to grid.y sub-streams; sub-stream j folds into copy j of the
     // best state (best_* + j * sub_stride; copy 0 is the state itself) and k_best_fold merges the
@@ -705,11 +755,12 @@ SB_DEVICE void fit_rows_g_body(const Geom& g, int count, const int* SB_RESTRICT 
     // with xr > 0 (.x .. .y) and xr < 0 (.z .. .w), k_err_cross.
     // REGION: best_* are unused; the thresholds come from rg.best (state 0 for every sub-stream)
     // and nothing writes a best state.
+    // SECOND: best_* are state 1's planes; `sec` rules out the templates too close to the winner.
     constexpr int T = N / E;
     constexpr int THREADS = T > 256 ? T : 256;
     constexpr int GP = THREADS / T;
     constexpr int PL = sbfft::padded_len(N);
-    typedef FitPairCtx<N, MASKED, REGION> Ctx;
+    typedef FitPairCtx<N, MASKED, REGION, SECOND> Ctx;
     const int grp = sb_tid() / T, t = sb_tid() % T;
     float2* sm = (float2*)sb_shared();
     FitT* s_fit = (FitT*)(sm + (long)GP * 2 * PL);
@@ -776,6 +827,7 @@ SB_DEVICE void fit_rows_g_body(const Geom& g, int count, const int* SB_RESTRICT 
     c.s_fm = s_fm;
     c.park = park;
     c.comp = false;
+    if constexpr (SECOND) c.sec = sec;
     if constexpr (REGION) {
         c.rg = rg;
     } else {
@@ -810,6 +862,7 @@ SB_DEVICE void fit_rows_g_body(const Geom& g, int count, const int* SB_RESTRICT 
     for (int i = 0; i < n_act; ++i) {
         const int p = s_list[i];
         c.slot = p;
+        if constexpr (SECOND) c.tpos = sec.angle_pos[s_fit[p].idx];
         if constexpr (MASKED) {
             // the companion's row pair first (its gbuf plane is comp_off slots further on); no
             // barrier between the two passes, for the reason given below
@@ -878,6 +931,27 @@ k_fit_rows_gmr(Geom g, int count, const int* SB_RESTRICT slots, const FitT* SB_R
                const float2* SB_RESTRICT tw, const int4* SB_RESTRICT cross, RegionOut rg) {
     fit_rows_g_body<N, true, true>(g, count, slots, fit, fitm, comp_off, gbuf, nullptr, nullptr, nullptr, tw, cross, 0,
                                    rg);
+}
+
+// the sweep of a secondary fit (sb_secondary_sweep): k_fit_rows_g / k_fit_rows_gm folding into best
+// state 1 (best_*) only the templates `sec` admits at each pixel
+template <int N>
+SB_GLOBAL SB_LAUNCH_BOUNDS((N / E > 256 ? N / E : 256), (N / E > 256 ? 1 : 2))
+k_fit_rows_gs(Geom g, int count, const int* SB_RESTRICT slots, const FitT* SB_RESTRICT fit,
+              const float4* SB_RESTRICT gbuf, float* SB_RESTRICT best_snr, float* SB_RESTRICT best_amp, int* best_idx,
+              const float2* SB_RESTRICT tw, const int4* SB_RESTRICT cross, long sub_stride, SecondOut sec) {
+    fit_rows_g_body<N, false, false, true>(g, count, slots, fit, nullptr, 0, gbuf, best_snr, best_amp, best_idx, tw,
+                                           cross, sub_stride, RegionOut(), sec);
+}
+
+template <int N>
+SB_GLOBAL SB_LAUNCH_BOUNDS((N / E > 256 ? N / E : 256), 1)
+k_fit_rows_gms(Geom g, int count, const int* SB_RESTRICT slots, const FitT* SB_RESTRICT fit,
+               const FitM* SB_RESTRICT fitm, int comp_off, const float4* SB_RESTRICT gbuf, float* SB_RESTRICT best_snr,
+               float* SB_RESTRICT best_amp, int* best_idx, const float2* SB_RESTRICT tw, const int4* SB_RESTRICT cross,
+               long sub_stride, SecondOut sec) {
+    fit_rows_g_body<N, true, false, true>(g, count, slots, fit, fitm, comp_off, gbuf, best_snr, best_amp, best_idx, tw,
+                                          cross, sub_stride, RegionOut(), sec);
 }
 
 // Hermitian split (sb_kernels.cuh) of the spectrum parked in natural order in `sm`

@@ -117,6 +117,9 @@ struct sb_plan {
     // rows (allocated on first use), and the per-flat-index age rank / orientation position tables
     Buf region, rtab;
     int region_words = 0, region_npos = 0, region_nranks = 0;
+    // secondary fit (sb_secondary_sweep): the winner's orientation position per pixel of the plan's
+    // rows (uint16; its per-flat-index position table goes in rtab)
+    Buf spos;
     int profile = 0;
     std::vector<sb_event_t> ev_pool;
     struct EvPair { int kind; sb_event_t a, b; };
@@ -484,6 +487,9 @@ struct SweepOut {
     // the threshold pass of a fit confidence region (sb_region_sweep): the fit kernel records the
     // templates that reach each pixel's threshold in these planes; no best state changes
     const sb::RegionOut* region = nullptr;
+    // the sweep of a secondary fit (sb_secondary_sweep): every record folds into best state 1, through
+    // the fit kernel's separation test
+    const sb::SecondOut* second = nullptr;
 };
 
 // the templates of one best state inside a chunk (one launch of the column kernel)
@@ -747,9 +753,18 @@ int run_sweep_t(sb_plan* pl, const sb_angle* angles, int n_angles, const sb_temp
             pl->d_bsnr = s2; pl->d_bamp = a2; pl->d_bidx = i2;
             pl->best_copies = nsub;
         }
-        const long cnt_x = (long)(nsub - 1) * sub_stride;
-        SB_OK(launch(pl, "k_best_init", sb::k_best_init, dim3(div_up(cnt_x, 256)), dim3(256), 0, cnt_x,
-                     pl->d_bsnr + sub_stride, pl->d_bamp + sub_stride, pl->d_bidx + sub_stride));
+        if (so.second) {
+            // state 1's copies only: an empty copy folded into state 0 could rewrite its indices
+            const long b1 = pl->bn();
+            for (int c = 1; c < nsub; ++c)
+                SB_OK(launch(pl, "k_best_init", sb::k_best_init, dim3(div_up(b1, 256)), dim3(256), 0, b1,
+                             pl->d_bsnr + c * sub_stride + b1, pl->d_bamp + c * sub_stride + b1,
+                             pl->d_bidx + c * sub_stride + b1));
+        } else {
+            const long cnt_x = (long)(nsub - 1) * sub_stride;
+            SB_OK(launch(pl, "k_best_init", sb::k_best_init, dim3(div_up(cnt_x, 256)), dim3(256), 0, cnt_x,
+                         pl->d_bsnr + sub_stride, pl->d_bamp + sub_stride, pl->d_bidx + sub_stride));
+        }
     }
 
     pl->last_geom[0] = Pym; pl->last_geom[1] = Pxm; pl->last_geom[2] = (int)ay.tiles.size();
@@ -933,9 +948,10 @@ int run_sweep_t(sb_plan* pl, const sb_angle* angles, int n_angles, const sb_temp
                     // fold: one launch per best state present in the chunk
                     for (auto& gp : ch.groups) {
                         const int* d_slots = gp.off < 0 ? nullptr : (const int*)pl->slots.p + gp.off;
-                        float* bsnr = pl->d_bsnr + (long)gp.state * bn - boff;
-                        float* bamp = pl->d_bamp + (long)gp.state * bn - boff;
-                        int* bidx = pl->d_bidx + (long)gp.state * bn - boff;
+                        const int state = so.second ? 1 : gp.state;
+                        float* bsnr = pl->d_bsnr + (long)state * bn - boff;
+                        float* bamp = pl->d_bamp + (long)state * bn - boff;
+                        int* bidx = pl->d_bidx + (long)state * bn - boff;
                         if constexpr (kF32) {
                             if (fast_fit) {
                                 const int4* cross = gp.err ? (const int4*)pl->cross.p : (const int4*)nullptr;
@@ -961,6 +977,24 @@ int run_sweep_t(sb_plan* pl, const sb_angle* angles, int n_angles, const sb_temp
                                                       S::smem_fit_f, g, gp.count, d_slots, (const sb::FitT*)pl->fit.p,
                                                       (const float4*)pl->gbuf.p, (const float2*)twx, cross,
                                                       *so.region);
+                                    }
+                                    if (so.second) {
+                                        if (masked) {
+                                            if constexpr (N <= kMaxFftMasked) {
+                                                return launch(pl, "k_fit_rows_gms", sb::k_fit_rows_gms<N>, grid,
+                                                              dim3(S::threads),
+                                                              S::smem_fit_f + sb::fit_masked_extra_smem<N>(), g,
+                                                              gp.count, d_slots, (const sb::FitT*)pl->fit.p,
+                                                              (const sb::FitM*)pl->fitm.p, ch.cnt,
+                                                              (const float4*)pl->gbuf.p, bsnr, bamp, bidx,
+                                                              (const float2*)twx, cross, sub_stride, *so.second);
+                                            }
+                                            return fail("internal: masked fit at FFT length " + std::to_string(N));
+                                        }
+                                        return launch(pl, "k_fit_rows_gs", sb::k_fit_rows_gs<N>, grid, dim3(S::threads),
+                                                      S::smem_fit_f, g, gp.count, d_slots, (const sb::FitT*)pl->fit.p,
+                                                      (const float4*)pl->gbuf.p, bsnr, bamp, bidx, (const float2*)twx,
+                                                      cross, sub_stride, *so.second);
                                     }
                                     if (masked) {
                                         // FFT lengths <= 4096 only: the park buffers need 2 N float2 per group
@@ -1004,15 +1038,18 @@ int run_sweep_t(sb_plan* pl, const sb_angle* angles, int n_angles, const sb_temp
                 }
             }
         }
+    // a secondary sweep folds and clears best state 1 alone
+    const long st_off = so.second ? bn : 0, st_len = so.second ? bn : sub_stride;
     if (nsub > 1 && !so.region) {
-        SB_OK(launch(pl, "k_best_fold", sb::k_best_fold, dim3(div_up(sub_stride, 256)), dim3(256), 0, sub_stride,
-                     nsub - 1, sub_stride, (const float*)pl->d_bsnr + sub_stride, (const float*)pl->d_bamp + sub_stride,
-                     (const int*)pl->d_bidx + sub_stride, pl->d_bsnr, pl->d_bamp, pl->d_bidx));
+        SB_OK(launch(pl, "k_best_fold", sb::k_best_fold, dim3(div_up(st_len, 256)), dim3(256), 0, st_len,
+                     nsub - 1, sub_stride, (const float*)pl->d_bsnr + sub_stride + st_off,
+                     (const float*)pl->d_bamp + sub_stride + st_off, (const int*)pl->d_bidx + sub_stride + st_off,
+                     pl->d_bsnr + st_off, pl->d_bamp + st_off, pl->d_bidx + st_off));
     }
     if (masked && !so.region) {
         SB_OK(launch(pl, "k_best_clear_nodata", sb::k_best_clear_nodata, dim3(div_up(bn, 256)), dim3(256), 0, pl->ny,
-                     pl->nx, pl->row0, pl->slab_lo, (int)pl->brows(), pl->n_states, bn, (const double*)pl->d_dem,
-                     pl->d_bsnr, pl->d_bamp, pl->d_bidx));
+                     pl->nx, pl->row0, pl->slab_lo, (int)pl->brows(), so.second ? 1 : pl->n_states, bn,
+                     (const double*)pl->d_dem, pl->d_bsnr + st_off, pl->d_bamp + st_off, pl->d_bidx + st_off));
     }
     drain_profile(pl);
     return 0;
@@ -1103,7 +1140,7 @@ int sb_plan_destroy(sb_plan* pl) {
     for (auto e : pl->ev_pool) sb_rt_event_destroy(e);
     for (Buf* b : {&pl->cr, &pl->fct, &pl->trt, &pl->part, &pl->gbuf, &pl->sums, &pl->fit, &pl->tmpls, &pl->angles,
                    &pl->tables, &pl->raw, &pl->tbox, &pl->slots, &pl->cross, &pl->casa, &pl->aux, &pl->spec9, &pl->coef,
-                   &pl->fitm, &pl->fs_idx, &pl->fs_out, &pl->region, &pl->rtab})
+                   &pl->fitm, &pl->fs_idx, &pl->fs_out, &pl->region, &pl->rtab, &pl->spos})
         release(*b);
 #ifndef SB_EMU
     if (pl->own_stream) cudaStreamDestroy(pl->stream);
@@ -1208,7 +1245,7 @@ long sb_plan_device_bytes(const sb_plan* pl) {
     b += (size_t)pl->bn() * pl->n_states * pl->best_copies * 12;
     for (const Buf* q : {&pl->cr, &pl->fct, &pl->trt, &pl->part, &pl->gbuf, &pl->sums, &pl->fit, &pl->tmpls, &pl->angles,
                          &pl->tables, &pl->raw, &pl->tbox, &pl->slots, &pl->cross, &pl->casa, &pl->aux, &pl->spec9, &pl->coef,
-                         &pl->fitm, &pl->fs_idx, &pl->fs_out, &pl->region, &pl->rtab})
+                         &pl->fitm, &pl->fs_idx, &pl->fs_out, &pl->region, &pl->rtab, &pl->spos})
         b += q->cap;
     return (long)b;
 }
@@ -1564,6 +1601,51 @@ int sb_region_sweep(sb_plan* pl, const sb_angle* angles, int n_angles, const sb_
     pl->region_words = words;
     pl->region_npos = n_pos;
     pl->region_nranks = n_ranks;
+    return 0;
+}
+
+int sb_secondary_sweep(sb_plan* pl, const sb_angle* angles, int n_angles, const sb_template* tmpls, int n_tmpls,
+                       const int32_t* whole_search5, const int32_t* angle_pos_host, int n_idx, int n_pos, int periodic,
+                       int min_sep_pos) {
+    if (!pl || !angles || !tmpls || !angle_pos_host || n_idx <= 0) return fail("sb_secondary_sweep: bad arguments");
+    if (pl->n_states < 2) return fail("sb_secondary_sweep: needs 2 best states (option \"states\"), the plan has " +
+                                      std::to_string(pl->n_states));
+    if (pl->precision != 32 || !pl->fast)
+        return fail("sb_secondary_sweep: secondary fit needs precision 32 and the option fast");
+    if (n_pos < 1 || n_pos > 256) return fail("sb_secondary_sweep: n_pos must be in 1 .. 256");
+    const int max_dist = periodic ? n_pos / 2 : n_pos - 1;
+    if (min_sep_pos < 1 || min_sep_pos > max_dist)
+        return fail("sb_secondary_sweep: min_sep_pos must be in 1 .. " + std::to_string(max_dist) +
+                    " (the largest distance between two orientation positions)");
+    for (int k = 0; k < n_idx; ++k)
+        if (angle_pos_host[k] < 0 || angle_pos_host[k] >= n_pos)
+            return fail("sb_secondary_sweep: orientation position out of range at flat index " + std::to_string(k));
+    for (int k = 0; k < n_tmpls; ++k) {
+        if (tmpls[k].idx < 0 || tmpls[k].idx >= n_idx)
+            return fail("sb_secondary_sweep: template flat index outside 0 .. n_idx - 1");
+        if (tmpls[k].state != 0)
+            return fail("sb_secondary_sweep: every record must be in best state 0 (state != 0)");
+    }
+    const long bn = pl->bn(), boff = (long)pl->slab_lo * pl->nx;
+    SB_OK(ensure(pl->rtab, (size_t)n_idx * sizeof(int32_t)));
+    SB_OK(ensure(pl->spos, (size_t)bn * sizeof(unsigned short)));
+    int* tab = (int*)pl->rtab.p;
+    unsigned short* pos = (unsigned short*)pl->spos.p;
+    SB_TRY(sb_rt_h2d(tab, angle_pos_host, (size_t)n_idx * sizeof(int32_t), pl->stream));
+    SB_OK(launch(pl, "k_secondary_pos", sb::k_secondary_pos, dim3(div_up(bn, 256)), dim3(256), 0, bn,
+                 (const float*)pl->d_bsnr, (const int*)pl->d_bidx, (const int*)tab, n_idx, pos));
+    SB_OK(launch(pl, "k_best_init", sb::k_best_init, dim3(div_up(bn, 256)), dim3(256), 0, bn, pl->d_bsnr + bn,
+                 pl->d_bamp + bn, pl->d_bidx + bn));
+    sb::SecondOut sec;
+    sec.pos = pos - boff;
+    sec.angle_pos = tab;
+    sec.n_pos = n_pos;
+    sec.min_sep = min_sep_pos;
+    sec.periodic = periodic ? 1 : 0;
+    SweepOut so;
+    so.second = &sec;
+    SB_OK(run_sweep(pl, angles, n_angles, tmpls, n_tmpls, so, whole_search5));
+    SB_TRY(sb_rt_sync(pl->stream));
     return 0;
 }
 

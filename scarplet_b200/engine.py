@@ -482,6 +482,20 @@ class Plan(object):
                                                  rank.ctypes.data, pos.ctypes.data, len(rank),
                                                  len(tables.pos_angle)))
 
+    def secondary_sweep(self, angle_records, template_records, tables, min_sep_pos):
+        """The sweep of a secondary fit (``sb_secondary_sweep``, DESIGN.md section 16): best state 0
+        must hold the result of ``sweep`` over the same records, on a plan with 2 best states.  Resets
+        best state 1 and sweeps the records into it, folding at each pixel only the templates at least
+        ``min_sep_pos`` orientation positions (``params.separation_positions``) from the winner of
+        state 0; ``tables``: ``params.region_tables`` of the search.  ``finalize(state=1)`` decodes
+        the result; state 0 is not modified."""
+        arr_a, na = angle_records
+        arr_t, nt = template_records[0], template_records[1]
+        whole = template_records[2] if len(template_records) > 2 else None
+        pos = np.ascontiguousarray(tables.angle_pos, dtype=np.int32)
+        check(self.lib, self.lib.sb_secondary_sweep(self._h, arr_a, na, arr_t, nt, whole, pos.ctypes.data, len(pos),
+                                                    len(tables.pos_angle), int(tables.periodic), int(min_sep_pos)))
+
     def region_finalize(self, age_of, angle_of, tables, rows=None):
         """(9, rows, nx) float64 [amp, age, angle, snr, age_lo, age_hi, angle_lo, angle_hi, n_fits] after
         ``region_sweep`` (``sb_region_finalize``): planes 0..3 are ``finalize``'s, 4..8 the region's

@@ -69,6 +69,28 @@ def region_tables(ages, angles, order="age_major"):
     return RegionTables(age_rank, angle_pos, np.sort(ages), angles[:n_pos].copy(), bool(periodic))
 
 
+def separation_positions(min_separation, angles):
+    """The orientation separation ``min_separation`` (radians) of a secondary fit as a whole number of
+    orientation positions of ``region_tables(ages, angles)``: ``ceil(min_separation / step - 1e-9)``
+    with ``step = angles[1] - angles[0]``, so that 10 degrees on the 1-degree grid is 10 positions.
+    ``ValueError`` for a single orientation, a ``min_separation`` that is not finite or gives less
+    than 1 position, and more positions than the largest distance between two positions
+    (``n_pos // 2`` in a periodic search, ``len(angles) - 1`` otherwise)."""
+    angles = np.atleast_1d(np.asarray(angles, dtype=np.float64))
+    if len(angles) < 2:
+        raise ValueError("a secondary fit needs at least 2 orientations, not %d" % len(angles))
+    if not np.isfinite(min_separation):
+        raise ValueError("min_separation must be finite, not %r" % (min_separation,))
+    m = int(np.ceil(float(min_separation) / (angles[1] - angles[0]) - 1e-9))
+    t = region_tables([1.0], angles)
+    n_pos = len(t.pos_angle)
+    max_dist = n_pos // 2 if t.periodic else n_pos - 1
+    if not 1 <= m <= max_dist:
+        raise ValueError("min_separation %r is %d orientation positions; it must be 1 .. %d" % (min_separation, m,
+                                                                                               max_dist))
+    return m
+
+
 def default_ages():
     """core.py:107, 286"""
     return 10 ** np.arange(0, 3.5, 0.1)
