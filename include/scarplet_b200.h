@@ -269,6 +269,45 @@ int sb_secondary_sweep(sb_plan* plan, const sb_angle* angles, int n_angles, cons
                        const int32_t* whole_search5, const int32_t* angle_pos_host, int n_idx, int n_pos,
                        int periodic, int min_sep_pos);
 
+/* Sub-grid fit peak (DESIGN §17), pass 2 of 2: best state 0 must hold the result of a sweep
+ * (sb_sweep / sb_sweep_ex) over the same records.  Runs that sweep again with the peak variant of
+ * the fit kernel, which writes no best state.  The winner of state 0 at a pixel (where its SNR is
+ * > 0) has age rank r = age_rank_host[idx] (0 .. n_ranks - 1) and orientation position
+ * p = angle_pos_host[idx] (0 .. n_pos - 1).  The plan's four neighbour planes (float32, cleared
+ * first) receive per pixel the largest SNR s > 0 of the records at (r - 1, p), (r + 1, p), (r, p - 1)
+ * and (r, p + 1) -- positions wrap round when periodic -- that the masks (window, get_err_mask,
+ * min_coverage) leave a candidate there; 0 where there is none.  The winner and its periodic twin
+ * are not recorded.  Integer atomics: the result does not depend on batches, sub-streams or launch
+ * order.  Device memory: 20 B per pixel of the plan's rows (the four planes and a winner code
+ * plane), allocated on first use.
+ * Fails for precision 64 or fast = 0, n_ranks or n_pos outside 1 .. 65535 (16-bit fields of the
+ * winner code), a periodic search with n_pos < 3, ranks / positions out of range, and a record whose
+ * idx is outside 0 .. n_idx - 1 or whose state is not 0. */
+int sb_peak_sweep(sb_plan* plan, const sb_angle* angles, int n_angles, const sb_template* tmpls, int n_tmpls,
+                  const int32_t* whole_search5, const int32_t* age_rank_host, const int32_t* angle_pos_host,
+                  int n_idx, int n_ranks, int n_pos, int periodic);
+
+/* Decode the fit peak for raster rows row_lo .. row_hi-1: out8 = host float64[8][rows][nx]
+ *   [0..3] amp, age, angle, snr of best state 0 (as sb_finalize_ex);
+ *   [4] age_peak: 10^(x[r] + u), u the vertex of the parabola through (x[r -+ 1], s_age-+) and
+ *       (x[r], snr), x = log10_rank_age_host (log10 of the sorted ages), where 0 < r < n_ranks - 1,
+ *       both neighbours are > 0 and d- + d+ > 0 (d-+ = snr - s_age-+); the grid age elsewhere;
+ *   [5] angle_peak = angle + step * (d- - d+) / (2 (d- + d+)) from the orientation neighbours, where
+ *       the winner has both (periodic with n_pos >= 3, or 0 < p < n_pos - 1), they are > 0 and
+ *       d- + d+ > 0; the grid angle elsewhere;
+ *   [6] snr_peak = snr + the gain of the refined axes;  [7] refined = 1 (age) + 2 (orientation).
+ * Float64 without contraction.  Planes 4..7 are 0 where state 0's SNR is 0, [0, 0, NaN, 0] where it
+ * is NaN.  Fails without a peak sweep since the best state was last allocated (option "states",
+ * sb_plan_set_slab), for n_ranks / n_pos other than the sweep's, and rows outside the plan. */
+int sb_peak_finalize(sb_plan* plan, int row_lo, int row_hi, const double* age_of_host, const double* angle_of_host,
+                     int n_idx, const double* log10_rank_age_host, int n_ranks, int n_pos, int periodic, double step,
+                     double* out8);
+
+/* The neighbour planes of the last peak sweep: int32 device memory, the bits of float32 SNRs >= 0
+ * (they order as integers), plane j (0 age-, 1 age+, 2 orientation-, 3 orientation+) of pixel i of
+ * the plan's rows at [j * rows * nx + i]. */
+int sb_peak_planes(sb_plan* plan, int32_t** planes_dev);
+
 /* Raw best state for a cross-GPU merge: device pointers into the plan, one value per pixel of
  * the plan's rows. */
 int sb_best_state(sb_plan* plan, float** snr_dev, float** amp_dev, int32_t** idx_dev);

@@ -73,6 +73,11 @@ def _declare(lib):
     lib.sb_secondary_sweep.argtypes = [P, POINTER(SbAngle), c_int, POINTER(SbTemplate), c_int, POINTER(c_int32),
                                        c_void_p, c_int, c_int, c_int, c_int]
     lib.sb_region_merge.argtypes = [P, c_int, c_int, c_int, c_void_p]
+    lib.sb_peak_sweep.argtypes = [P, POINTER(SbAngle), c_int, POINTER(SbTemplate), c_int, POINTER(c_int32), c_void_p,
+                                  c_void_p, c_int, c_int, c_int, c_int]
+    lib.sb_peak_finalize.argtypes = [P, c_int, c_int, c_void_p, c_void_p, c_int, c_void_p, c_int, c_int, c_int,
+                                     c_double, c_void_p]
+    lib.sb_peak_planes.argtypes = [P, POINTER(c_void_p)]
     lib.sb_curvature_noise_moments.argtypes = [P, c_double, c_double, dp]
     lib.sb_fill_nodata.argtypes = [P, c_void_p, c_double, POINTER(c_long)]
     lib.sb_plan_last_geometry.argtypes = [P, POINTER(c_int)]
@@ -112,7 +117,7 @@ def _declare(lib):
                  "sb_plan_curv_stats", "sb_plan_set_curv_stats", "sb_finalize_ex", "sb_best_state_ex",
                  "sb_best_merge", "sb_curvature_noise_moments", "sb_fill_nodata", "sb_plan_set_nodata",
                  "sb_fit_surface", "sb_age_range", "sb_region_sweep", "sb_region_finalize", "sb_region_planes",
-                 "sb_region_merge", "sb_secondary_sweep"):
+                 "sb_region_merge", "sb_secondary_sweep", "sb_peak_sweep", "sb_peak_finalize", "sb_peak_planes"):
         getattr(lib, name).restype = c_int
     return lib
 
@@ -128,7 +133,7 @@ EXPORTED = ("sb_last_error", "sb_build_info", "sb_plan_create", "sb_plan_destroy
             "sb_finalize_ex", "sb_best_state_ex", "sb_best_merge", "sb_curvature_noise_moments",
             "sb_fill_nodata", "sb_debug_fft_bench", "sb_sweep_ex", "sb_plan_set_nodata", "sb_fit_surface",
             "sb_age_range", "sb_region_sweep", "sb_region_finalize", "sb_region_planes", "sb_region_merge",
-            "sb_secondary_sweep")
+            "sb_secondary_sweep", "sb_peak_sweep", "sb_peak_finalize", "sb_peak_planes")
 
 
 def library_path():

@@ -287,7 +287,7 @@ def fit_surface(data, Template, scale, pixels, ages=None, ang_min=-np.pi / 2, an
     return FitSurface(amp, snr, ages, angles)
 
 
-def _age_search(name, Template, ages, kwargs, snr_ratio=None, max_ages=64, angles=None):
+def _age_search(name, Template, ages, kwargs, snr_ratio=None, max_ages=64, angles=None, max_angles=256):
     """(device spec, float64 ages) of an age-resolved search; ``ValueError`` for what it does not take."""
     if kwargs:
         raise ValueError("%s takes no template keyword arguments (%s): the per-age states need a built-in "
@@ -295,15 +295,15 @@ def _age_search(name, Template, ages, kwargs, snr_ratio=None, max_ages=64, angle
     spec = device_spec(Template)
     if spec is None:
         raise ValueError("%s needs a built-in template class; %r has no on-device generator" % (name, Template))
-    return spec, search_args(name, ages, snr_ratio, max_ages, angles)
+    return spec, search_args(name, ages, snr_ratio, max_ages, angles, max_angles)
 
 
-def search_args(name, ages, snr_ratio=None, max_ages=64, angles=None):
+def search_args(name, ages, snr_ratio=None, max_ages=64, angles=None, max_angles=256):
     """Float64 ages of an age-resolved search or a fit region (``None``: the 35 default ages);
     ``ValueError`` for what ``name`` does not take: no or more than ``max_ages`` ages (``None``: no
     limit), duplicate ages, ``snr_ratio`` outside (0, 1] and, when ``angles`` is given (a fit region),
-    more than 256 orientations.  Shared by ``core`` and the multi-GPU drivers of ``distributed``,
-    which check before any device work or collective."""
+    more than ``max_angles`` orientations.  Shared by ``core`` and the multi-GPU drivers of
+    ``distributed``, which check before any device work or collective."""
     ages = P.default_ages() if ages is None else np.atleast_1d(np.asarray(ages, dtype=np.float64))
     if max_ages is None:
         if ages.ndim != 1 or len(ages) < 1:
@@ -314,8 +314,8 @@ def search_args(name, ages, snr_ratio=None, max_ages=64, angles=None):
         raise ValueError("%s: duplicate ages" % name)
     if snr_ratio is not None and not (np.isfinite(snr_ratio) and 0.0 < snr_ratio <= 1.0):
         raise ValueError("snr_ratio must be in (0, 1], not %r" % (snr_ratio,))
-    if angles is not None and len(angles) > 256:
-        raise ValueError("%s takes at most 256 orientations, not %d" % (name, len(angles)))
+    if angles is not None and len(angles) > max_angles:
+        raise ValueError("%s takes at most %d orientations, not %d" % (name, max_angles, len(angles)))
     return ages
 
 
@@ -430,6 +430,46 @@ def secondary_fit(data, Template, scale, min_separation, ages=None, ang_min=-np.
         plan.finalize(age_of, angle_of, state=0, out=out[:4])
         plan.finalize(age_of, angle_of, state=1, out=out[4:])
         return out
+
+
+def fit_peak(data, Template, scale, ages=None, ang_min=-np.pi / 2, ang_max=np.pi / 2, nodata="propagate",
+             min_coverage=1.0, **kwargs):
+    """Each pixel's age and orientation between the grid points: the vertex of the parabola through
+    the SNR of its best template and of the templates one age and one orientation either side.
+    Returns (8, ny, nx) float64 [amp, age, angle, snr, age_peak, angle_peak, snr_peak, refined]:
+
+    * planes 0..3 are exactly ``match(data, Template, scale=scale, ages=ages, ...)``;
+    * the winner has age rank r and orientation position p (``params.region_tables``); its neighbour
+      values are the largest float32 SNR > 0 among the templates at (r -+ 1, p) and (r, p -+ 1) that
+      the masks leave a candidate at the pixel, 0 where there is none.  A search spanning pi (the
+      default) is periodic: -pi/2 and pi/2 share position 0 and positions wrap round;
+    * the age axis is refined where 0 < r < len(ages) - 1, both neighbours are > 0 and
+      d- + d+ > 0 (d-+ = snr - neighbour, in float64).  On x = log10(sorted ages), with
+      h- = x[r] - x[r-1] and h+ = x[r+1] - x[r], ``age_peak = 10 ** (x[r] + u)`` with
+      ``u = (d- h+^2 - d+ h-^2) / (2 (d- h+ + d+ h-))`` in [-h-/2, h+/2];
+    * the orientation axis is refined where the winner has both orientation neighbours (always in
+      a periodic search), they are > 0 and d- + d+ > 0: ``angle_peak = angle + step * (d- - d+) /
+      (2 (d- + d+))``, within half a step of ``angle``;
+    * ``snr_peak`` is ``snr`` plus the gain of each refined axis (the maximum of the separable
+      quadratic), ``refined`` is 1 (age) + 2 (orientation); an unrefined axis keeps its grid value.
+
+    Planes 4..7 are 0 where the pixel has no fit and ``[0, 0, NaN, 0]`` where plane 3 is NaN.  Two
+    device sweeps on one plan (DESIGN.md section 17): ``match``'s, then a neighbour pass that
+    records the four neighbour SNRs.  Device memory beyond ``match``'s: 20 B per pixel (336 MB at
+    4096^2).  Built-in template classes only, distinct ages; at most 65535 ages and orientations
+    (the 16-bit fields of the winner's code); ``nodata`` / ``min_coverage``: see
+    ``calculate_best_fit_parameters``."""
+    angles = P.search_angles(ang_min, ang_max)
+    spec, ages = _age_search("fit_peak", Template, ages, kwargs, max_ages=None, angles=angles, max_angles=0xffff)
+    if len(ages) > 0xffff:
+        raise ValueError("fit_peak takes at most 65535 ages, not %d" % len(ages))
+    tables = P.region_tables(ages, angles)
+    with _plan_for(data, nodata=nodata, min_coverage=min_coverage) as plan:
+        a_rec, t_rec, age_of, angle_of = plan.build_sweep(spec, scale, ages, angles, "age_major")
+        plan.reset()
+        plan.sweep(a_rec, t_rec)
+        plan.peak_sweep(a_rec, t_rec, tables)
+        return plan.peak_finalize(age_of, angle_of, tables)
 
 
 def compare(results, ny, nx):

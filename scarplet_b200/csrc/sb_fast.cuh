@@ -501,6 +501,102 @@ SB_GLOBAL k_secondary_pos(long n, const float* SB_RESTRICT snr, const int* SB_RE
 }
 
 // ---------------------------------------------------------------------------
+// Sub-grid fit peak (DESIGN.md 17): a second sweep of the same templates records, at each pixel, the
+// largest SNR of each of the four axis neighbours of the winner of best state 0 -- the templates one
+// age rank either side at its orientation position, and one position either side at its age rank.
+// The running-best registers hold each pixel's winner code (rank << 16 | pos, k_peak_code); every
+// template carries the four winner codes it neighbours (`codes`, built on the host with the periodic
+// wrap), so the test per pixel is four integer compares.  A hit is an integer atomicMax of the SNR's
+// bits (positive floats order as their bits): the planes do not depend on batches, sub-streams or
+// launch order.
+// ---------------------------------------------------------------------------
+constexpr unsigned kNoCode = 0xffffffffu;          // code of a pixel without a fit: it neighbours nothing
+
+struct PeakOut {
+    const unsigned* code;     // winner code per pixel, addressed by raster row (gi * nx + gj)
+    int* planes;              // [age-][age+][ang-][ang+] float32 SNR bits, addressed like `code`
+    const int4* codes;        // per flat index: the winner codes whose age-, age+, ang-, ang+ neighbour
+                              // it is (0xfffffffe where there is none: rank 0xffff is nobody's)
+    long plane;               // elements of one plane
+};
+
+template <bool PEAK> struct PeakSlot {};
+template <> struct PeakSlot<true> {
+    PeakOut pk;
+    int4 tcodes;              // `codes` of the current template
+};
+
+// the code plane of a fit peak from best state 0: (age rank << 16) | orientation position of the winner
+// where decode_best sees a hit (SNR > 0, index in range), kNoCode elsewhere (no fit, NaN)
+SB_GLOBAL k_peak_code(long n, const float* SB_RESTRICT snr, const int* SB_RESTRICT idx,
+                      const int* SB_RESTRICT age_rank, const int* SB_RESTRICT angle_pos, int n_idx,
+                      unsigned* SB_RESTRICT code) {
+    const long i = (long)sb_bx() * 256 + sb_tid();
+    if (i >= n) return;
+    const int k = idx[i];
+    code[i] = (snr[i] > 0.f && k >= 0 && k < n_idx) ? ((unsigned)age_rank[k] << 16) | (unsigned)angle_pos[k] : kNoCode;
+}
+
+// Fit peak (sb_peak_finalize): [amp, age, angle, snr] of best state 0 as k_finalize decodes it, then
+// [age_peak, angle_peak, snr_peak, refined] from the winner code and the four neighbour SNRs, by the
+// vertex of the parabola through the winner and its two neighbours on each axis (ages on the log10
+// axis `lx`, log10 of the sorted ages).  Float64 without contraction (sb_mul ...), so that planes 5..7
+// can equal a NumPy restatement bit for bit; only age_peak goes through exp10.  Planes 4..7 are 0
+// where the pixel has no fit, [0, 0, NaN, 0] where its SNR is NaN.
+SB_GLOBAL k_peak_finalize(long n, long plane, const float* SB_RESTRICT snr, const float* SB_RESTRICT amp,
+                          const int* SB_RESTRICT idx, const unsigned* SB_RESTRICT code,
+                          const float* SB_RESTRICT nb, const double* SB_RESTRICT age_of,
+                          const double* SB_RESTRICT angle_of, int n_idx, const double* SB_RESTRICT lx, int n_ranks,
+                          int n_pos, int periodic, double step, double* SB_RESTRICT out8) {
+    const long i = (long)sb_bx() * 256 + sb_tid();
+    if (i >= n) return;
+    const float s = snr[i];
+    double o[4];
+    decode_best(s, idx[i], amp + i, age_of, angle_of, n_idx, o);
+    double age_pk = 0.0, ang_pk = 0.0, snr_pk = s != s ? (double)s : 0.0, refined = 0.0;
+    if (o[3] > 0.0) {
+        const double s0 = o[3];
+        const unsigned c = code[i];
+        const int r = (int)(c >> 16), p = (int)(c & 0xffffu);
+        const double am = (double)nb[i], ap = (double)nb[plane + i];
+        const double gm = (double)nb[2 * plane + i], gp = (double)nb[3 * plane + i];
+        double g_age = 0.0, g_ang = 0.0;
+        age_pk = o[1];
+        ang_pk = o[2];
+        if (r > 0 && r < n_ranks - 1 && am > 0.0 && ap > 0.0) {
+            const double dm = sb_sub(s0, am), dp = sb_sub(s0, ap);
+            if (sb_add(dm, dp) > 0.0) {
+                const double hm = sb_sub(lx[r], lx[r - 1]), hp = sb_sub(lx[r + 1], lx[r]);
+                const double num = sb_sub(sb_mul(dm, sb_mul(hp, hp)), sb_mul(dp, sb_mul(hm, hm)));
+                const double u = sb_div(num, sb_mul(2.0, sb_add(sb_mul(dm, hp), sb_mul(dp, hm))));
+                age_pk = exp10(sb_add(lx[r], u));
+                g_age = sb_div(sb_mul(u, num), sb_mul(sb_mul(sb_mul(2.0, hm), hp), sb_add(hm, hp)));
+                refined = 1.0;
+            }
+        }
+        if ((periodic ? n_pos >= 3 : (p > 0 && p < n_pos - 1)) && gm > 0.0 && gp > 0.0) {
+            const double dm = sb_sub(s0, gm), dp = sb_sub(s0, gp);
+            const double sum = sb_add(dm, dp);
+            if (sum > 0.0) {
+                const double t = sb_sub(dm, dp);
+                ang_pk = sb_add(o[2], sb_mul(sb_div(t, sb_mul(2.0, sum)), step));
+                g_ang = sb_div(sb_mul(t, t), sb_mul(8.0, sum));
+                refined = sb_add(refined, 2.0);
+            }
+        }
+        snr_pk = sb_add(sb_add(s0, g_age), g_ang);
+    }
+    out8[i] = o[0];
+    out8[n + i] = o[1];
+    out8[2 * n + i] = o[2];
+    out8[3 * n + i] = o[3];
+    out8[4 * n + i] = age_pk;
+    out8[5 * n + i] = ang_pk;
+    out8[6 * n + i] = snr_pk;
+    out8[7 * n + i] = refined;
+}
+
+// ---------------------------------------------------------------------------
 // k_fit_rows_g<Px>: grid (Py / 2 / GP).  The two transforms
 // a thread group pipelines are the two raster rows that share every 32-byte sector of the
 // interleaved planes (gbuf_index), of ONE template: a thread fetches whole sectors with
@@ -514,8 +610,10 @@ SB_GLOBAL k_secondary_pos(long n, const float* SB_RESTRICT snr, const int* SB_RE
 // REGION (k_fit_rows_gr / _gmr): bsA / bsB hold each pixel's region threshold (region_threshold) and
 // never change; a candidate is confirmed in float64 and recorded in the region planes (region_hit).
 // SECOND (k_fit_rows_gs / _gms): a candidate the separation rules out (second_ok) is skipped.
-template <int N, bool MASKED = false, bool REGION = false, bool SECOND = false>
-struct FitPairCtx : RegionSlot<REGION>, SecondSlot<SECOND> {
+// PEAK (k_fit_rows_gp / _gmp): bsA / bsB hold each pixel's winner code (as float bits) and never
+// change; a template that neighbours the winner (peak_any) and has SNR > 0 is recorded (peak_hit).
+template <int N, bool MASKED = false, bool REGION = false, bool SECOND = false, bool PEAK = false>
+struct FitPairCtx : RegionSlot<REGION>, SecondSlot<SECOND>, PeakSlot<PEAK> {
     static constexpr int K = sbfft::num_stages(N);
     static constexpr int T = N / E;
     static constexpr int LOG2T = ilog2(T);
@@ -592,6 +690,20 @@ struct FitPairCtx : RegionSlot<REGION>, SecondSlot<SECOND> {
         return d >= s.min_sep;
     }
 
+    // PEAK: the current template is an axis neighbour of the winner of code `c`
+    SB_DEVICE bool peak_any(unsigned c) const {
+        const int4 t = this->tcodes;
+        const int v = (int)c;
+        return (v == t.x) | (v == t.y) | (v == t.z) | (v == t.w);
+    }
+    // PEAK: record SNR `snr` > 0 of the current template, a neighbour of code `c`, at pixel `pix`
+    SB_DEVICE void peak_hit(long pix, unsigned c, float snr) const {
+        const int4 t = this->tcodes;
+        const int v = (int)c;
+        const int j = v == t.x ? 0 : v == t.y ? 1 : v == t.z ? 2 : 3;
+        sb_atomic_max(this->pk.planes + j * this->pk.plane + pix, (int)sb_float_bits(snr));
+    }
+
     template <int F> SB_DEVICE void epilogue(const float2 (&v)[E], float (&bs)[E]) {
         const int gi = F == 0 ? giA : giB;
         const FitT k = s_fit[slot];
@@ -604,6 +716,11 @@ struct FitPairCtx : RegionSlot<REGION>, SecondSlot<SECOND> {
             if constexpr (MASKED) fit_pixel_masked(v[q].y, v[q].x, k, s_fm[slot], park[F * N + t + q * T], amp, snr);
             else fit_pixel_fast(v[q].y, v[q].x, k, amp, snr);
             snr = ((mk >> q) & 1u) ? snr : -1.f;              // edge-masked: never wins
+            if constexpr (PEAK) {
+                const unsigned cq = sb_float_bits(bs[q]);
+                if (snr > 0.f && peak_any(cq)) peak_hit((long)gi * nx + ox + ((m0 + q * T) & (N - 1)), cq, snr);
+                continue;
+            }
             // first maximum wins (core.py:230-240); equal positive SNRs (in float32 mostly the
             // -90 / +90 degree pair) go to the lower flat index, whatever the batch order.
             // (A branch-free select over the 16 pixels was measured 3 % slower: it spills.)
@@ -655,8 +772,13 @@ struct FitPairCtx : RegionSlot<REGION>, SecondSlot<SECOND> {
             const float s_hi = fabsf(sb_fdiv_fast(t1.y, err.y));
             snr2[j] = make_float2(s_lo, s_hi);
             // (a NaN SNR -- NaN in the DEM -- never wins here; k_poison_windows marks those pixels)
-            cand |= (s_lo >= bs[j] && s_lo > 0.f) ? (1u << j) : 0u;
-            cand |= (s_hi >= bs[j + 8] && s_hi > 0.f) ? (1u << (j + 8)) : 0u;
+            if constexpr (PEAK) {
+                cand |= (s_lo > 0.f && peak_any(sb_float_bits(bs[j]))) ? (1u << j) : 0u;
+                cand |= (s_hi > 0.f && peak_any(sb_float_bits(bs[j + 8]))) ? (1u << (j + 8)) : 0u;
+            } else {
+                cand |= (s_lo >= bs[j] && s_lo > 0.f) ? (1u << j) : 0u;
+                cand |= (s_hi >= bs[j + 8] && s_hi > 0.f) ? (1u << (j + 8)) : 0u;
+            }
         }
         cand &= mk;                                                            // edge-masked: never wins
         if (cand != 0u) {
@@ -670,6 +792,10 @@ struct FitPairCtx : RegionSlot<REGION>, SecondSlot<SECOND> {
                     const float snr = q < 8 ? snr2[q & 7].x : snr2[q & 7].y;
                     const float amp = q < 8 ? amp2[q & 7].x : amp2[q & 7].y;
                     const int jo = (m0 + q * T) & (N - 1);
+                    if constexpr (PEAK) {
+                        peak_hit((long)gi * nx + ox + jo, sb_float_bits(bs[q]), snr);
+                        continue;
+                    }
                     if constexpr (REGION) {
                         region_hit((long)gi * nx + ox + jo, snr, k.idx);
                         continue;
@@ -738,12 +864,13 @@ SB_CONSTEXPR size_t fit_masked_extra_smem() {
     return kFitMaxBatch * sizeof(FitM) + (size_t)((N / E > 256 ? N / E : 256) / (N / E)) * 2 * N * sizeof(float2);
 }
 
-template <int N, bool MASKED, bool REGION = false, bool SECOND = false>
+template <int N, bool MASKED, bool REGION = false, bool SECOND = false, bool PEAK = false>
 SB_DEVICE void fit_rows_g_body(const Geom& g, int count, const int* SB_RESTRICT slots, const FitT* SB_RESTRICT fit,
                                const FitM* SB_RESTRICT fitm, int comp_off, const float4* SB_RESTRICT gbuf,
                                float* SB_RESTRICT best_snr, float* SB_RESTRICT best_amp, int* best_idx,
                                const float2* SB_RESTRICT tw, const int4* SB_RESTRICT cross, long sub_stride,
-                               const RegionOut& rg = RegionOut(), const SecondOut& sec = SecondOut()) {
+                               const RegionOut& rg = RegionOut(), const SecondOut& sec = SecondOut(),
+                               const PeakOut& pk = PeakOut()) {
     // grid.y > 1 (small rasters, whose row pairs alone do not fill the GPU): the templates of the
     // launch are dealt round-robin to grid.y sub-streams; sub-stream j folds into copy j of the
     // best state (best_* + j * sub_stride; copy 0 is the state itself) and k_best_fold merges the
@@ -756,11 +883,12 @@ SB_DEVICE void fit_rows_g_body(const Geom& g, int count, const int* SB_RESTRICT 
     // REGION: best_* are unused; the thresholds come from rg.best (state 0 for every sub-stream)
     // and nothing writes a best state.
     // SECOND: best_* are state 1's planes; `sec` rules out the templates too close to the winner.
+    // PEAK: as REGION, with the winner codes of pk.code and the neighbour planes of `pk`.
     constexpr int T = N / E;
     constexpr int THREADS = T > 256 ? T : 256;
     constexpr int GP = THREADS / T;
     constexpr int PL = sbfft::padded_len(N);
-    typedef FitPairCtx<N, MASKED, REGION, SECOND> Ctx;
+    typedef FitPairCtx<N, MASKED, REGION, SECOND, PEAK> Ctx;
     const int grp = sb_tid() / T, t = sb_tid() % T;
     float2* sm = (float2*)sb_shared();
     FitT* s_fit = (FitT*)(sm + (long)GP * 2 * PL);
@@ -830,6 +958,8 @@ SB_DEVICE void fit_rows_g_body(const Geom& g, int count, const int* SB_RESTRICT 
     if constexpr (SECOND) c.sec = sec;
     if constexpr (REGION) {
         c.rg = rg;
+    } else if constexpr (PEAK) {
+        c.pk = pk;
     } else {
         best_snr += sb_by() * sub_stride;
         best_amp += sb_by() * sub_stride;
@@ -846,6 +976,9 @@ SB_DEVICE void fit_rows_g_body(const Geom& g, int count, const int* SB_RESTRICT 
         if constexpr (REGION) {
             bsA[q] = (actA && in) ? region_threshold(rg.best[(long)c.giA * g.nx + g.ox + jo], rg.ratio) : INFINITY;
             bsB[q] = (actB && in) ? region_threshold(rg.best[(long)c.giB * g.nx + g.ox + jo], rg.ratio) : INFINITY;
+        } else if constexpr (PEAK) {
+            bsA[q] = sb_bits_float((actA && in) ? pk.code[(long)c.giA * g.nx + g.ox + jo] : kNoCode);
+            bsB[q] = sb_bits_float((actB && in) ? pk.code[(long)c.giB * g.nx + g.ox + jo] : kNoCode);
         } else {
             bsA[q] = (actA && in) ? best_snr[(long)c.giA * g.nx + g.ox + jo] : 0.f;
             bsB[q] = (actB && in) ? best_snr[(long)c.giB * g.nx + g.ox + jo] : 0.f;
@@ -863,6 +996,7 @@ SB_DEVICE void fit_rows_g_body(const Geom& g, int count, const int* SB_RESTRICT 
         const int p = s_list[i];
         c.slot = p;
         if constexpr (SECOND) c.tpos = sec.angle_pos[s_fit[p].idx];
+        if constexpr (PEAK) c.tcodes = pk.codes[s_fit[p].idx];
         if constexpr (MASKED) {
             // the companion's row pair first (its gbuf plane is comp_off slots further on); no
             // barrier between the two passes, for the reason given below
@@ -882,7 +1016,7 @@ SB_DEVICE void fit_rows_g_body(const Geom& g, int count, const int* SB_RESTRICT 
         // buffer B is next written after the coming template's first barrier
         leapfrog<Ctx::K>(c, va, vb);
     }
-    if constexpr (!REGION) {
+    if constexpr (!REGION && !PEAK) {
 #pragma unroll
         for (int q = 0; q < E; ++q) {
             const int jo = (t + q * T + g.dlx) & (N - 1);
@@ -952,6 +1086,26 @@ k_fit_rows_gms(Geom g, int count, const int* SB_RESTRICT slots, const FitT* SB_R
                long sub_stride, SecondOut sec) {
     fit_rows_g_body<N, true, false, true>(g, count, slots, fit, fitm, comp_off, gbuf, best_snr, best_amp, best_idx, tw,
                                           cross, sub_stride, RegionOut(), sec);
+}
+
+// the neighbour pass of a fit peak (sb_peak_sweep): k_fit_rows_g / k_fit_rows_gm recording the axis
+// neighbours of each pixel's winner in the planes of `pk`; grid.y sub-streams all read state 0
+template <int N>
+SB_GLOBAL SB_LAUNCH_BOUNDS((N / E > 256 ? N / E : 256), (N / E > 256 ? 1 : 2))
+k_fit_rows_gp(Geom g, int count, const int* SB_RESTRICT slots, const FitT* SB_RESTRICT fit,
+              const float4* SB_RESTRICT gbuf, const float2* SB_RESTRICT tw, const int4* SB_RESTRICT cross,
+              PeakOut pk) {
+    fit_rows_g_body<N, false, false, false, true>(g, count, slots, fit, nullptr, 0, gbuf, nullptr, nullptr, nullptr, tw,
+                                                  cross, 0, RegionOut(), SecondOut(), pk);
+}
+
+template <int N>
+SB_GLOBAL SB_LAUNCH_BOUNDS((N / E > 256 ? N / E : 256), 1)
+k_fit_rows_gmp(Geom g, int count, const int* SB_RESTRICT slots, const FitT* SB_RESTRICT fit,
+               const FitM* SB_RESTRICT fitm, int comp_off, const float4* SB_RESTRICT gbuf,
+               const float2* SB_RESTRICT tw, const int4* SB_RESTRICT cross, PeakOut pk) {
+    fit_rows_g_body<N, true, false, false, true>(g, count, slots, fit, fitm, comp_off, gbuf, nullptr, nullptr, nullptr,
+                                                 tw, cross, 0, RegionOut(), SecondOut(), pk);
 }
 
 // Hermitian split (sb_kernels.cuh) of the spectrum parked in natural order in `sm`

@@ -120,6 +120,10 @@ struct sb_plan {
     // secondary fit (sb_secondary_sweep): the winner's orientation position per pixel of the plan's
     // rows (uint16; its per-flat-index position table goes in rtab)
     Buf spos;
+    // fit peak (sb_peak_sweep): four neighbour SNR planes and the winner code plane of the plan's rows
+    // (allocated on first use), and the ranks / positions of the sweep that wrote them (0: none)
+    Buf peak;
+    int peak_nranks = 0, peak_npos = 0;
     int profile = 0;
     std::vector<sb_event_t> ev_pool;
     struct EvPair { int kind; sb_event_t a, b; };
@@ -306,6 +310,7 @@ int alloc_best(sb_plan* pl) {
     pl->d_bsnr = nullptr; pl->d_bamp = nullptr; pl->d_bidx = nullptr;
     pl->best_copies = 1;
     pl->region_npos = 0;           // region planes of the old rows / states are void
+    pl->peak_npos = 0;             // and so are the fit peak's
     const size_t n = (size_t)pl->bn() * pl->n_states;
     int e = 0;
     e |= sb_rt_malloc((void**)&pl->d_bsnr, n * sizeof(float));
@@ -490,6 +495,9 @@ struct SweepOut {
     // the sweep of a secondary fit (sb_secondary_sweep): every record folds into best state 1, through
     // the fit kernel's separation test
     const sb::SecondOut* second = nullptr;
+    // the neighbour pass of a fit peak (sb_peak_sweep): the fit kernel records the axis neighbours of
+    // each pixel's winner in these planes; no best state changes
+    const sb::PeakOut* peak = nullptr;
 };
 
 // the templates of one best state inside a chunk (one launch of the column kernel)
@@ -525,6 +533,9 @@ int run_sweep_t(sb_plan* pl, const sb_angle* angles, int n_angles, const sb_temp
     if (masked && so.raw_amp) return fail("nodata mask: sb_match_template keeps the reference's NaN semantics");
     if (masked && !fast) return fail("nodata mask needs precision 32 and the option fast");
     if (so.region && !fast) return fail("fit region needs precision 32 and the option fast");
+    if (so.peak && !fast) return fail("fit peak needs precision 32 and the option fast");
+    // a region or peak pass reads best state 0 and writes planes of its own
+    const bool reads_best = so.region || so.peak;
     if (!fast) SB_OK(ensure_diffs64(pl));
 
     // order templates by search angle (then best state) so that each curvature spectrum is built once
@@ -540,6 +551,7 @@ int run_sweep_t(sb_plan* pl, const sb_angle* angles, int n_angles, const sb_temp
         if (t.angle_id < 0 || t.angle_id >= n_angles) return fail("template angle_id out of range");
         if (t.state < 0 || t.state >= pl->n_states) return fail("template state out of range (option \"states\")");
         if (so.region && t.state != 0) return fail("fit region: every record must be in best state 0 (state != 0)");
+        if (so.peak && t.state != 0) return fail("fit peak: every record must be in best state 0 (state != 0)");
         if (t.sy_hi < t.sy_lo || t.sx_hi < t.sx_lo) return fail("empty template support box");
         if (t.sy_lo < -(pl->ny / 2) || t.sy_hi > pl->ny - 1 - pl->ny / 2 || t.sx_lo < -(pl->nx / 2) ||
             t.sx_hi > pl->nx - 1 - pl->nx / 2)
@@ -736,8 +748,8 @@ int run_sweep_t(sb_plan* pl, const sb_angle* angles, int n_angles, const sb_temp
         nsub = std::max(1, std::min(nsub, Bt / 2));
     }
     const long sub_stride = bn_all(pl);
-    // (a region pass keeps the sub-streams, whose templates all compare with state 0: no copies)
-    if (nsub > 1 && !so.region) {
+    // (a region or peak pass keeps the sub-streams, whose templates all compare with state 0: no copies)
+    if (nsub > 1 && !reads_best) {
         if (nsub > pl->best_copies) {
             // grow the best-state arrays to nsub copies, keeping copy 0 (the accumulated state)
             float *s2 = nullptr, *a2 = nullptr;
@@ -978,6 +990,23 @@ int run_sweep_t(sb_plan* pl, const sb_angle* angles, int n_angles, const sb_temp
                                                       (const float4*)pl->gbuf.p, (const float2*)twx, cross,
                                                       *so.region);
                                     }
+                                    if (so.peak) {
+                                        if (masked) {
+                                            if constexpr (N <= kMaxFftMasked) {
+                                                return launch(pl, "k_fit_rows_gmp", sb::k_fit_rows_gmp<N>, grid,
+                                                              dim3(S::threads),
+                                                              S::smem_fit_f + sb::fit_masked_extra_smem<N>(), g,
+                                                              gp.count, d_slots, (const sb::FitT*)pl->fit.p,
+                                                              (const sb::FitM*)pl->fitm.p, ch.cnt,
+                                                              (const float4*)pl->gbuf.p, (const float2*)twx, cross,
+                                                              *so.peak);
+                                            }
+                                            return fail("internal: masked fit at FFT length " + std::to_string(N));
+                                        }
+                                        return launch(pl, "k_fit_rows_gp", sb::k_fit_rows_gp<N>, grid, dim3(S::threads),
+                                                      S::smem_fit_f, g, gp.count, d_slots, (const sb::FitT*)pl->fit.p,
+                                                      (const float4*)pl->gbuf.p, (const float2*)twx, cross, *so.peak);
+                                    }
                                     if (so.second) {
                                         if (masked) {
                                             if constexpr (N <= kMaxFftMasked) {
@@ -1015,7 +1044,7 @@ int run_sweep_t(sb_plan* pl, const sb_angle* angles, int n_angles, const sb_temp
                                                   (const float4*)pl->gbuf.p, bsnr, bamp, bidx, (const float2*)twx,
                                                   cross, sub_stride);
                                 }));
-                                if (g.poison && !so.region)
+                                if (g.poison && !reads_best)
                                     SB_OK(launch(pl, "k_poison_windows", sb::k_poison_windows,
                                                  dim3(div_up((long)g.out_ny * g.out_nx, 256)), dim3(256), 0, g,
                                                  gp.count, d_slots, (const sb::FitT*)pl->fit.p, bsnr));
@@ -1040,13 +1069,13 @@ int run_sweep_t(sb_plan* pl, const sb_angle* angles, int n_angles, const sb_temp
         }
     // a secondary sweep folds and clears best state 1 alone
     const long st_off = so.second ? bn : 0, st_len = so.second ? bn : sub_stride;
-    if (nsub > 1 && !so.region) {
+    if (nsub > 1 && !reads_best) {
         SB_OK(launch(pl, "k_best_fold", sb::k_best_fold, dim3(div_up(st_len, 256)), dim3(256), 0, st_len,
                      nsub - 1, sub_stride, (const float*)pl->d_bsnr + sub_stride + st_off,
                      (const float*)pl->d_bamp + sub_stride + st_off, (const int*)pl->d_bidx + sub_stride + st_off,
                      pl->d_bsnr + st_off, pl->d_bamp + st_off, pl->d_bidx + st_off));
     }
-    if (masked && !so.region) {
+    if (masked && !reads_best) {
         SB_OK(launch(pl, "k_best_clear_nodata", sb::k_best_clear_nodata, dim3(div_up(bn, 256)), dim3(256), 0, pl->ny,
                      pl->nx, pl->row0, pl->slab_lo, (int)pl->brows(), so.second ? 1 : pl->n_states, bn,
                      (const double*)pl->d_dem, pl->d_bsnr + st_off, pl->d_bamp + st_off, pl->d_bidx + st_off));
@@ -1140,7 +1169,7 @@ int sb_plan_destroy(sb_plan* pl) {
     for (auto e : pl->ev_pool) sb_rt_event_destroy(e);
     for (Buf* b : {&pl->cr, &pl->fct, &pl->trt, &pl->part, &pl->gbuf, &pl->sums, &pl->fit, &pl->tmpls, &pl->angles,
                    &pl->tables, &pl->raw, &pl->tbox, &pl->slots, &pl->cross, &pl->casa, &pl->aux, &pl->spec9, &pl->coef,
-                   &pl->fitm, &pl->fs_idx, &pl->fs_out, &pl->region, &pl->rtab, &pl->spos})
+                   &pl->fitm, &pl->fs_idx, &pl->fs_out, &pl->region, &pl->rtab, &pl->spos, &pl->peak})
         release(*b);
 #ifndef SB_EMU
     if (pl->own_stream) cudaStreamDestroy(pl->stream);
@@ -1245,7 +1274,7 @@ long sb_plan_device_bytes(const sb_plan* pl) {
     b += (size_t)pl->bn() * pl->n_states * pl->best_copies * 12;
     for (const Buf* q : {&pl->cr, &pl->fct, &pl->trt, &pl->part, &pl->gbuf, &pl->sums, &pl->fit, &pl->tmpls, &pl->angles,
                          &pl->tables, &pl->raw, &pl->tbox, &pl->slots, &pl->cross, &pl->casa, &pl->aux, &pl->spec9, &pl->coef,
-                         &pl->fitm, &pl->fs_idx, &pl->fs_out, &pl->region, &pl->rtab, &pl->spos})
+                         &pl->fitm, &pl->fs_idx, &pl->fs_out, &pl->region, &pl->rtab, &pl->spos, &pl->peak})
         b += q->cap;
     return (long)b;
 }
@@ -1646,6 +1675,103 @@ int sb_secondary_sweep(sb_plan* pl, const sb_angle* angles, int n_angles, const 
     so.second = &sec;
     SB_OK(run_sweep(pl, angles, n_angles, tmpls, n_tmpls, so, whole_search5));
     SB_TRY(sb_rt_sync(pl->stream));
+    return 0;
+}
+
+int sb_peak_sweep(sb_plan* pl, const sb_angle* angles, int n_angles, const sb_template* tmpls, int n_tmpls,
+                  const int32_t* whole_search5, const int32_t* age_rank_host, const int32_t* angle_pos_host, int n_idx,
+                  int n_ranks, int n_pos, int periodic) {
+    if (!pl || !angles || !tmpls || !age_rank_host || !angle_pos_host || n_idx <= 0)
+        return fail("sb_peak_sweep: bad arguments");
+    if (pl->precision != 32 || !pl->fast) return fail("sb_peak_sweep: fit peak needs precision 32 and the option fast");
+    // 16-bit fields of the winner code; rank 0xffff is left free for the codes that match nothing
+    if (n_ranks < 1 || n_ranks > 0xffff) return fail("sb_peak_sweep: n_ranks must be in 1 .. 65535");
+    if (n_pos < 1 || n_pos > 0xffff) return fail("sb_peak_sweep: n_pos must be in 1 .. 65535");
+    if (periodic && n_pos < 3) return fail("sb_peak_sweep: a periodic search needs n_pos >= 3");
+    for (int k = 0; k < n_idx; ++k)
+        if (age_rank_host[k] < 0 || age_rank_host[k] >= n_ranks || angle_pos_host[k] < 0 || angle_pos_host[k] >= n_pos)
+            return fail("sb_peak_sweep: age rank or orientation position out of range at flat index " + std::to_string(k));
+    for (int k = 0; k < n_tmpls; ++k) {
+        if (tmpls[k].idx < 0 || tmpls[k].idx >= n_idx)
+            return fail("sb_peak_sweep: template flat index outside 0 .. n_idx - 1");
+        if (tmpls[k].state != 0) return fail("sb_peak_sweep: every record must be in best state 0 (state != 0)");
+    }
+    // per flat index, the winner codes it neighbours: winner rank + 1 (it is age-), rank - 1 (age+),
+    // position + 1 (ang-) and position - 1 (ang+), the positions wrapping round in a periodic search
+    const int none = (int)0xfffffffeu;
+    std::vector<int4> codes(n_idx);
+    for (int k = 0; k < n_idx; ++k) {
+        const int r = age_rank_host[k], p = angle_pos_host[k];
+        const int up = p + 1 < n_pos ? p + 1 : periodic ? 0 : -1, down = p > 0 ? p - 1 : periodic ? n_pos - 1 : -1;
+        codes[k].x = r + 1 < n_ranks ? (r + 1) << 16 | p : none;
+        codes[k].y = r > 0 ? (r - 1) << 16 | p : none;
+        codes[k].z = up >= 0 ? r << 16 | up : none;
+        codes[k].w = down >= 0 ? r << 16 | down : none;
+    }
+    const long bn = pl->bn(), boff = (long)pl->slab_lo * pl->nx;
+    SB_OK(ensure(pl->rtab, (size_t)n_idx * (sizeof(int4) + 2 * sizeof(int32_t))));
+    SB_OK(ensure(pl->peak, (size_t)5 * bn * sizeof(int)));
+    int4* d_codes = (int4*)pl->rtab.p;
+    int* d_rank = (int*)(d_codes + n_idx);
+    int* d_pos = d_rank + n_idx;
+    int* planes = (int*)pl->peak.p;
+    unsigned* code = (unsigned*)(planes + 4 * bn);
+    SB_TRY(sb_rt_h2d(d_codes, codes.data(), (size_t)n_idx * sizeof(int4), pl->stream));
+    SB_TRY(sb_rt_h2d(d_rank, age_rank_host, (size_t)n_idx * sizeof(int32_t), pl->stream));
+    SB_TRY(sb_rt_h2d(d_pos, angle_pos_host, (size_t)n_idx * sizeof(int32_t), pl->stream));
+    SB_TRY(sb_rt_memset(planes, 0, (size_t)4 * bn * sizeof(int), pl->stream));
+    SB_OK(launch(pl, "k_peak_code", sb::k_peak_code, dim3(div_up(bn, 256)), dim3(256), 0, bn, (const float*)pl->d_bsnr,
+                 (const int*)pl->d_bidx, (const int*)d_rank, (const int*)d_pos, n_idx, code));
+    SB_TRY(sb_rt_sync(pl->stream));                     // `codes` must outlive its copy
+    sb::PeakOut pk;
+    pk.code = code - boff;
+    pk.planes = planes - boff;
+    pk.codes = d_codes;
+    pk.plane = bn;
+    pl->peak_npos = 0;
+    SweepOut so;
+    so.peak = &pk;
+    SB_OK(run_sweep(pl, angles, n_angles, tmpls, n_tmpls, so, whole_search5));
+    SB_TRY(sb_rt_sync(pl->stream));
+    pl->peak_nranks = n_ranks;
+    pl->peak_npos = n_pos;
+    return 0;
+}
+
+int sb_peak_finalize(sb_plan* pl, int row_lo, int row_hi, const double* age_of_host, const double* angle_of_host,
+                     int n_idx, const double* log10_rank_age_host, int n_ranks, int n_pos, int periodic, double step,
+                     double* out8) {
+    if (!pl || !age_of_host || !angle_of_host || !log10_rank_age_host || !out8 || n_idx <= 0)
+        return fail("sb_peak_finalize: bad arguments");
+    if (pl->peak_npos == 0) return fail("sb_peak_finalize: no peak sweep since the best state was last allocated");
+    if (n_ranks != pl->peak_nranks || n_pos != pl->peak_npos)
+        return fail("sb_peak_finalize: n_ranks / n_pos differ from the peak sweep's");
+    if (!std::isfinite(step)) return fail("sb_peak_finalize: step must be finite");
+    if (row_lo < pl->slab_lo || row_hi > pl->slab_hi || row_lo >= row_hi) return fail("sb_peak_finalize: rows outside the plan");
+    const long n = (long)(row_hi - row_lo) * pl->nx;
+    const long off = (long)(row_lo - pl->slab_lo) * pl->nx;
+    const long bn = pl->bn();
+    SB_OK(ensure(pl->tables, (size_t)(2 * n_idx + n_ranks) * sizeof(double)));
+    double* d_age = (double*)pl->tables.p;
+    double* d_ang = d_age + n_idx;
+    double* d_lx = d_ang + n_idx;
+    SB_TRY(sb_rt_h2d(d_age, age_of_host, (size_t)n_idx * sizeof(double), pl->stream));
+    SB_TRY(sb_rt_h2d(d_ang, angle_of_host, (size_t)n_idx * sizeof(double), pl->stream));
+    SB_TRY(sb_rt_h2d(d_lx, log10_rank_age_host, (size_t)n_ranks * sizeof(double), pl->stream));
+    SB_OK(ensure(pl->raw, (size_t)n * 8 * sizeof(double)));
+    double* dst = (double*)pl->raw.p;
+    const int* planes = (const int*)pl->peak.p + off;
+    SB_OK(launch(pl, "k_peak_finalize", sb::k_peak_finalize, dim3(div_up(n, 256)), dim3(256), 0, n, bn,
+                 (const float*)pl->d_bsnr + off, (const float*)pl->d_bamp + off, (const int*)pl->d_bidx + off,
+                 (const unsigned*)(planes + 4 * bn), (const float*)planes, (const double*)d_age, (const double*)d_ang,
+                 n_idx, (const double*)d_lx, n_ranks, n_pos, periodic ? 1 : 0, step, dst));
+    return copy_out(pl, out8, dst, (size_t)n * 8, 0);
+}
+
+int sb_peak_planes(sb_plan* pl, int32_t** planes_dev) {
+    if (!pl || !planes_dev) return fail("sb_peak_planes: bad arguments");
+    if (pl->peak_npos == 0) return fail("sb_peak_planes: no peak sweep since the best state was last allocated");
+    *planes_dev = (int32_t*)pl->peak.p;
     return 0;
 }
 

@@ -496,6 +496,45 @@ class Plan(object):
         check(self.lib, self.lib.sb_secondary_sweep(self._h, arr_a, na, arr_t, nt, whole, pos.ctypes.data, len(pos),
                                                     len(tables.pos_angle), int(tables.periodic), int(min_sep_pos)))
 
+    def peak_sweep(self, angle_records, template_records, tables):
+        """Pass 2 of a sub-grid fit peak (``sb_peak_sweep``, DESIGN.md section 17): best state 0 must
+        hold the result of ``sweep`` over the same records.  Sweeps them again and records, per pixel,
+        the largest SNR of the templates one age rank and one orientation position either side of the
+        winner (``peak_planes``); ``tables``: ``params.region_tables`` of the search.  The best state
+        is not modified."""
+        arr_a, na = angle_records
+        arr_t, nt = template_records[0], template_records[1]
+        whole = template_records[2] if len(template_records) > 2 else None
+        rank = np.ascontiguousarray(tables.age_rank, dtype=np.int32)
+        pos = np.ascontiguousarray(tables.angle_pos, dtype=np.int32)
+        check(self.lib, self.lib.sb_peak_sweep(self._h, arr_a, na, arr_t, nt, whole, rank.ctypes.data,
+                                               pos.ctypes.data, len(rank), len(tables.rank_age),
+                                               len(tables.pos_angle), int(tables.periodic)))
+
+    def peak_finalize(self, age_of, angle_of, tables, rows=None):
+        """(8, rows, nx) float64 [amp, age, angle, snr, age_peak, angle_peak, snr_peak, refined] after
+        ``peak_sweep`` (``sb_peak_finalize``): planes 0..3 are ``finalize``'s, 4..7 the vertex of the
+        parabola through the winner and its neighbours on each axis (``core.fit_peak``).
+        ``rows=(lo, hi)``: a band of the plan's rows (default: all of them)."""
+        age_of, angle_of = _as_f64(age_of), _as_f64(angle_of)
+        lx = np.log10(_as_f64(tables.rank_age))
+        pos_angle = _as_f64(tables.pos_angle)
+        step = float(pos_angle[1] - pos_angle[0]) if len(pos_angle) > 1 else 0.0
+        lo, hi = (self.row_lo, self.row_hi) if rows is None else (int(rows[0]), int(rows[1]))
+        out = np.empty((8, max(hi - lo, 0), self.nx), dtype=np.float64)
+        check(self.lib, self.lib.sb_peak_finalize(self._h, lo, hi, age_of.ctypes.data, angle_of.ctypes.data,
+                                                  len(age_of), lx.ctypes.data, len(lx), len(pos_angle),
+                                                  int(tables.periodic), step, out.ctypes.data))
+        return out
+
+    def peak_planes(self):
+        """Device pointer (int32) of the four neighbour planes after ``peak_sweep`` (``sb_peak_planes``):
+        the bits of float32 SNRs, plane ``j`` (age-, age+, orientation-, orientation+) of pixel ``i``
+        of the plan's rows at ``[j * rows * nx + i]``."""
+        p = c_void_p()
+        check(self.lib, self.lib.sb_peak_planes(self._h, byref(p)))
+        return p.value
+
     def region_finalize(self, age_of, angle_of, tables, rows=None):
         """(9, rows, nx) float64 [amp, age, angle, snr, age_lo, age_hi, angle_lo, angle_hi, n_fits] after
         ``region_sweep`` (``sb_region_finalize``): planes 0..3 are ``finalize``'s, 4..8 the region's
