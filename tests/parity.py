@@ -120,6 +120,55 @@ def assert_parity(rep, frac=None, agreement=INDEX_AGREEMENT, explain=True, tie_s
     assert rep["frac_snr_over_tol"] <= frac and rep["frac_amp_over_tol"] <= frac, rep
 
 
+def template_shares(z, spec, scale, ages, angles, device=None, curv=None, options=None, geometry=None, run=None,
+                    angle_ids=None, **plan_kw):
+    """Yields ``(i, snr, amp)``: the float32 SNR and amplitude planes [ages, rows, nx] of the templates of
+    orientation i, from one-orientation shares of the search on a plan with one best state per age
+    (read in place through the plan's device pointers; valid until the next yield).  Each share carries
+    the whole search's extents (``sb_sweep_ex``), so its planes are those the whole search computes.
+    ``curv``: the curvature statistics of a row slab's whole raster.  ``options``: plan options
+    (``set_option``) set before the DEM.  ``geometry``: a list that gets each share's ``last_geometry()``.
+    ``run``: a slice of at most 64 of ``ages`` (a search over more ages goes in runs); the planes are then
+    [len(ages[run]), rows, nx] and the shares still carry the extents of the search over all ``ages``.
+    ``angle_ids``: the orientations to yield (default: all)."""
+    import ctypes
+    from scarplet_b200 import params as P
+    from scarplet_b200.distributed import _as_tensor
+    from scarplet_b200.engine import Plan
+    ny, nx = z.shape
+    ages = np.asarray(ages, dtype=np.float64)
+    G = len(ages if run is None else ages[run])
+    cuda = device is not None
+    with Plan(ny, nx, 1.0, 1.0, states=G, **plan_kw) as plan:
+        for key, value in (options or {}).items():
+            plan.set_option(key, value)
+        plan.set_dem(z)
+        if curv is not None:
+            plan.set_curv_stats(*curv)
+        rows = plan.row_hi - plan.row_lo
+        if run is not None:
+            whole = (ctypes.c_int * 5)(*P.support_extents(spec, scale, ages, angles, nx, ny, 1.0), len(ages))
+        for i in (range(len(angles)) if angle_ids is None else angle_ids):
+            if run is None:
+                a, t, _, _ = plan.build_sweep(spec, scale, ages, angles, angle_slice=(i, i + 1), state_per_age=True)
+            else:
+                a, t, _, _ = plan.build_sweep(spec, scale, ages[run], angles, angle_slice=(i, i + 1),
+                                              state_per_age=True)
+                t = (t[0], t[1], whole)
+            assert t[2] is not None or len(angles) == 1     # the whole search's extents go with the share
+            plan.reset()
+            plan.sweep(a, t)
+            plan.sync()
+            if geometry is not None:
+                geometry.append(plan.last_geometry())
+            ps, pa, _ = plan.best_state_pointers(0)
+            yield (i, _as_tensor(ps, G * rows * nx, "f4", device).reshape(G, rows, nx),
+                   _as_tensor(pa, G * rows * nx, "f4", device).reshape(G, rows, nx))
+            if cuda:
+                import torch
+                torch.cuda.synchronize(device)
+
+
 def save_report(name, rep, extra=None):
     """Keep a parity report as JSON (``gpurun_out/parity/<name>.json`` by default; the kept
     copies of a round live under ``profiles/``)."""

@@ -4,16 +4,16 @@ one orientation position either side of its winner, recorded by a second sweep o
 
 Planes 0..3 must equal ``match`` bit for bit.  The four neighbour planes (``Plan.peak_planes``) are
 checked exactly against a restatement built from every template's float32 SNR plane, taken from
-one-orientation shares of the same search (``tests.test_secondary_fit.template_shares``); planes 5..7
+one-orientation shares of the same search (``tests.parity.template_shares``); planes 5..7
 against a NumPy float64 restatement of the formulas on those neighbours, bit for bit, and plane 4 (the
 one ``exp10``) within 2 ulp.  The CPU cases run the emulator build of the kernels (tests/emu), the
 ``gpu`` cases the B200."""
 import numpy as np
 import pytest
 
-from tests.parity import save_report
+from tests.parity import save_report, template_shares
 from tests.test_nodata_mask import _gpu_holes, _holes
-from tests.test_secondary_fit import positions_of, template_shares
+from tests.test_secondary_fit import positions_of
 
 
 def _template(name):
@@ -73,7 +73,7 @@ def restated_neighbours(z, spec, scale, ages, angles, ref, device=None, **plan_k
     for g0 in range(0, len(ages), 64):
         run = slice(g0, g0 + 64)
         shares = (template_shares(z, spec, scale, ages, angles, device, **plan_kw) if len(ages) <= 64 else
-                  _age_run_shares(z, spec, scale, ages, run, angles, **plan_kw))
+                  template_shares(z, spec, scale, ages, angles, run=run, **plan_kw))
         for i, snr, _ in shares:
             pos = i % w.n_pos
             for g, rk in enumerate(rank[run]):
@@ -82,27 +82,6 @@ def restated_neighbours(z, spec, scale, ages, angles, ref, device=None, **plan_k
                     q = fit & (tr == int(rk)) & (tp == pos) & (s > out[j])
                     out[j] = torch.where(q, s, out[j])
     return out.cpu().numpy()
-
-
-def _age_run_shares(z, spec, scale, ages, run, angles):
-    """``template_shares`` (on the host) for the ages ``ages[run]`` of a search over more than 64 ages: each
-    one-orientation share carries the extents of the whole search, so that every template's SNR is the
-    one the whole search computes."""
-    from scarplet_b200.distributed import _as_tensor
-    from scarplet_b200.engine import Plan
-    ny, nx = z.shape
-    G = len(ages[run])
-    with Plan(ny, nx, 1.0, 1.0, states=G) as plan:
-        plan.set_dem(z)
-        for i in range(len(angles)):
-            whole = plan.build_sweep(spec, scale, ages, angles, angle_slice=(i, i + 1))[1][2]
-            a, t, _, _ = plan.build_sweep(spec, scale, ages[run], angles, angle_slice=(i, i + 1), state_per_age=True)
-            plan.reset()
-            plan.sweep(a, (t[0], t[1], whole))
-            plan.sync()
-            ps, pa, _ = plan.best_state_pointers(0)
-            yield (i, _as_tensor(ps, G * ny * nx, "f4", None).reshape(G, ny, nx),
-                   _as_tensor(pa, G * ny * nx, "f4", None).reshape(G, ny, nx))
 
 
 def restated_peak(ref, nb, ages, angles):

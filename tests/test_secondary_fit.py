@@ -11,7 +11,7 @@ cases run the emulator build of the kernels (tests/emu), the ``gpu`` cases the B
 import numpy as np
 import pytest
 
-from tests.parity import save_report
+from tests.parity import save_report, template_shares
 from tests.test_nodata_mask import _gpu_holes, _holes
 
 
@@ -33,35 +33,6 @@ def _dem(shape, seed):
 # ---------------------------------------------------------------------------
 # the contract, restated
 # ---------------------------------------------------------------------------
-def template_shares(z, spec, scale, ages, angles, device=None, curv=None, **plan_kw):
-    """Yields ``(i, snr, amp)``: the float32 SNR and amplitude planes [ages, rows, nx] of the templates of
-    orientation i, from one-orientation shares of the search on a plan with one best state per age
-    (read in place through the plan's device pointers; valid until the next yield).  ``curv``: the
-    curvature statistics of a row slab's whole raster."""
-    from scarplet_b200.distributed import _as_tensor
-    from scarplet_b200.engine import Plan
-    ny, nx = z.shape
-    G = len(ages)
-    cuda = device is not None
-    with Plan(ny, nx, 1.0, 1.0, states=G, **plan_kw) as plan:
-        plan.set_dem(z)
-        if curv is not None:
-            plan.set_curv_stats(*curv)
-        rows = plan.row_hi - plan.row_lo
-        for i in range(len(angles)):
-            a, t, _, _ = plan.build_sweep(spec, scale, ages, angles, angle_slice=(i, i + 1), state_per_age=True)
-            assert t[2] is not None             # the whole search's extents go with the share
-            plan.reset()
-            plan.sweep(a, t)
-            plan.sync()
-            ps, pa, _ = plan.best_state_pointers(0)
-            yield (i, _as_tensor(ps, G * rows * nx, "f4", device).reshape(G, rows, nx),
-                   _as_tensor(pa, G * rows * nx, "f4", device).reshape(G, rows, nx))
-            if cuda:
-                import torch
-                torch.cuda.synchronize(device)
-
-
 def position_distance(p, q, n_pos, periodic):
     d = np.abs(np.asarray(p) - np.asarray(q))
     return np.minimum(d, n_pos - d) if periodic else d
